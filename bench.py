@@ -10,7 +10,9 @@ performs one suffix-match + draft query (DraftModel.update + DraftModel.lookup o
 Extra objects on the same JSON line: `verify` (config c4: fused verify + KV compaction,
 us/step and GB/s against the HBM roofline) and `static` (config c3 at a host-buildable corpus size).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+With --dump-outputs the headline's last timed step (drafts, lengths, sources, match lengths, state indices) goes to
+DIR/<name>.npy; the inputs are seeded, so two builds run with the same arguments can be compared array for array.
 Under torchrun (N > 1) every rank runs the same per-GPU workload on its own requests (weak
 scaling, no data-path collective); rank 0 prints ONE JSON line.
 """
@@ -65,7 +67,14 @@ def parse():
     ap.add_argument("--ngram", type=int, default=None, help="tuning aid: depth of the short-context scouts (-1 off)")
     ap.add_argument("--prewalk", type=int, default=None, help="tuning aid: draft tokens the scouts walk ahead for the next step")
     ap.add_argument("--variant", type=int, default=1, help="step kernel variant: 1 = one thread per request (default), 0 = warp-cooperative (round 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the headline workload as DIR/<name>.npy (float64)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and (a.impl != "ours" or a.only_verify or a.only_static or a.only_tree or a.only_c1):
+        ap.error("--dump-outputs needs the headline workload of --impl ours")
+    return a
 
 
 # --------------------------------------------------------------------------------------
@@ -285,8 +294,7 @@ def run_reference(a):
     real = have_staged_reference()
     # bounded sample: a step of the reference arm is one pass over `n_sample` requests of the c2 workload
     n_sample = cores * (16 if real else 64)
-    steps = min(a.steps, 256)
-    warm = min(a.warmup, 16)
+    steps, warm = a.steps, a.warmup
     t0 = time.time()
     qps, wall, used = cpu_arm(n_sample, a.prompt, steps, warm, 2000, cores, worker=_cpu_worker_ref if real else None)
     if real:
@@ -431,6 +439,7 @@ def run_ours(a):
     stats1 = dyn.stats()
     assert stats1["overflowed"] == 0, "arena overflow in the timed region"
     draft_checksum = int(eng.draft.sum().item())
+    last_step = step_outputs(eng) if a.dump_outputs and rank == 0 else None
 
     # per-launch duration of the step kernel, measured live with CUDA events (eager launches)
     warm()
@@ -663,8 +672,35 @@ def run_ours(a):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+    if last_step is not None:
+        save_outputs(a.dump_outputs, last_step)
     if rank == 0:
         print(json.dumps(out))
+
+
+DUMP_LIMIT_BYTES = 63_000_000      # under 64 MB with the .npy headers
+
+
+def step_outputs(eng):
+    """What DraftEngine.step hands its caller, per request, as float64 (the int32 values are exact): the draft
+    [R, n_predicts], its length, the draft source, and match length and state index in the dynamic and static automata."""
+    fields = {"draft": eng.draft, "draft_len": eng.draft_len, "type": eng.out_type, "match_dyn": eng.match_dyn,
+              "match_static": eng.match_static, "index_dyn": eng.index_dyn, "index_static": eng.index_static}
+    return {name: t.cpu().numpy().astype(np.float64) for name, t in fields.items()}
+
+
+def save_outputs(path, arrays):
+    """DIR/<name>.npy for every array; above DUMP_LIMIT_BYTES only a fixed, seeded sample of the requests is kept and
+    their indices go to request_index.npy."""
+    n = len(arrays["draft"])
+    row_bytes = sum(v.nbytes for v in arrays.values()) // n
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // (row_bytes + 8), replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+        arrays["request_index"] = keep.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), v)
 
 
 def bench_verify(a, dev, hbm_peak, iters=40, warm=5, vocab=None, heads=32, kv_len=None, name="c4", recycle=True):
