@@ -228,6 +228,51 @@ int samd_static_tree_draft(samd_static_t h, int n_requests, const int32_t *type_
                            int32_t *out_retrieve_dev, int32_t max_paths, int32_t max_depth,
                            int32_t *out_retrieve_shape_dev, void *stream);
 
+/* sam_only batch buffers (gen_buffers samd_sam_only/sam/static_sam.py:148-180, sequence positions
+ * samd_sam_only/sam/dyn_sam.py:116-121, the mask splice samd_sam_only/model_patch/llama.py:94-96, the decode step
+ * samd_sam_only/samd_model.py:117-157): per request b, its sequence draft (samd_step: draft_len tokens) or, when
+ * type_dev[b] == SAMD_DRAFT_STATIC_TREE, its static tree (samd_static_tree_draft) becomes uniform rows:
+ *   tokens[b][T]            node tokens, 0 past the request's node count
+ *   position_ids[b][T]      cache_len[b] + depth of the node (a sequence: the node index; pad rows: the row index)
+ *   n_nodes[b], n_paths[b]
+ *   retrieve[b][P][D]       a tree's leaf paths, or the sequence's one path 0..draft_len-1; -1 padded
+ *   mask[b][T][kv_len]      additive, in the LM's dtype: 0 where node i may attend, the dtype's lowest finite value
+ *                           (torch.finfo(dtype).min) elsewhere.  Node i sees every column < cache_len[b] and column
+ *                           cache_len[b] + j for j = i and every ancestor of i (a sequence: every j <= i).  Rows
+ *                           i >= n_nodes[b] see the past and themselves, never nothing.
+ * Any type other than SAMD_DRAFT_STATIC_TREE is a sequence, and a non-tree request's tree arrays are not read (they are
+ * stale).  tree_tokens_dev NULL = no tree drafter: every request is a sequence.  A finished request (done_dev[b] != 0)
+ * gets a one-node draft: n_nodes = 1, retrieve row 0 = [0, -1, ...], n_paths = 0 - the verify walk accepts nothing and
+ * maps index 0 to 0, so samd_verify_compact moves none of its KV rows.  T <= 256, kv_len >= T.  No argument depends on
+ * the step, so the launch can be captured in a CUDA graph. */
+typedef struct samd_assemble_args {
+    int32_t        batch;
+    int32_t        n_nodes;           /* T: node rows per request */
+    int32_t        n_paths, depth;    /* P x D path table */
+    const int32_t *type_dev;          /* [B] SAMD_DRAFT_* (samd_step out_type), or NULL = all sequences */
+    const int32_t *draft_dev;         /* [B][draft_stride] sequence drafts (samd_step out_draft) */
+    int32_t        draft_stride;
+    const int32_t *draft_len_dev;     /* [B] */
+    /* samd_static_tree_draft outputs, or tree_tokens_dev NULL */
+    const int32_t *tree_tokens_dev, *tree_parents_dev, *tree_depth_dev;  /* [B][tree_stride], tree_stride <= T */
+    int32_t        tree_stride;
+    const int32_t *tree_n_dev;        /* [B] */
+    const int32_t *tree_retrieve_dev; /* [B][tree_max_paths][tree_max_depth], tree_max_paths <= P, tree_max_depth <= D */
+    int32_t        tree_max_paths, tree_max_depth;
+    const int32_t *tree_shape_dev;    /* [B][2] {leaves, deepest path} */
+    const int32_t *cache_len_dev;     /* [B] */
+    const uint8_t *done_dev;          /* [B] finished requests, or NULL */
+    int32_t        mask_dtype;        /* SAMD_DTYPE_* */
+    int32_t        kv_len;
+    /* outputs */
+    int32_t *out_tokens_dev;          /* [B][T] */
+    int64_t *out_position_ids_dev;    /* [B][T] */
+    int32_t *out_n_nodes_dev, *out_n_paths_dev;   /* [B] */
+    int32_t *out_retrieve_dev;        /* [B][P][D] */
+    void    *out_mask_dev;            /* [B][T][kv_len] */
+} samd_assemble_args;
+int samd_draft_assemble(const samd_assemble_args *args, void *stream);
+
 /* ----------------------------------------------------------------------------------------
  * Document-sharded static SAM (SURVEY.md section 8e): per-shard packed keys
  *   key = (match_len << 32) | (0xFFFFFFFF - (shard_offset + min_endpos)), 0 when no match,

@@ -407,7 +407,8 @@ __global__ void __launch_bounds__(VT, 4) verify_compact_kernel(VerifyParams P) {
         const int n_paths = A.retrieve_dev ? (A.n_paths_dev ? A.n_paths_dev[b] : A.n_paths) : 1;
         const int depth = A.retrieve_dev ? A.depth : n_rows;
         constexpr int WD = 8;                                   // path depth held in registers
-        const bool fast = A.retrieve_dev && depth <= WD && n_paths <= 32;
+        // (a request with no live path - a finished one, samd_draft_assemble - takes the general walk: acc = 0, index 0 -> 0)
+        const bool fast = A.retrieve_dev && depth <= WD && n_paths > 0 && n_paths <= 32;
         int rp[WD];
 #pragma unroll
         for (int j = 0; j < WD; ++j) rp[j] = (fast && lane < n_paths && j < depth) ? ri_at(P, b, lane, j) : -1;

@@ -62,6 +62,18 @@ class SampleArgs(C.Structure):
     ]
 
 
+class AssembleArgs(C.Structure):
+    _fields_ = [
+        ("batch", C.c_int32), ("n_nodes", C.c_int32), ("n_paths", C.c_int32), ("depth", C.c_int32), ("type_dev", vp),
+        ("draft_dev", vp), ("draft_stride", C.c_int32), ("draft_len_dev", vp), ("tree_tokens_dev", vp),
+        ("tree_parents_dev", vp), ("tree_depth_dev", vp), ("tree_stride", C.c_int32), ("tree_n_dev", vp),
+        ("tree_retrieve_dev", vp), ("tree_max_paths", C.c_int32), ("tree_max_depth", C.c_int32), ("tree_shape_dev", vp),
+        ("cache_len_dev", vp), ("done_dev", vp), ("mask_dtype", C.c_int32), ("kv_len", C.c_int32),
+        ("out_tokens_dev", vp), ("out_position_ids_dev", vp), ("out_n_nodes_dev", vp), ("out_n_paths_dev", vp),
+        ("out_retrieve_dev", vp), ("out_mask_dev", vp),
+    ]
+
+
 # name -> (restype, argtypes); every symbol include/samd_b200.h declares
 SYMBOLS = {
     "samd_abi_version": (C.c_int, []),
@@ -108,6 +120,7 @@ SYMBOLS = {
     "samd_debug_replay_trace": (C.c_int, [vp, vp, C.c_int, C.c_int, vp, vp]),
     "samd_static_tree_draft": (C.c_int, [vp, C.c_int, vp, vp, vp, vp, C.c_int32, C.c_double, C.c_int32, C.c_int32,
                                          vp, vp, vp, vp, vp, C.c_int32, C.c_int32, vp, vp]),
+    "samd_draft_assemble": (C.c_int, [C.POINTER(AssembleArgs), vp]),
     "samd_static_lookup_keys": (C.c_int, [vp, vp, vp, C.c_int, C.c_int64, vp, vp]),
     "samd_draft_from_keys": (C.c_int, [vp, vp, C.c_int64, vp, C.c_int, C.c_int32, vp, vp, C.c_int32, vp]),
     "samd_xchg_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(vp)]),

@@ -18,6 +18,9 @@ a chain (one path), a tree request uses the tree's ancestor mask and path table;
 positions and path tables are selected per request on the device, and samd_verify_compact moves the accepted
 rows into place (cache.py:118-133).  Greedy verification makes any draft lossless, so the output stream equals
 plain greedy decoding token for token.
+
+BatchedSamOnlyDecoder runs the same loop with the samd_sam_only flavour's drafts: per-request variable-length
+sequences and static-SAM trees, assembled into uniform batch buffers on the device by samd_draft_assemble.
 """
 from __future__ import annotations
 
@@ -28,6 +31,8 @@ from transformers.cache_utils import Cache, CacheLayerMixin
 
 from . import _cabi as K
 from . import engine as E
+
+_cabi = K                       # (BatchedSamOnlyDecoder takes a parameter named K)
 
 
 class _Layer(CacheLayerMixin):
@@ -182,25 +187,33 @@ class BatchedSamdDecoder:
                                move_kv=True, n_nodes=self._n_nodes[kind].contiguous(), n_paths=self._n_paths[kind].contiguous(),
                                out=res, recycle=self.table)
 
+    def _draft_forward_verify(self, kv_len: int) -> dict:
+        """Drafts in, LM forward, fused verify: the part of a step that depends on the draft flavour."""
+        st, T, cache = self._st, self.T, self.cache
+        self.eng.step(st["acc_tokens"], st["acc_count"], st["start"])              # update(accepted) + lookup(start): one launch
+        cache.begin(T, kv_len)
+        if self.tree is not None:
+            return self._tree_step(st["start"], kv_len, st["res"])
+        draft = self.eng.draft
+        draft[:, 0] = st["start"]                                                  # short matches verify the start token only
+        pos = cache.cache_len.long()[:, None] + self._ar[None, :]
+        logits = self.lm(input_ids=draft.long(), position_ids=pos, past_key_values=cache,
+                         attention_mask=self._mask(T, kv_len, cache.cache_len)).logits
+        return self.ver.verify(logits.contiguous(), draft, None, cache_len=cache.cache_len, out=st["res"])
+
     # ---- one decode step, entirely on the device (no host read anywhere: it is what gets captured in a CUDA graph) ----
     def _step_body(self, kv_len: int, max_new_tokens: int):
         st, T = self._st, self.T
         cache = self.cache
         # a request whose step could run past the cache is finished (samd_model.py:251-254)
         st["done"].logical_or_(cache.cache_len + T > cache.max_len)
-        self.eng.step(st["acc_tokens"], st["acc_count"], st["start"])              # update(accepted) + lookup(start): one launch
-        cache.begin(T, kv_len)
         saved_len = cache.cache_len.clone()
-        if self.tree is None:
-            draft = self.eng.draft
-            draft[:, 0] = st["start"]                                              # short matches verify the start token only
-            pos = cache.cache_len.long()[:, None] + self._ar[None, :]
-            logits = self.lm(input_ids=draft.long(), position_ids=pos, past_key_values=cache,
-                             attention_mask=self._mask(T, kv_len, cache.cache_len)).logits
-            res = self.ver.verify(logits.contiguous(), draft, None, cache_len=cache.cache_len, out=st["res"])
-        else:
-            res = self._tree_step(st["start"], kv_len, st["res"])
-        st["res"] = res
+        res = st["res"] = self._draft_forward_verify(kv_len)
+        self._commit(res, saved_len, max_new_tokens)
+
+    def _commit(self, res: dict, saved_len: torch.Tensor, max_new_tokens: int):
+        """EOS truncation, emission, cache lengths, the next step's inputs, history and the host flag."""
+        st, cache = self._st, self.cache
         done = st["done"]
         n_acc = torch.where(done, torch.zeros_like(res["accept_len"]), res["accept_len"])
         ar = self._ar[:res["tokens"].shape[1]]
@@ -227,6 +240,20 @@ class BatchedSamdDecoder:
         # what the host reads every `check_every` steps: [all finished?, longest cache]
         st["flag"][0] = done.all().to(torch.int32)
         st["flag"][1] = cache.cache_len.max()
+
+    def _prefill_hook(self, ids: torch.Tensor, lens: torch.Tensor, logits: torch.Tensor):
+        """After the prompt's forward and automaton update: TokenRecycle.update over the prompt rows (tree mode)."""
+        if self.tree is not None:
+            n_max = ids.shape[1]
+            valid = torch.arange(n_max, device=ids.device)[None, :] < lens[:, None]
+            self.table.update(ids[valid].to(torch.int32), logits[valid])
+            if not self.ver_bound:
+                self.ver.bind_kv([self.cache.kv[i] for i in range(self.cache.kv.shape[0])])
+                self.ver_bound = True
+
+    def _extra_state(self, mk) -> dict:
+        """Step state of a subclass, kept with the rest (persistent, snapshotted around a capture, zeroed per call)."""
+        return {}
 
     @torch.inference_mode()
     def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4):
@@ -258,12 +285,7 @@ class BatchedSamdDecoder:
                          attention_mask=self._mask(n_max, n_max, torch.zeros(B, dtype=torch.int32, device=dev))).logits
         self.cache.cache_len.copy_(lens)
         self.eng.step(ids.to(torch.int32).contiguous(), lens, None)                # DraftModel.update(prompt), ragged counts
-        if self.tree is not None:                                                  # TokenRecycle.update over the prompt rows
-            valid = torch.arange(n_max, device=dev)[None, :] < lens[:, None]
-            self.table.update(ids[valid].to(torch.int32), logits[valid])
-            if not self.ver_bound:
-                self.ver.bind_kv([self.cache.kv[i] for i in range(self.cache.kv.shape[0])])
-                self.ver_bound = True
+        self._prefill_hook(ids, lens, logits)
         max_steps = max_new_tokens + check_every + 1
         width = T if self.tree is None else self._ret.shape[2]
         first_tok = logits[torch.arange(B, device=dev), lens.long() - 1].argmax(-1).to(torch.int32)
@@ -273,11 +295,12 @@ class BatchedSamdDecoder:
             mk = lambda *sh: torch.zeros(*sh, dtype=torch.int32, device=dev)
             self._st = dict(start=mk(B), acc_tokens=mk(B, width), acc_count=mk(B), out=mk(B, max_new_tokens + T), out_len=mk(B),
                             done=torch.zeros(B, dtype=torch.bool, device=dev), hist=mk(max_steps, B),
-                            step=torch.zeros(1, dtype=torch.long, device=dev), flag=mk(2), res=None)
+                            step=torch.zeros(1, dtype=torch.long, device=dev), flag=mk(2), res=None, **self._extra_state(mk))
             self._st_key, self._graphs = key, {}
         else:
-            for k in ("acc_tokens", "acc_count", "out", "out_len", "done", "hist", "step", "flag"):
-                self._st[k].zero_()
+            for k, v in self._st.items():
+                if k not in ("start", "res"):
+                    v.zero_()
         self._st["start"].copy_(first_tok)
         flag_host = torch.zeros(2, dtype=torch.int32).pin_memory()
         # ---- decode ---------------------------------------------------------------------------
@@ -350,3 +373,81 @@ class BatchedSamdDecoder:
         return ([rows[b][:lens_out[b]] for b in range(B)],
                 dict(steps=n_live, steps_run=steps, host_syncs=syncs, graphed=self.last_graphed, graphs=len(graphs),
                      accept_lengths=[h[:n_live] for h in hist]))
+
+
+class BatchedSamOnlyDecoder(BatchedSamdDecoder):
+    """Batched decoding with the `samd_sam_only` flavour (samd_sam_only/samd_model.py:117-157 for B requests in lockstep):
+    every request drafts either a dynamic-automaton sequence of min(max_predicts, 1 + int(match * alpha)) tokens or, when
+    a static automaton built with counts is bound and wins by more than `len_bias`, the static SAM's best-first tree of up
+    to max_predicts nodes (K children per level).  One step, all on the device:
+
+        samd_step              update(accepted) + lookup(start): per-request type, draft, draft_len
+        samd_static_tree_draft the trees of the requests typed DRAFT_STATIC_TREE (static automaton only)
+        samd_draft_assemble    uniform [B, T] tokens / position ids, [B, T, kv_len] additive mask, [B, P, D] path table,
+                               node and path counts; finished requests get a one-node draft with no path
+        LM forward             position_ids and attention_mask = mask[:, None]
+        samd_verify_compact    accept lengths, accepted tokens, next tokens, the accepted KV rows moved into place
+
+    T = P = D = max_predicts.  The rest of the loop (prefill, one CUDA graph per key-length bucket, the commit, one host
+    read per `check_every` steps) is BatchedSamdDecoder's.  stats["tree_steps"] counts the request-steps of live requests
+    that drafted a static tree.
+
+    Known corner, inherited from the reference (SURVEY Appendix A9): a -1 pad column of a path selects token 0, so it is
+    "accepted" when the compared row's argmax is token 0, and the KV move then copies row cache_len - 1.  The batched path
+    table is D wide while a reference tree is only as wide as its own deepest path (and a reference sequence as long as
+    its draft), so here pads beyond a request's own width can be compared too - only after every real node of the path
+    was accepted, i.e. when the LM's greedy next token is 0."""
+
+    def __init__(self, lm, batch: int, max_cache_len: int, max_predicts: int = 40, alpha: float = 4.0, K: int = 8,
+                 len_bias: int = 5, static: Optional[E.StaticSamDevice] = None, eos_token_id: Optional[int] = None,
+                 max_tokens: int = 16384, dtype=torch.float16, device="cuda"):
+        if static is not None and not static.with_counts:
+            raise _cabi.SamdError("BatchedSamOnlyDecoder: the static automaton must be built with_counts=True "
+                                  "(the sam_only tree drafter reads its occurrence counts and top-8 successors)")
+        if not 1 <= max_predicts <= 128:
+            raise _cabi.SamdError(f"BatchedSamOnlyDecoder: max_predicts must be in [1, 128], got {max_predicts}")
+        self.lm, self.B, self.T = lm, batch, max_predicts
+        self.device, self.dtype, self.eos = torch.device(device), dtype, eos_token_id
+        self.tree, self.K_top = None, int(K)
+        self.cache = RaggedKVCache(lm.config, batch, max_cache_len, dtype, self.device)
+        self.dyn = E.DynSamBatch(batch, max_tokens, self.device)
+        self.eng = E.DraftEngine(self.dyn, static, _cabi.FLAVOUR_SAM_ONLY, n_predicts=max_predicts, len_bias=len_bias,
+                                 alpha=alpha)
+        self.ver = E.Verifier(batch, max_predicts, self.device)
+        self.ver.bind_kv([self.cache.kv[i] for i in range(self.cache.kv.shape[0])])
+        self._ar = torch.arange(max_predicts, device=self.device)
+        # the assembled buffers persist: the captured graphs refer to them.  The mask of a kv_len bucket is the leading
+        # [B, T, kv_len] block of one flat allocation sized for the whole cache.
+        T, dev = max_predicts, self.device
+        mk = lambda *s: torch.zeros(*s, dtype=torch.int32, device=dev)
+        self.buf = dict(tokens=mk(batch, T), position_ids=torch.zeros(batch, T, dtype=torch.long, device=dev),
+                        n_nodes=mk(batch), n_paths=mk(batch), retrieve=mk(batch, T, T),
+                        mask=torch.zeros(batch * T * max_cache_len, dtype=dtype, device=dev))
+
+    def _extra_state(self, mk) -> dict:
+        return dict(tree_steps=torch.zeros(1, dtype=torch.long, device=self.device))
+
+    def mask_view(self, kv_len: int) -> torch.Tensor:
+        return self.buf["mask"][:self.B * self.T * kv_len].view(self.B, self.T, kv_len)
+
+    def _draft_forward_verify(self, kv_len: int) -> dict:
+        st, T, cache, eng, buf = self._st, self.T, self.cache, self.eng, self.buf
+        eng.step(st["acc_tokens"], st["acc_count"], st["start"])
+        if eng.static is not None:
+            eng.tree_draft(st["start"], K_top=self.K_top)
+        st["tree_steps"].add_(((eng.out_type == _cabi.DRAFT_STATIC_TREE) & ~st["done"]).sum())
+        mask = self.mask_view(kv_len)
+        eng.assemble(cache.cache_len, buf["tokens"], buf["position_ids"], buf["n_nodes"], buf["n_paths"], buf["retrieve"],
+                     mask, done=st["done"])
+        cache.begin(T, kv_len)
+        logits = self.lm(input_ids=buf["tokens"].long(), position_ids=buf["position_ids"], past_key_values=cache,
+                         attention_mask=mask[:, None]).logits
+        return self.ver.verify(logits.contiguous(), buf["tokens"], buf["retrieve"], cache_len=cache.cache_len, move_kv=True,
+                               n_nodes=buf["n_nodes"], n_paths=buf["n_paths"], out=st["res"])
+
+    @torch.inference_mode()
+    def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4):
+        """BatchedSamdDecoder.generate; stats also carry "tree_steps"."""
+        out, stats = super().generate(prompts, max_new_tokens, graph=graph, check_every=check_every)
+        stats["tree_steps"] = int(self._st["tree_steps"].item())
+        return out, stats

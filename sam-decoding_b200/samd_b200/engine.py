@@ -440,6 +440,44 @@ class DraftEngine:
                 self.tree_retrieve.data_ptr(), self.tree_retrieve.shape[1], self.tree_retrieve.shape[2],
                 self.tree_shape.data_ptr(), K.stream_ptr()), "samd_static_tree_draft")
 
+    _MASK_DTYPES = {torch.bfloat16: K.DTYPE_BF16, torch.float16: K.DTYPE_FP16, torch.float32: K.DTYPE_FP32}
+
+    def assemble(self, cache_len: torch.Tensor, tokens: torch.Tensor, position_ids: torch.Tensor, n_nodes: torch.Tensor,
+                 n_paths: torch.Tensor, retrieve: torch.Tensor, mask: torch.Tensor, done: Optional[torch.Tensor] = None):
+        """samd_draft_assemble: the last step()'s sequence drafts and, for the requests typed DRAFT_STATIC_TREE, the last
+        tree_draft()'s trees, as uniform batch buffers written into the caller's tensors (persistent ones when the call
+        is captured in a graph): tokens [B, T] int32, position_ids [B, T] int64, n_nodes / n_paths [B] int32, retrieve
+        [B, P, D] int32 and the additive mask [B, T, kv_len] in the LM dtype.  `done` [B] bool / uint8: finished
+        requests get a one-node draft with no path (no KV row moves in the verify launch)."""
+        B = self.dyn.n_requests
+        T, kv_len = tokens.shape[1], mask.shape[2]
+        for t in (tokens, n_nodes, n_paths, retrieve, cache_len):
+            _i32(t)
+        assert tokens.shape == (B, T) and position_ids.shape == (B, T) and position_ids.dtype == torch.int64
+        assert position_ids.is_contiguous() and n_nodes.numel() == B and n_paths.numel() == B and cache_len.numel() == B
+        assert retrieve.dim() == 3 and retrieve.shape[0] == B and mask.dim() == 3 and mask.shape[:2] == (B, T)
+        assert mask.is_cuda and mask.is_contiguous()
+        dt = self._MASK_DTYPES.get(mask.dtype)
+        if dt is None:
+            raise K.SamdError(f"unsupported mask dtype {mask.dtype} (bf16 / fp16 / fp32)")
+        if done is not None:
+            assert done.dtype in (torch.bool, torch.uint8) and done.is_cuda and done.is_contiguous() and done.numel() == B
+        a = K.AssembleArgs()
+        a.batch, a.n_nodes, a.n_paths, a.depth = B, T, retrieve.shape[1], retrieve.shape[2]
+        a.type_dev, a.draft_dev, a.draft_stride = self.out_type.data_ptr(), self.draft.data_ptr(), self.n_predicts
+        a.draft_len_dev = self.draft_len.data_ptr()
+        if hasattr(self, "tree_tokens"):
+            a.tree_tokens_dev, a.tree_parents_dev = self.tree_tokens.data_ptr(), self.tree_parents.data_ptr()
+            a.tree_depth_dev, a.tree_stride, a.tree_n_dev = self.tree_depth.data_ptr(), self.n_predicts, self.tree_n.data_ptr()
+            a.tree_retrieve_dev, a.tree_shape_dev = self.tree_retrieve.data_ptr(), self.tree_shape.data_ptr()
+            a.tree_max_paths, a.tree_max_depth = self.tree_retrieve.shape[1], self.tree_retrieve.shape[2]
+        a.cache_len_dev, a.done_dev, a.mask_dtype, a.kv_len = cache_len.data_ptr(), K.ptr(done), dt, kv_len
+        a.out_tokens_dev, a.out_position_ids_dev = tokens.data_ptr(), position_ids.data_ptr()
+        a.out_n_nodes_dev, a.out_n_paths_dev = n_nodes.data_ptr(), n_paths.data_ptr()
+        a.out_retrieve_dev, a.out_mask_dev = retrieve.data_ptr(), mask.data_ptr()
+        with torch.cuda.device(self.dyn.device):
+            K.check(K.lib().samd_draft_assemble(C.byref(a), K.stream_ptr()), "samd_draft_assemble")
+
 
 class Verifier:
     """Fused greedy verification + KV compaction (samd/utils.py:127-141, samd/samd_model.py:159-211,
