@@ -67,6 +67,17 @@ int samd_dyn_reset(samd_dyn_t h, const uint8_t *mask_dev, void *stream);
 int64_t samd_dyn_bytes(samd_dyn_t h);
 /* Snapshot / restore: copy every arena of `src` into `dst` (same n_requests, max_tokens). */
 int samd_dyn_copy(samd_dyn_t dst, samd_dyn_t src, void *stream);
+/* Per-request copy, for prefix reuse: the automaton of P + S is the automaton of P extended by S (the online
+ * construction of dyn_sam.py:41-67 is deterministic), so a request whose prompt starts with a registered P starts from a
+ * copy of P's automaton.  For each pair i, request dst_idx_dev[i] of `dst` becomes an exact copy of request
+ * src_idx_dev[i] of `src`: state records, overflow table, token history and the 16 meta words (cursor included).  Both
+ * handles must have the same max_tokens (equal record, overflow-table and history capacities: nothing is re-hashed).
+ * The arena invariants hold afterwards: the source's live records are copied and the EMPTY TEMPLATE is written over the
+ * destination's records beyond them, up to its own former n_states - the traffic follows the live sizes, plus the whole
+ * overflow table.  dst_idx_dev entries must be distinct, and none may name a request of `src` that another pair writes.
+ * One launch; the arguments do not depend on the step. */
+int samd_dyn_clone(samd_dyn_t dst, const int32_t *dst_idx_dev, samd_dyn_t src, const int32_t *src_idx_dev,
+                   int32_t n_pairs, void *stream);
 /* Capacity growth: a new batch with max_tokens = new_max_tokens holding the same automata (state
  * numbering, cursors and histories preserved; the edge tables are re-hashed).  Synchronises; the
  * old handle stays valid and must still be destroyed by the caller. */
@@ -421,6 +432,17 @@ void samd_verify_set_debug_times(uint64_t *times_dev);
 int samd_kv_compact(void *const *kv_ptrs_dev, int32_t n_kv, int32_t n_heads, int32_t row_bytes, int64_t kv_batch_stride,
                     int64_t kv_head_stride, int64_t kv_pos_stride, const int32_t *indices_dev, int32_t depth,
                     const int32_t *accept_len_dev, int32_t *cache_len_dev, int32_t batch, void *stream);
+/* Prefix reuse at admission (the prefill a causal LM would repeat: KV row i depends only on tokens 0..i; the rows that
+ * samd/cache.py:SamdStaticCache holds for one request): for each pair i, rows [0, n_rows_dev[i]) of batch row
+ * src_row_dev[i] of the source cache are copied into batch row dst_row_dev[i] of the destination, in every one of the n_kv
+ * tensors and every head.  Each side is described like samd_kv_compact's KV (a device table of n_kv base pointers, byte
+ * strides), with its own strides: the two caches may differ in batch size and length.  n_rows 0 is allowed; nothing
+ * outside the listed rows is written.  16-byte accesses where row_bytes and the alignment allow, narrower ones
+ * otherwise.  One launch; the arguments do not depend on the step. */
+int samd_kv_copy_rows(void *const *dst_ptrs_dev, int64_t dst_batch_stride, int64_t dst_head_stride, int64_t dst_pos_stride,
+                      void *const *src_ptrs_dev, int64_t src_batch_stride, int64_t src_head_stride, int64_t src_pos_stride,
+                      int32_t n_kv, int32_t n_heads, int32_t row_bytes, const int32_t *dst_row_dev,
+                      const int32_t *src_row_dev, const int32_t *n_rows_dev, int32_t n_pairs, void *stream);
 /* profiling aid: n_warps warps each chase `hops` dependent pointers through n_records 64-byte records
  * (record word 0 = next index); measures dependent-load latency at the step kernel's concurrency */
 int samd_debug_pointer_chase(const void *recs_dev, int64_t n_records, int n_warps, int hops, int32_t *sink_dev, void *stream);

@@ -5,6 +5,7 @@
 #include "sam_scalar.cuh"
 #include "../../include/samd_b200.h"
 
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -56,6 +57,8 @@ extern "C" int samd_dyn_create(int n_requests, int max_tokens, samd_dyn_t *out) 
     SAMD_CUDA(cudaMalloc(&a.slots, b_slots));
     SAMD_CUDA(cudaMalloc(&a.text, b_text));
     SAMD_CUDA(cudaMalloc(&a.meta, b_meta));
+    SAMD_CUDA(cudaMalloc(&h->tickets, (size_t)n_requests * sizeof(int32_t)));
+    SAMD_CUDA(cudaMemset(h->tickets, 0, (size_t)n_requests * sizeof(int32_t)));
     h->bytes = (int64_t)(b_recs + b_slots + b_text + b_meta);
     *out = h;
     // the arenas are filled on the default stream; the caller's first launch may come on any other (non-blocking) stream
@@ -71,6 +74,7 @@ extern "C" int samd_dyn_destroy(samd_dyn_t h) {
     cudaFree(h->a.slots);
     cudaFree(h->a.text);
     cudaFree(h->a.meta);
+    cudaFree(h->tickets);
     delete h;
     return 0;
 }
@@ -87,6 +91,77 @@ extern "C" int samd_dyn_copy(samd_dyn_t dst, samd_dyn_t src, void *stream) {
     SAMD_CUDA(cudaMemcpyAsync(d.slots, s.slots, (size_t)s.n_requests * s.h_cap * sizeof(uint4), cudaMemcpyDeviceToDevice, st));
     SAMD_CUDA(cudaMemcpyAsync(d.text, s.text, (size_t)s.n_requests * s.t_cap * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
     SAMD_CUDA(cudaMemcpyAsync(d.meta, s.meta, (size_t)s.n_requests * META_WORDS * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
+#define CLONE_THREADS 256
+// One request of `s` onto one request of `d` (same s_cap / h_cap / t_cap): blockIdx.y = pair, gridDim.x CTAs share its
+// 16-byte units - the live records [0, n_src), the EMPTY TEMPLATE over the destination's stale records [n_src, n_dst_old),
+// the whole overflow table (hashed: no live prefix to follow) and text[0 .. max_length].  Every CTA reads n_dst_old from
+// the destination's meta before it counts itself in on tickets[dst]; the last CTA to arrive - the others have all read it
+// by then - writes the 16 meta words and clears the ticket for the next launch.
+__global__ void __launch_bounds__(CLONE_THREADS) dyn_clone_kernel(DynArena d, const int32_t *dst_idx, DynArena s,
+                                                                  const int32_t *src_idx, int32_t *tickets) {
+    __shared__ int sh_old, sh_last;
+    const int rd = dst_idx[blockIdx.y], rs = src_idx[blockIdx.y];
+    if (rd < 0 || rd >= d.n_requests || rs < 0 || rs >= s.n_requests || (d.recs == s.recs && rd == rs)) return;
+    const int32_t *sm = s.meta + (size_t)rs * META_WORDS;
+    int32_t *dm = d.meta + (size_t)rd * META_WORDS;
+    if (threadIdx.x == 0) {
+        sh_old = dm[META_NSTATES];
+        __threadfence();
+        sh_last = atomicAdd(&tickets[rd], 1) == (int)gridDim.x - 1;
+    }
+    __syncthreads();
+    const long long n_src = sm[META_NSTATES], n_old = sh_old;
+    const long long u_rec = 4 * (n_src > n_old ? n_src : n_old);         // records: 4 units of 16 B each
+    const long long u_tab = d.h_cap;
+    const long long u_txt = ((long long)sm[META_N] + 1 + 3) >> 2;          // text[0 .. max_length], t_cap is a multiple of 4
+    const int4 *srec = reinterpret_cast<const int4 *>(s.recs + (size_t)rs * s.s_cap * SAMD_REC);
+    int4 *drec = reinterpret_cast<int4 *>(d.recs + (size_t)rd * d.s_cap * SAMD_REC);
+    const uint4 *stab = s.slots + (size_t)rs * s.h_cap;
+    uint4 *dtab = d.slots + (size_t)rd * d.h_cap;
+    const int4 *stxt = reinterpret_cast<const int4 *>(s.text + (size_t)rs * s.t_cap);
+    int4 *dtxt = reinterpret_cast<int4 *>(d.text + (size_t)rd * d.t_cap);
+    const long long total = u_rec + u_tab + u_txt, stride = (long long)gridDim.x * CLONE_THREADS;
+    for (long long u = (long long)blockIdx.x * CLONE_THREADS + threadIdx.x; u < total; u += stride) {
+        if (u < u_rec) {
+            if (u < 4 * n_src) {
+                drec[u] = __ldg(srec + u);
+            } else {                                                     // the template of dyn_reset_kernel
+                const int q = (int)(u & 3);
+                drec[u] = q == 0 ? make_int4(-1, 0, 0, -1) : q == 1 ? make_int4(-1, -1, -1, -1) : q == 2 ? make_int4(-1, 0, 0, 0) : make_int4(0, 0, -1, 0);
+            }
+        } else if (u < u_rec + u_tab) {
+            dtab[u - u_rec] = __ldg(stab + (u - u_rec));
+        } else {
+            dtxt[u - u_rec - u_tab] = __ldg(stxt + (u - u_rec - u_tab));
+        }
+    }
+    if (sh_last && threadIdx.x < META_WORDS) {
+        dm[threadIdx.x] = sm[threadIdx.x];
+        if (threadIdx.x == 0) tickets[rd] = 0;
+    }
+}
+
+extern "C" int samd_dyn_clone(samd_dyn_t dst, const int32_t *dst_idx_dev, samd_dyn_t src, const int32_t *src_idx_dev,
+                              int32_t n_pairs, void *stream) {
+    SAMD_REQUIRE(dst && src && n_pairs >= 0, "samd_dyn_clone: bad arguments");
+    if (dst->a.max_tokens != src->a.max_tokens) {
+        samd_set_error("samd_dyn_clone: max_tokens differ (dst %d, src %d): the record, overflow-table and history "
+                       "capacities must agree", dst->a.max_tokens, src->a.max_tokens);
+        return 2;
+    }
+    if (n_pairs == 0) return 0;
+    SAMD_REQUIRE(dst_idx_dev && src_idx_dev, "samd_dyn_clone: null index array");
+    SAMD_REQUIRE(n_pairs <= 65535, "samd_dyn_clone: at most 65535 pairs per launch");
+    // CTAs per pair from the capacity alone (about 16 units per thread at a full arena): no argument depends on the step
+    const long long units = 4LL * dst->a.s_cap + dst->a.h_cap;
+    const unsigned per_pair = (unsigned)std::max(4LL, std::min(64LL, units / (CLONE_THREADS * 16)));
+    dyn_clone_kernel<<<dim3(per_pair, (unsigned)n_pairs), CLONE_THREADS, 0, (cudaStream_t)stream>>>(
+        dst->a, dst_idx_dev, src->a, src_idx_dev, dst->tickets);
+    samd_count_launch();
+    SAMD_CUDA(cudaGetLastError());
     return 0;
 }
 

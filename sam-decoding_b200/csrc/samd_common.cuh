@@ -103,6 +103,7 @@ struct samd_static_s {
 
 struct samd_dyn_s {
     DynArena a;
+    int32_t *tickets;   // [n_requests] arrival counters of samd_dyn_clone (0 between launches)
     int device;
     int64_t bytes;
 };

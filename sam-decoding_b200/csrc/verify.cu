@@ -1312,6 +1312,96 @@ extern "C" int samd_kv_compact(void *const *kv_ptrs_dev, int32_t n_kv, int32_t n
 }
 
 // ---------------------------------------------------------------------------------------
+// Prefix rows from one KV cache into another (prefix reuse at admission): pair i copies rows [0, n_rows[i]) of batch row
+// src_row[i] into batch row dst_row[i], every tensor and head.  blockIdx.y = pair; its rows are cut into 16-byte chunks
+// (consecutive threads -> consecutive chunks of one row, so a head's rows stream contiguously) and every lane keeps
+// CP_UNROLL chunks in flight.  A chunk whose two addresses are 16-byte aligned and that lies inside the row moves as one
+// uint4; the row's partial last chunk, or any chunk of a row that is not 16-byte aligned, moves in the widest of 4 / 2 / 1
+// bytes both addresses allow.
+// ---------------------------------------------------------------------------------------
+#define CP_THREADS 256
+#define CP_UNROLL 4
+
+struct KvSide {
+    void *const *ptrs;
+    long long batch_stride, head_stride, pos_stride;
+};
+
+__device__ __forceinline__ void copy_bytes(char *d, const char *s, int n) {
+    const unsigned a = (unsigned)(((uintptr_t)d | (uintptr_t)s) & 3) | (unsigned)(n & 3);
+    if (a == 0) {
+        for (int k = 0; k < n; k += 4) *reinterpret_cast<uint32_t *>(d + k) = *reinterpret_cast<const uint32_t *>(s + k);
+    } else if ((a & 1) == 0) {
+        for (int k = 0; k < n; k += 2) *reinterpret_cast<uint16_t *>(d + k) = *reinterpret_cast<const uint16_t *>(s + k);
+    } else {
+        for (int k = 0; k < n; ++k) d[k] = s[k];
+    }
+}
+
+__global__ void __launch_bounds__(CP_THREADS) kv_copy_rows_kernel(KvSide dst, KvSide src, int n_kv, int n_heads, int row_bytes,
+                                                                  const int32_t *dst_row, const int32_t *src_row,
+                                                                  const int32_t *n_rows) {
+    const int p = blockIdx.y;
+    const long long rows = n_rows[p];
+    if (rows <= 0) return;
+    const int cols = (row_bytes + 15) >> 4;
+    const long long total = (long long)n_kv * n_heads * rows * cols;
+    const long long db = (long long)dst_row[p] * dst.batch_stride, sb = (long long)src_row[p] * src.batch_stride;
+    const long long stride = (long long)gridDim.x * CP_THREADS;
+    for (long long u0 = (long long)blockIdx.x * CP_THREADS + threadIdx.x; u0 < total; u0 += stride * CP_UNROLL) {
+        char *dp[CP_UNROLL];
+        const char *sp[CP_UNROLL];
+        int nb[CP_UNROLL];
+        uint4 v[CP_UNROLL];
+#pragma unroll
+        for (int k = 0; k < CP_UNROLL; ++k) {
+            const long long u = u0 + k * stride;
+            nb[k] = 0;
+            if (u >= total) continue;
+            const int col = (int)(u % cols);
+            long long rest = u / cols;
+            const long long row = rest % rows;
+            rest /= rows;
+            const int hd = (int)(rest % n_heads), kv = (int)(rest / n_heads);
+            const long long off = (long long)col << 4;
+            dp[k] = reinterpret_cast<char *>(dst.ptrs[kv]) + db + hd * dst.head_stride + row * dst.pos_stride + off;
+            sp[k] = reinterpret_cast<const char *>(src.ptrs[kv]) + sb + hd * src.head_stride + row * src.pos_stride + off;
+            nb[k] = min(16, row_bytes - (int)off);
+            if (nb[k] == 16 && (((uintptr_t)dp[k] | (uintptr_t)sp[k]) & 15) == 0) {
+                v[k] = *reinterpret_cast<const uint4 *>(sp[k]);
+                nb[k] = -16;                                             // vector chunk, loaded
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < CP_UNROLL; ++k) {
+            if (nb[k] == -16) *reinterpret_cast<uint4 *>(dp[k]) = v[k];
+            else if (nb[k] > 0) copy_bytes(dp[k], sp[k], nb[k]);
+        }
+    }
+}
+
+extern "C" int samd_kv_copy_rows(void *const *dst_ptrs_dev, int64_t dst_batch_stride, int64_t dst_head_stride,
+                                 int64_t dst_pos_stride, void *const *src_ptrs_dev, int64_t src_batch_stride,
+                                 int64_t src_head_stride, int64_t src_pos_stride, int32_t n_kv, int32_t n_heads,
+                                 int32_t row_bytes, const int32_t *dst_row_dev, const int32_t *src_row_dev,
+                                 const int32_t *n_rows_dev, int32_t n_pairs, void *stream) {
+    SAMD_REQUIRE(n_pairs >= 0 && n_pairs <= 65535, "samd_kv_copy_rows: n_pairs must be in [0, 65535]");
+    if (n_pairs == 0) return 0;
+    SAMD_REQUIRE(dst_ptrs_dev && src_ptrs_dev && dst_row_dev && src_row_dev && n_rows_dev,
+                 "samd_kv_copy_rows: null pointer argument");
+    SAMD_REQUIRE(n_kv > 0 && n_heads > 0 && row_bytes > 0, "samd_kv_copy_rows: bad KV shape");
+    // about eight CTAs per SM in all, whatever the pair count: the grid depends on n_pairs only
+    const unsigned per_pair = (unsigned)std::min(1024, std::max(8, (148 * 8 + n_pairs - 1) / n_pairs));
+    const KvSide d{dst_ptrs_dev, dst_batch_stride, dst_head_stride, dst_pos_stride};
+    const KvSide s{src_ptrs_dev, src_batch_stride, src_head_stride, src_pos_stride};
+    kv_copy_rows_kernel<<<dim3(per_pair, (unsigned)n_pairs), CP_THREADS, 0, (cudaStream_t)stream>>>(
+        d, s, n_kv, n_heads, row_bytes, dst_row_dev, src_row_dev, n_rows_dev);
+    samd_count_launch();
+    SAMD_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------
 // TokenRecycle.gen_draft (samd/tree_model/token_recycle/token_recycle.py:49-59): one warp per request fills the
 // static tree level by level from the [vocab][8] successor table (a node's token is known once its parent's is).
 // ---------------------------------------------------------------------------------------

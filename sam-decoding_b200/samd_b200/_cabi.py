@@ -85,6 +85,7 @@ SYMBOLS = {
     "samd_dyn_reset": (C.c_int, [vp, vp, vp]),
     "samd_dyn_bytes": (C.c_int64, [vp]),
     "samd_dyn_copy": (C.c_int, [vp, vp, vp]),
+    "samd_dyn_clone": (C.c_int, [vp, vp, vp, vp, C.c_int32, vp]),
     "samd_dyn_grow": (C.c_int, [vp, C.c_int, C.POINTER(vp)]),
     "samd_dyn_stats": (C.c_int, [vp, c_i64p]),
     "samd_dyn_meta": (C.c_int, [vp, c_i32p]),
@@ -134,6 +135,8 @@ SYMBOLS = {
     "samd_dyn_transfer": (C.c_int, [vp, vp, C.c_int32, vp, vp]),
     "samd_kv_compact": (C.c_int, [vp, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int64, vp, C.c_int32,
                                   vp, vp, C.c_int32, vp]),
+    "samd_kv_copy_rows": (C.c_int, [vp, C.c_int64, C.c_int64, C.c_int64, vp, C.c_int64, C.c_int64, C.c_int64, C.c_int32,
+                                    C.c_int32, C.c_int32, vp, vp, vp, C.c_int32, vp]),
     "samd_debug_pointer_chase": (C.c_int, [vp, C.c_int64, C.c_int, C.c_int, vp, vp]),
     "samd_verify_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(vp)]),
     "samd_verify_destroy": (C.c_int, [vp]),

@@ -26,6 +26,8 @@ generate() decodes exactly B prompts in lockstep.  serve() is continuous batchin
 requests, each admitted into a slot as soon as the host sees that slot's request finished (prefill of the admitted
 prompts alone, masked drafter reset, prompt ingestion with count 0 for every other request, the slot's state written in
 place), so the graphs captured per key-length bucket stay valid and nothing waits for the longest request of a batch.
+With a prefix pool (max_prefixes > 0, add_prefix) an admitted request whose prompt starts with a registered prefix copies
+that prefix's KV rows, automaton and static cursor and prefills / ingests only the rest of its prompt.
 """
 from __future__ import annotations
 
@@ -85,10 +87,11 @@ class RaggedKVCache(Cache):
         self._bidx = torch.arange(batch, device=device)[:, None]
         self._slots = None              # [n, 1] requests of a sub-batch forward (begin(slots=...)), None = the whole batch
 
-    def begin(self, n_new: int, kv_len: int, slots: Optional[torch.Tensor] = None):
+    def begin(self, n_new: int, kv_len: int, slots: Optional[torch.Tensor] = None, base: Optional[torch.Tensor] = None):
         """Set up the next forward.  By default it carries every request and writes its new rows at cache_len[b] + t.
         With `slots` (int64 [n]) it carries only those requests, in that order - a prefill of newly admitted requests:
-        rows 0 .. n_new - 1 of those slots are written and attention reads those slots alone."""
+        rows 0 .. n_new - 1 of those slots are written and attention reads those slots alone; with `base` (int32 [n])
+        too, rows base[i] .. base[i] + n_new - 1 of slot i (the suffix of a prompt whose first base[i] rows are there)."""
         ar = torch.arange(n_new, device=self.kv.device)[None, :]
         if slots is None:
             # (clamped: a finished request still rides along in the batch; its rows may be written past its end, never
@@ -97,7 +100,10 @@ class RaggedKVCache(Cache):
             self.rows = (self.cache_len.long()[:, None] + ar).clamp_(max=self.max_len - 1)
         else:
             self._slots = slots[:, None]
-            self.rows = ar.expand(slots.numel(), -1)
+            if base is None:
+                self.rows = ar.expand(slots.numel(), -1)
+            else:                       # (a right-padded suffix's pad rows likewise: clamped, never past the cache)
+                self.rows = (base.long()[:, None] + ar).clamp_(max=self.max_len - 1)
         self.kv_len = kv_len
 
     def write(self, k, v, layer):
@@ -112,11 +118,29 @@ class RaggedKVCache(Cache):
     def get_seq_length(self, layer_idx=0):
         return 0
 
+    def kv_table(self) -> tuple:
+        """The 2L tensors as the C ABI sees them (engine.kv_table), built once."""
+        if getattr(self, "_kv_table", None) is None:
+            self._kv_table = E.kv_table([self.kv[i] for i in range(self.kv.shape[0])], self.kv.device)
+        return self._kv_table
+
 
 class BatchedSamdDecoder:
+    """Batched lossless speculative decoding with the samd flavour: B slots, generate() for exactly B prompts in
+    lockstep, serve() for any number of requests (continuous batching).
+
+    Prefix reuse (max_prefixes > 0): add_prefix(tokens) registers a prompt head - a system prompt, a few-shot block, a
+    document, an earlier chat turn - once, in a pool of max_prefixes entries: its KV rows (a RaggedKVCache of
+    max_prefixes rows), its automaton and static cursor (a DynSamBatch and DraftEngine of max_prefixes requests), its
+    greedy next token and, in Token-Recycle tree mode, the top-8 rows of its positions.  Every admission, in serve() and
+    generate(), then starts a request whose prompt begins with a registered prefix P (the longest such P; a prompt equal
+    to P included) from copies of that state - samd_kv_copy_rows for rows [0, len(P)), samd_dyn_clone for the automaton
+    - and runs only the rest of the prompt through the LM and the step kernel.  The outputs are the same as without the
+    pool.  With max_prefixes = 0 (the default) nothing is allocated and add_prefix raises."""
+
     def __init__(self, lm, batch: int, max_cache_len: int, n_predicts: int = 16, len_bias: int = 5, len_threshold: int = 5,
                  static: Optional[E.StaticSamDevice] = None, eos_token_id: Optional[int] = None, max_tokens: int = 16384,
-                 dtype=torch.float16, device="cuda", tree: Optional[List[List[int]]] = None):
+                 dtype=torch.float16, device="cuda", tree: Optional[List[List[int]]] = None, max_prefixes: int = 0):
         self.lm, self.B, self.T = lm, batch, n_predicts
         self.n_seq = n_predicts
         self.device, self.dtype, self.eos = torch.device(device), dtype, eos_token_id
@@ -129,6 +153,19 @@ class BatchedSamdDecoder:
             self._init_tree(tree)
         self.ver = E.Verifier(batch, self.T, self.device)
         self._ar = torch.arange(self.T, device=self.device)
+        self._init_pool(max_prefixes)
+
+    def _init_pool(self, max_prefixes: int):
+        """The prefix pool (nothing at all when max_prefixes is 0)."""
+        self._prefixes = self.pool = None
+        if max_prefixes > 0:
+            cache = RaggedKVCache(self.lm.config, max_prefixes, self.cache.max_len, self.dtype, self.device)
+            dyn = E.DynSamBatch(max_prefixes, self.dyn.max_tokens, self.device)
+            # ingestion only (no lookup); it has cursors on the decoder's static automaton
+            eng = E.DraftEngine(dyn, self.eng.static, self.eng.flavour, n_predicts=self.eng.n_predicts)
+            self.pool = dict(cache=cache, dyn=dyn, eng=eng)
+            self._prefixes = [None] * max_prefixes      # per pool row: dict(tokens, next, topk) or None
+            self._slot_plen = [0] * self.B
 
     def _init_tree(self, tree):
         """Per-type tables, selected per request each step: ancestor masks, depths, path tables."""
@@ -354,12 +391,84 @@ class BatchedSamdDecoder:
         self._step_body(kv_len)
         return False
 
+    # ---- prefix reuse: a pool of registered prompt heads --------------------------------------------------------------
+    @torch.inference_mode()
+    def add_prefix(self, tokens: Sequence[int]) -> int:
+        """Register a prompt head; returns its id (the id it already has when these tokens are registered).  The
+        prefix's LM prefill runs alone into a pool row, its automaton and static cursor ingest it, and its greedy next
+        token (and, in tree mode, the top-8 rows of its positions) are kept.  No slot and no captured graph is touched:
+        it may be called between calls and while a serve() generator is suspended."""
+        tokens = tuple(int(t) for t in tokens)
+        pid = self._check_prefix(tokens)
+        if self._prefixes[pid] is not None:
+            return pid
+        pool, dev, n = self.pool, self.device, len(tokens)
+        ids = torch.tensor([tokens], dtype=torch.long, device=dev)
+        slot = torch.tensor([pid], dtype=torch.long, device=dev)
+        logits = self._prefill_slots(ids, slot, cache=pool["cache"])
+        P = pool["dyn"].n_requests
+        eng = pool["eng"]
+        eng.reset(torch.zeros(P, dtype=torch.uint8, device=dev).index_fill_(0, slot, 1))
+        tok = torch.zeros(P, n, dtype=torch.int32, device=dev).index_copy_(0, slot, ids.to(torch.int32))
+        eng.step(tok, torch.zeros(P, dtype=torch.int32, device=dev).index_fill_(0, slot, n), None)
+        topk = self.table.topk(ids[0], logits[0]) if self.tree is not None else None
+        self._prefixes[pid] = dict(tokens=tokens, ids=ids[0], next=logits[0, n - 1].argmax(-1).to(torch.int32), topk=topk)
+        return pid
+
+    def drop_prefix(self, pid: int):
+        """Forget prefix `pid`: no admission matches it any more and its pool row is free."""
+        if self._prefixes is None or not 0 <= pid < len(self._prefixes) or self._prefixes[pid] is None:
+            raise K.SamdError(f"drop_prefix: no registered prefix {pid}")
+        self._prefixes[pid] = None
+
+    def _check_prefix(self, tokens: tuple) -> int:
+        """add_prefix's validation: the id of these tokens, or of the free pool row they would take."""
+        if getattr(self, "_prefixes", None) is None:
+            raise K.SamdError("add_prefix: this decoder has no prefix pool (construct it with max_prefixes > 0)")
+        n, T, max_len, cap = len(tokens), self.T, self.cache.max_len, self.dyn.max_tokens
+        if n == 0:
+            raise K.SamdError("add_prefix: empty prefix")
+        if n + T > max_len:
+            raise K.SamdError(f"add_prefix: prefix of {n} tokens + one decode step of {T} does not fit "
+                              f"max_cache_len={max_len}")
+        if n + 1 + T > cap:
+            raise K.SamdError(f"add_prefix: prefix of {n} tokens + one new token + one step exceeds the automaton "
+                              f"capacity max_tokens={cap}")
+        free = None
+        for pid, e in enumerate(self._prefixes):
+            if e is None:
+                free = pid if free is None else free
+            elif e["tokens"] == tokens:
+                return pid
+        if free is None:
+            raise K.SamdError(f"add_prefix: the prefix pool is full ({len(self._prefixes)} prefixes); drop_prefix one first")
+        return free
+
+    def _longest_prefix(self, prompt: Sequence[int]) -> tuple:
+        """(id, length) of the longest registered prefix P with prompt[:len(P)] == P, or (None, 0)."""
+        best, best_len = None, 0
+        for pid, e in enumerate(self._prefixes):
+            if e is None:
+                continue
+            P = e["tokens"]
+            n = len(P)
+            if best_len < n <= len(prompt) and prompt[n - 1] == P[-1] and prompt[0] == P[0] and tuple(prompt[:n]) == P:
+                best, best_len = pid, n
+        return best, best_len
+
     # ---- admission: new requests into free slots, between two steps ---------------------------------------------------
     def _admit(self, reqs: List[tuple]) -> int:
         """Start the requests `reqs` = [(slot, prompt, limit)] in their (free) slots; returns the longest prompt.  Only
         the persistent state is written, in place, so the captured graphs stay valid."""
         dev = self.device
         n_max = max(len(p) for _, p, _ in reqs)
+        if self._prefixes is not None:
+            hits = [self._longest_prefix(p) for _, p, _ in reqs]
+            for (b, _, _), (_, n) in zip(reqs, hits):
+                self._slot_plen[b] = n
+            if any(pid is not None for pid, _ in hits):
+                self._admit_prefixed(reqs, hits)
+                return n_max
         ids = torch.zeros(len(reqs), n_max, dtype=torch.long)
         for i, (_, p, _) in enumerate(reqs):
             ids[i, :len(p)] = torch.as_tensor(p, dtype=torch.long)
@@ -368,17 +477,114 @@ class BatchedSamdDecoder:
         slots, lens, limits = meta[0], meta[1].to(torch.int32), meta[2].to(torch.int32)
         logits = self._prefill_slots(ids, slots)
         self._ingest(ids, slots, lens, logits)
-        self._set_slots(slots, lens, limits, logits)
+        first = logits[torch.arange(slots.numel(), device=dev), lens.long() - 1].argmax(-1).to(torch.int32)
+        self._set_slots(slots, lens, limits, first)
         return n_max
 
-    def _prefill_slots(self, ids: torch.Tensor, slots: torch.Tensor) -> torch.Tensor:
+    def _admit_prefixed(self, reqs: List[tuple], hits: List[tuple]):
+        """_admit when some requests start with a registered prefix (pool row hits[i][0], length hits[i][1]; (None, 0)
+        for the others): their KV rows [0, len(P)) come from the pool (one samd_kv_copy_rows launch), one LM forward
+        runs over the suffixes alone (right padded, rows from len(P) on), the unmatched slots' drafters are reset and
+        the matched ones cloned from the pool (one samd_dyn_clone launch, static-cursor rows copied), and one samd_step
+        ingests the suffixes - count 0 for a prompt equal to its prefix, which starts from the prefix's next token."""
+        dev, pool = self.device, self.pool
+        n = len(reqs)
+        sufs = [p[m:] for (_, p, _), (_, m) in zip(reqs, hits)]
+        n_suf = max(len(x) for x in sufs)
+        hit = [i for i in range(n) if hits[i][0] is not None]
+        fw = [i for i in range(n) if len(sufs[i])]                                   # requests with a suffix
+        ids = torch.zeros(n, n_suf, dtype=torch.long)
+        for i, x in enumerate(sufs):
+            ids[i, :len(x)] = torch.as_tensor(x, dtype=torch.long)
+        meta = torch.tensor([[r[0] for r in reqs], [len(r[1]) for r in reqs], [r[2] for r in reqs], [m for _, m in hits],
+                             [len(x) for x in sufs], [-1 if pid is None else pid for pid, _ in hits]], dtype=torch.long)
+        ids, meta = ids.to(dev), meta.to(dev)
+        slots, lens, limits = meta[0], meta[1].to(torch.int32), meta[2].to(torch.int32)
+        base, suf_lens, pids = meta[3].to(torch.int32), meta[4].to(torch.int32), meta[5]
+        h = torch.tensor(hit, dtype=torch.long, device=dev)
+        h_slots, h_pids = slots[h], pids[h]
+        self._copy_prefix_kv(h_slots, h_pids, base[h])
+        logits = None
+        if fw:
+            f = torch.tensor(fw, dtype=torch.long, device=dev)
+            logits = self._prefill_slots(ids[f], slots[f], base=base[f], kv_len=max(hits[i][1] + len(sufs[i]) for i in fw))
+        self._clone_drafters(slots, pids, h_slots, h_pids)
+        self._ingest_suffixes(ids, slots, suf_lens, [(hits[i][0], len(sufs[i])) for i in range(n)], fw, logits)
+        self.prefix_hits += len(hit)
+        self.prefix_tokens += sum(hits[i][1] for i in hit)
+        # first start token: the greedy token after the last suffix row, or after the prefix itself
+        first = torch.zeros(n, dtype=torch.int32, device=dev)
+        if fw:
+            first[f] = logits[torch.arange(len(fw), device=dev), suf_lens[f].long() - 1].argmax(-1).to(torch.int32)
+        exact = [i for i in range(n) if not len(sufs[i])]
+        if exact:
+            first[torch.tensor(exact, device=dev)] = torch.stack([self._prefixes[hits[i][0]]["next"] for i in exact])
+        self._set_slots(slots, lens, limits, first)
+
+    def _copy_prefix_kv(self, slots: torch.Tensor, pids: torch.Tensor, plens: torch.Tensor):
+        """KV rows [0, plens[i]) of pool row pids[i] into slot slots[i]: one samd_kv_copy_rows launch."""
+        E.kv_copy_rows(self.cache.kv_table(), self.pool["cache"].kv_table(), slots.to(torch.int32),
+                       pids.to(torch.int32), plens.to(torch.int32))
+
+    def _clone_drafters(self, slots: torch.Tensor, pids: torch.Tensor, h_slots: torch.Tensor, h_pids: torch.Tensor):
+        """Masked DraftModel.reset of the unmatched slots; the matched ones take a copy of their prefix's automaton (one
+        samd_dyn_clone launch) and static cursor."""
+        B, dev, pool = self.B, self.device, self.pool
+        miss = slots[pids < 0]
+        if miss.numel():
+            self.eng.reset(torch.zeros(B, dtype=torch.uint8, device=dev).index_fill_(0, miss, 1))
+        self.dyn.clone_from(pool["dyn"], h_pids.to(torch.int32), h_slots.to(torch.int32))
+        if self.eng.static_cursor is not None:
+            self.eng.static_cursor.index_copy_(0, h_slots, pool["eng"].static_cursor.index_select(0, h_pids))
+
+    def _ingest_suffixes(self, ids: torch.Tensor, slots: torch.Tensor, suf_lens: torch.Tensor, parts: List[tuple],
+                         fw: List[int], logits: Optional[torch.Tensor]):
+        """DraftModel.update(suffix) of every admitted request in one launch (count 0 for every other slot), then in
+        tree mode the successor table as an uncached admission leaves it: per request in admission order, its prefix's
+        stored rows then its suffix rows, the last writer of a token winning (RecycleTable.apply)."""
+        B, dev = self.B, self.device
+        if ids.shape[1]:
+            tokens = torch.zeros(B, ids.shape[1], dtype=torch.int32, device=dev).index_copy_(0, slots, ids.to(torch.int32))
+            counts = torch.zeros(B, dtype=torch.int32, device=dev).index_copy_(0, slots, suf_lens)
+            self.eng.step(tokens, counts, None)
+        if self.tree is None:
+            return
+        rows_s = None
+        if fw:
+            f = torch.tensor(fw, dtype=torch.long, device=dev)
+            valid = torch.arange(ids.shape[1], device=dev)[None, :] < suf_lens[f][:, None]
+            rows_s = self.table.topk(ids[f][valid], logits[valid])
+        toks, rows, at = [], [], 0
+        for i, (pid, m) in enumerate(parts):                                         # admission order
+            if pid is not None:
+                e = self._prefixes[pid]
+                toks.append(e["ids"])
+                rows.append(e["topk"])
+            if m:
+                toks.append(ids[i, :m])
+                rows.append(rows_s[at:at + m])
+                at += m
+        self.table.apply(torch.cat(toks), torch.cat(rows))
+        if not self.ver_bound:
+            self.ver.bind_kv([self.cache.kv[i] for i in range(self.cache.kv.shape[0])])
+            self.ver_bound = True
+
+    def _prefill_slots(self, ids: torch.Tensor, slots: torch.Tensor, base: Optional[torch.Tensor] = None,
+                       kv_len: Optional[int] = None, cache: Optional[RaggedKVCache] = None) -> torch.Tensor:
         """LM prefill of the admitted prompts alone ([n, n_max], right padded) into KV rows 0 .. n_max - 1 of their
-        slots: the cost follows the admitted prompts, not the batch."""
+        slots: the cost follows the admitted prompts, not the batch.  With `base` (int32 [n]), the prompts are suffixes
+        whose first base[i] rows are in the cache: rows and positions start at base[i], attention spans kv_len keys.
+        `cache`: another cache than the decoder's (the prefix pool)."""
         n, n_max = ids.shape
-        self.cache.begin(n_max, n_max, slots=slots)
-        pos = torch.arange(n_max, device=self.device)[None, :].expand(n, -1)
-        return self.lm(input_ids=ids, position_ids=pos, past_key_values=self.cache,
-                       attention_mask=self._mask(n_max, n_max, torch.zeros(n, dtype=torch.int32, device=self.device))).logits
+        cache = self.cache if cache is None else cache
+        if base is None:
+            kv_len, base0 = n_max, torch.zeros(n, dtype=torch.int32, device=self.device)
+        else:
+            base0 = base
+        cache.begin(n_max, kv_len, slots=slots, base=base)
+        pos = base0.long()[:, None] + torch.arange(n_max, device=self.device)[None, :]
+        return self.lm(input_ids=ids, position_ids=pos, past_key_values=cache,
+                       attention_mask=self._mask(n_max, kv_len, base0)).logits
 
     def _ingest(self, ids: torch.Tensor, slots: torch.Tensor, lens: torch.Tensor, logits: torch.Tensor):
         """The admitted requests' drafters: masked DraftModel.reset (automaton and static cursor), then
@@ -390,11 +596,10 @@ class BatchedSamdDecoder:
         self.eng.step(tokens, counts, None)
         self._prefill_hook(ids, lens, logits)
 
-    def _set_slots(self, slots: torch.Tensor, lens: torch.Tensor, limits: torch.Tensor, logits: torch.Tensor):
+    def _set_slots(self, slots: torch.Tensor, lens: torch.Tensor, limits: torch.Tensor, first: torch.Tensor):
         """The admitted slots' step state: cache length, first start token (the prompt's greedy next token), limit, and
         zero emitted tokens / history."""
         st = self._st
-        first = logits[torch.arange(slots.numel(), device=self.device), lens.long() - 1].argmax(-1).to(torch.int32)
         self.cache.cache_len.index_copy_(0, slots, lens)
         st["start"].index_copy_(0, slots, first)
         st["limit"].index_copy_(0, slots, limits)
@@ -422,6 +627,7 @@ class BatchedSamdDecoder:
         W, max_accept = st["out"].shape[1], st["acc_tokens"].shape[1]              # (the most one step adds to a cache)
         flag_host = torch.zeros(2 * B + 1, dtype=torch.int32).pin_memory()
         steps = syncs = since = admissions = live_steps = 0
+        self.prefix_hits = self.prefix_tokens = 0
         self.last_graphed = False
 
         def admit() -> int:
@@ -465,6 +671,8 @@ class BatchedSamdDecoder:
             kv_hi = max(kv_hi, admit())
         self._run_stats = dict(steps_run=steps, host_syncs=syncs, graphed=self.last_graphed, graphs=len(self._graphs),
                                admissions=admissions, live_slot_steps=live_steps, **self._extra_stats())
+        if self._prefixes is not None:
+            self._run_stats.update(prefix_hits=self.prefix_hits, prefix_tokens=self.prefix_tokens)
 
     @torch.inference_mode()
     def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4):
@@ -503,7 +711,12 @@ class BatchedSamdDecoder:
         (SamdError naming its index).  self.serve_stats is set once the generator is exhausted: steps_run, host_syncs
         (flag reads), graphed, graphs, admissions, live_slot_steps (slot-steps of unfinished requests) and, for
         BatchedSamOnlyDecoder, tree_steps.  One call at a time: a generate() or serve() call while this generator is
-        suspended ends it (it raises when resumed); an abandoned generator leaves the decoder usable."""
+        suspended ends it (it raises when resumed); an abandoned generator leaves the decoder usable.
+
+        With a prefix pool (max_prefixes > 0) every request starts from the longest registered prefix its prompt begins
+        with (add_prefix may be called while this generator is suspended; it counts from the next admission on): its
+        info also holds "prefix_len" (0 without a match), and serve_stats "prefix_hits" (requests that started from a
+        prefix) and "prefix_tokens" (prompt tokens whose prefill and ingestion were skipped)."""
         self.serve_stats = None
         if hasattr(max_new_tokens, "__len__"):
             limits = [int(x) for x in max_new_tokens]
@@ -512,7 +725,10 @@ class BatchedSamdDecoder:
             limits, max_limit = None, int(max_new_tokens)
         for i, tokens, hist, slot in self._run(self._requests(prompts, max_new_tokens if limits is None else limits),
                                                max(max_limit, 1), graph, check_every):
-            yield i, tokens, {"slot": slot, "accept_lengths": hist}
+            info = {"slot": slot, "accept_lengths": hist}
+            if self._prefixes is not None:
+                info["prefix_len"] = self._slot_plen[slot]
+            yield i, tokens, info
         self.serve_stats = dict(self._run_stats)
 
     def _requests(self, prompts: Iterable[Sequence[int]], limits: Union[int, List[int]]) -> Iterator[tuple]:
@@ -553,7 +769,9 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
         samd_verify_compact    accept lengths, accepted tokens, next tokens, the accepted KV rows moved into place
 
     T = P = D = max_predicts.  The rest of the loop (prefill, one CUDA graph per key-length bucket, the commit, one host
-    read per `check_every` steps, generate() and serve()) is BatchedSamdDecoder's.  stats["tree_steps"] (and
+    read per `check_every` steps, generate() and serve()) is BatchedSamdDecoder's, and so is prefix reuse
+    (max_prefixes, add_prefix, drop_prefix): a registered prefix carries its automaton and static cursor, so the static
+    trees of a request that starts from one are those of its full prompt.  stats["tree_steps"] (and
     serve_stats["tree_steps"]) counts the request-steps of live requests that drafted a static tree.
 
     Known corner, inherited from the reference (SURVEY Appendix A9): a -1 pad column of a path selects token 0, so it is
@@ -564,7 +782,7 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
 
     def __init__(self, lm, batch: int, max_cache_len: int, max_predicts: int = 40, alpha: float = 4.0, K: int = 8,
                  len_bias: int = 5, static: Optional[E.StaticSamDevice] = None, eos_token_id: Optional[int] = None,
-                 max_tokens: int = 16384, dtype=torch.float16, device="cuda"):
+                 max_tokens: int = 16384, dtype=torch.float16, device="cuda", max_prefixes: int = 0):
         if static is not None and not static.with_counts:
             raise _cabi.SamdError("BatchedSamOnlyDecoder: the static automaton must be built with_counts=True "
                                   "(the sam_only tree drafter reads its occurrence counts and top-8 successors)")
@@ -587,6 +805,7 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
         self.buf = dict(tokens=mk(batch, T), position_ids=torch.zeros(batch, T, dtype=torch.long, device=dev),
                         n_nodes=mk(batch), n_paths=mk(batch), retrieve=mk(batch, T, T),
                         mask=torch.zeros(batch * T * max_cache_len, dtype=dtype, device=dev))
+        self._init_pool(max_prefixes)
 
     def _extra_state(self, mk) -> dict:
         return dict(tree_steps=torch.zeros(1, dtype=torch.long, device=self.device))

@@ -108,6 +108,16 @@ class DynSamBatch:
         with torch.cuda.device(self.device):
             K.check(K.lib().samd_dyn_copy(self._h, other.handle, K.stream_ptr()), "samd_dyn_copy")
 
+    def clone_from(self, src: "DynSamBatch", src_idx: torch.Tensor, dst_idx: torch.Tensor):
+        """Request dst_idx[i] of this batch becomes an exact copy of request src_idx[i] of `src` (samd_dyn_clone: one
+        launch, stream ordered; int32 CUDA index tensors, destinations distinct; both batches need the same max_tokens)."""
+        _i32(src_idx)
+        _i32(dst_idx)
+        assert src_idx.numel() == dst_idx.numel()
+        with torch.cuda.device(self.device):
+            K.check(K.lib().samd_dyn_clone(self._h, dst_idx.data_ptr(), src.handle, src_idx.data_ptr(), dst_idx.numel(),
+                                           K.stream_ptr()), "samd_dyn_clone")
+
     def stats(self) -> dict:
         out = np.zeros(8, dtype=np.int64)
         with torch.cuda.device(self.device):
@@ -479,6 +489,37 @@ class DraftEngine:
             K.check(K.lib().samd_draft_assemble(C.byref(a), K.stream_ptr()), "samd_draft_assemble")
 
 
+def kv_table(kv_tensors: List[torch.Tensor], device) -> tuple:
+    """The C ABI's view of a KV cache: a device table of the tensors' base pointers and their shared shape in bytes.
+    kv_tensors: the 2L cache tensors [B, H, max_len, Dh] (key_cache + value_cache order), all of one shape and stride."""
+    t0 = kv_tensors[0]
+    assert t0.dim() == 4 and t0.stride(3) == 1
+    es = t0.element_size()
+    for t in kv_tensors:
+        assert t.shape == t0.shape and t.stride() == t0.stride() and t.dtype == t0.dtype and t.device == t0.device
+    ptrs = torch.tensor([t.data_ptr() for t in kv_tensors], dtype=torch.int64, device=device)
+    meta = dict(n_kv=len(kv_tensors), n_heads=t0.shape[1], row_bytes=t0.shape[3] * es, batch_stride=t0.stride(0) * es,
+                head_stride=t0.stride(1) * es, pos_stride=t0.stride(2) * es)
+    return ptrs, meta
+
+
+def kv_copy_rows(dst: tuple, src: tuple, dst_row: torch.Tensor, src_row: torch.Tensor, n_rows: torch.Tensor):
+    """samd_kv_copy_rows: rows [0, n_rows[i]) of batch row src_row[i] of `src` into batch row dst_row[i] of `dst`, every
+    tensor and head, one launch.  dst / src: kv_table() of two caches with the same tensor count, heads and row size;
+    the pair arrays are int32 CUDA tensors."""
+    (dp, dm), (sp, sm) = dst, src
+    assert (dm["n_kv"], dm["n_heads"], dm["row_bytes"]) == (sm["n_kv"], sm["n_heads"], sm["row_bytes"])
+    for t in (dst_row, src_row, n_rows):
+        _i32(t)
+    assert dst_row.numel() == src_row.numel() == n_rows.numel()
+    with torch.cuda.device(dp.device):
+        K.check(K.lib().samd_kv_copy_rows(dp.data_ptr(), dm["batch_stride"], dm["head_stride"], dm["pos_stride"],
+                                          sp.data_ptr(), sm["batch_stride"], sm["head_stride"], sm["pos_stride"],
+                                          dm["n_kv"], dm["n_heads"], dm["row_bytes"], dst_row.data_ptr(),
+                                          src_row.data_ptr(), n_rows.data_ptr(), dst_row.numel(), K.stream_ptr()),
+                "samd_kv_copy_rows")
+
+
 class Verifier:
     """Fused greedy verification + KV compaction (samd/utils.py:127-141, samd/samd_model.py:159-211,
     samd/cache.py:118-133) for a batch of requests: one persistent launch."""
@@ -502,14 +543,7 @@ class Verifier:
         key = tuple(t.data_ptr() for t in kv_tensors)
         if key == self._kv_key:
             return
-        t0 = kv_tensors[0]
-        assert t0.dim() == 4 and t0.stride(3) == 1
-        es = t0.element_size()
-        for t in kv_tensors:
-            assert t.shape == t0.shape and t.stride() == t0.stride() and t.dtype == t0.dtype and t.device == t0.device
-        self._kv_ptrs = torch.tensor(list(key), dtype=torch.int64, device=self.device)
-        self._kv_meta = dict(n_kv=len(kv_tensors), n_heads=t0.shape[1], row_bytes=t0.shape[3] * es,
-                             batch_stride=t0.stride(0) * es, head_stride=t0.stride(1) * es, pos_stride=t0.stride(2) * es)
+        self._kv_ptrs, self._kv_meta = kv_table(kv_tensors, self.device)
         self._kv_key = key
 
     def verify(self, logits: torch.Tensor, tree_tokens: torch.Tensor, retrieve: Optional[torch.Tensor],
@@ -682,13 +716,34 @@ class RecycleTable:
         """table[tokens[i]] = top-8 of logits[i] for i in order (last occurrence of a token wins); [N] and [N, V].
         One launch: every row is a one-node request of the verify kernel.  Returns the [N, 8] top-8 indices."""
         assert logits.dim() == 2 and tokens.numel() == logits.shape[0]
+        return self._rows(tokens, logits, write=True)
+
+    def topk(self, tokens: torch.Tensor, logits: torch.Tensor) -> torch.Tensor:
+        """The [N, 8] rows update() would write for `tokens` / `logits`, without writing the table."""
+        return self._rows(tokens, logits, write=False)
+
+    def _rows(self, tokens: torch.Tensor, logits: torch.Tensor, write: bool) -> torch.Tensor:
+        assert logits.dim() == 2 and tokens.numel() == logits.shape[0]
         N, V = logits.shape
         self.ensure(V, logits.device)
         if self._ver is None or self._ver_cap < N:
             self._ver_cap = max(N, 256)
             self._ver = Verifier(self._ver_cap, 1, self.device)
-        out = self._ver.verify(logits.view(N, 1, V), _i32(tokens.to(torch.int32).contiguous().view(N, 1)), None, recycle=self)
+        out = self._ver.verify(logits.view(N, 1, V), _i32(tokens.to(torch.int32).contiguous().view(N, 1)), None,
+                               want_topk=True, recycle=self if write else None)
         return out["topk"].view(N, 8)
+
+    def apply(self, tokens: torch.Tensor, rows: torch.Tensor):
+        """table[tokens[i]] = rows[i] for i in order, the last occurrence of a token winning - what update() does, for
+        rows computed earlier (topk()).  Deterministic: only each token's last row is written, so no index repeats."""
+        tokens = tokens.long()
+        if tokens.numel() == 0:
+            return
+        order = torch.arange(tokens.numel(), device=tokens.device)
+        last = torch.full((self.vocab,), -1, dtype=torch.long, device=tokens.device)
+        last.scatter_reduce_(0, tokens, order, reduce="amax")
+        keep = last[tokens] == order
+        self.table[tokens[keep]] = rows[keep].to(torch.int32)
 
     def gen_tree(self, start_tok: torch.Tensor, types: Optional[torch.Tensor] = None, only_type: int = 0,
                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
