@@ -369,6 +369,8 @@ int samd_verify_compact(samd_verify_t h, const samd_verify_args *args, void *str
  * Level by level, each distinct candidate token x among the paths that share the accepted prefix is tested once, in
  * path order, with one uniform draw r:  accept iff r <= p(x) / (1 - mass rejected so far at this level), where
  * p = softmax(logits_processor(row)) and logits_processor = temperature, then top-p, then top-k (samd/utils.py:44-58).
+ * Top-p follows an ascending sort that keeps equal values in index order: of the tie group the cut falls into, the
+ * lowest-index members are removed while the cumulative mass stays within 1 - top_p (masses summed in double).
  * The next token is drawn from the level's residual distribution when its last level rejected something (and the path
  * is not complete), else from the plain softmax of the last accepted node's row (samd/utils.py:173-179).
  * RNG CONTRACT: Philox4x32-10; uniform number k of request b is
@@ -398,6 +400,31 @@ typedef struct samd_sample_args {
     float   *out_sample_p_dev;        /* [B][V] the next token's distribution (the reference's returned sample_p), or NULL */
 } samd_sample_args;
 int samd_verify_sample(const samd_sample_args *args, void *stream);
+/* The same launch with per-request arguments (every pointer NULL = the shared value of `args`), for a batch whose
+ * requests each have their own processor, path-table width and state - what a batched decoder with per-request
+ * sampling parameters needs.  Per request b:
+ *   temperature / top_p / top_k   its own processor (same validity rules as the scalars; not checked on the host)
+ *   greedy_dev[b] = 1             the greedy eval_posterior (samd/utils.py:127-141) instead of the typical walk: the
+ *                                 argmax of every node row (torch.argmax's rule), the match length of every path, the
+ *                                 first longest path, the next token = the argmax of its last accepted row; no draw -
+ *                                 the outputs equal samd_verify_compact's for the same rows and table
+ *   done_dev[b] = 1, or n_paths 0 a finished request: no draw, offsets_dev[b] untouched, accept_len 0 and no other output
+ *                                 (samd_kv_compact then moves none of its rows)
+ *   n_nodes_dev[b]                its own row count: a -1 entry of its paths wraps to row n_nodes_dev[b] - 1
+ *   depth_dev[b]                  its own path width (<= depth): the walk stops there, so -1 pads beyond a request's
+ *                                 own draft are never compared (inside it, a -1 selects token 0 as in the reference)
+ * The output layout is samd_verify_sample's ([B][depth] tokens / indices).  Greedy requests need n_nodes <= 256.  No
+ * argument depends on the step, so the launch can be captured in a CUDA graph. */
+typedef struct samd_sample_request_args {
+    const float   *temperature_dev;   /* [B]; NULL = args->temperature */
+    const float   *top_p_dev;         /* [B]; NULL = args->top_p */
+    const int32_t *top_k_dev;         /* [B]; NULL = args->top_k */
+    const uint8_t *greedy_dev;        /* [B] 1 = greedy eval_posterior for this request; NULL = none */
+    const uint8_t *done_dev;          /* [B] 1 = finished slot: no draw, no output but accept_len 0; NULL = none */
+    const int32_t *n_nodes_dev;       /* [B] the request's own node count (-1 wraps to ITS last row); NULL = n_nodes */
+    const int32_t *depth_dev;         /* [B] the request's own path width; NULL = depth */
+} samd_sample_request_args;
+int samd_verify_sample_requests(const samd_sample_args *args, const samd_sample_request_args *r, void *stream);
 
 /* TokenRecycle.gen_draft (token_recycle.py:49-59) for a batch: tokens[b][0] = start_tok[b]; every other node takes
  * table[token of its parent][its rank among the parent's children], or 0 when the parent's token has no entry.

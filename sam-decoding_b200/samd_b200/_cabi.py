@@ -62,6 +62,13 @@ class SampleArgs(C.Structure):
     ]
 
 
+class SampleRequestArgs(C.Structure):
+    _fields_ = [
+        ("temperature_dev", vp), ("top_p_dev", vp), ("top_k_dev", vp), ("greedy_dev", vp), ("done_dev", vp),
+        ("n_nodes_dev", vp), ("depth_dev", vp),
+    ]
+
+
 class AssembleArgs(C.Structure):
     _fields_ = [
         ("batch", C.c_int32), ("n_nodes", C.c_int32), ("n_paths", C.c_int32), ("depth", C.c_int32), ("type_dev", vp),
@@ -142,6 +149,7 @@ SYMBOLS = {
     "samd_verify_destroy": (C.c_int, [vp]),
     "samd_verify_compact": (C.c_int, [vp, C.POINTER(VerifyArgs), vp]),
     "samd_verify_sample": (C.c_int, [C.POINTER(SampleArgs), vp]),
+    "samd_verify_sample_requests": (C.c_int, [C.POINTER(SampleArgs), C.POINTER(SampleRequestArgs), vp]),
     "samd_recycle_gen_tree": (C.c_int, [vp, C.c_int32, vp, vp, C.c_int32, vp, vp, C.c_int32, C.c_int32, vp, vp]),
     "samd_verify_set_chunk": (None, [C.c_int]),
     "samd_verify_set_overlap": (None, [C.c_int]),

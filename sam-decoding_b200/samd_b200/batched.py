@@ -28,9 +28,16 @@ prompts alone, masked drafter reset, prompt ingestion with count 0 for every oth
 place), so the graphs captured per key-length bucket stay valid and nothing waits for the longest request of a batch.
 With a prefix pool (max_prefixes > 0, add_prefix) an admitted request whose prompt starts with a registered prefix copies
 that prefix's KV rows, automaton and static cursor and prefills / ingests only the rest of its prompt.
+
+generate(..., sampling=...) and serve(..., sampling=...) decode with sampling instead (SamplingParams: temperature, top-p,
+top-k and a seed per request, as the reference's SamdGenerationConfig(greedy=False)): the verify step is
+samd_verify_sample_requests with every slot's own processor and Philox stream, and the first token of a request is drawn
+from the plain softmax of its prompt's last row.  A request's tokens depend only on its prompt, its parameters and its
+seed - not on its slot, its neighbours, the batch size, graph or eager execution, check_every, or a prefix pool.
 """
 from __future__ import annotations
 
+import dataclasses
 from typing import Iterable, Iterator, List, Optional, Sequence, Union
 
 import torch
@@ -40,6 +47,34 @@ from . import _cabi as K
 from . import engine as E
 
 _cabi = K                       # (BatchedSamOnlyDecoder takes a parameter named K)
+
+
+@dataclasses.dataclass(frozen=True)
+class SamplingParams:
+    """Sampled decoding of one request (the fields of the reference's SamdGenerationConfig with greedy=False, plus the
+    seed of the request's device Philox stream).  temperature >= 1e-5 (unless greedy), 0 <= top_p <= 1 (active below 1,
+    0 = off), top_k >= 0 (0 = off), 0 <= seed < 2**63.  greedy=True decodes this request greedily inside a sampled call:
+    its tokens are plain greedy decoding and it makes no draw.  The decoders check the values of every request when it is
+    pulled and name its index in the error."""
+    temperature: float = 1.0
+    top_p: float = 0.0
+    top_k: int = 0
+    seed: int = 0
+    greedy: bool = False
+
+    def problem(self) -> Optional[str]:
+        """What is wrong with these values (None: nothing)."""
+        if not isinstance(self.greedy, bool):
+            return f"greedy must be a bool, got {self.greedy!r}"
+        if not self.greedy and not self.temperature >= 1e-5:
+            return f"temperature must be >= 1e-5, got {self.temperature}"
+        if not 0.0 <= self.top_p <= 1.0:
+            return f"top_p must be in [0, 1], got {self.top_p}"
+        if not isinstance(self.top_k, int) or self.top_k < 0:
+            return f"top_k must be an int >= 0, got {self.top_k!r}"
+        if not isinstance(self.seed, int) or not 0 <= self.seed < 2 ** 63:
+            return f"seed must be an int in [0, 2**63), got {self.seed!r}"
+        return None
 
 
 class _Layer(CacheLayerMixin):
@@ -164,7 +199,7 @@ class BatchedSamdDecoder:
             # ingestion only (no lookup); it has cursors on the decoder's static automaton
             eng = E.DraftEngine(dyn, self.eng.static, self.eng.flavour, n_predicts=self.eng.n_predicts)
             self.pool = dict(cache=cache, dyn=dyn, eng=eng)
-            self._prefixes = [None] * max_prefixes      # per pool row: dict(tokens, next, topk) or None
+            self._prefixes = [None] * max_prefixes      # per pool row: dict(tokens, ids, last, topk) or None
             self._slot_plen = [0] * self.B
 
     def _init_tree(self, tree):
@@ -255,7 +290,16 @@ class BatchedSamdDecoder:
         pos = cache.cache_len.long()[:, None] + self._ar[None, :]
         logits = self.lm(input_ids=draft.long(), position_ids=pos, past_key_values=cache,
                          attention_mask=self._mask(T, kv_len, cache.cache_len)).logits
+        if self._sampled:                                      # identity path: no row moves, the commit sets cache_len
+            return self._verify_sample(logits.contiguous(), draft, None)
         return self.ver.verify(logits.contiguous(), draft, None, cache_len=cache.cache_len, out=st["res"])
+
+    def _verify_sample(self, logits: torch.Tensor, tokens: torch.Tensor, retrieve: Optional[torch.Tensor], **kw) -> dict:
+        """samd_verify_sample_requests with every slot's processor, greedy flag and Philox stream; finished slots make no
+        draw and accept nothing."""
+        st = self._st
+        return self.ver.verify_sample(logits, tokens, retrieve, st["temperature"], st["top_p"], st["top_k"], st["seed"],
+                                      st["offset"], greedy=st["greedy"], done=st["done"], out=st["res"], **kw)
 
     # ---- one decode step, entirely on the device (no host read anywhere: it is what gets captured in a CUDA graph) ----
     def _step_body(self, kv_len: int):
@@ -331,9 +375,13 @@ class BatchedSamdDecoder:
             mk = lambda *sh: torch.zeros(*sh, dtype=torch.int32, device=dev)
             # out: a slot's tokens plus spare columns; hist: its live steps (each emits >= 1 token, so at most max_limit)
             # plus a spare column; hlen: its live-step count; limit: its max_new_tokens
+            # temperature .. offset: every slot's sampling parameters and the position of its Philox stream
             self._st = dict(start=mk(B), acc_tokens=mk(B, width), acc_count=mk(B), out=mk(B, max_limit + T), out_len=mk(B),
                             limit=mk(B), done=torch.zeros(B, dtype=torch.bool, device=dev), hist=mk(B, max_limit + 1),
-                            hlen=mk(B), flag=mk(2 * B + 1), res=None, **self._extra_state(mk))
+                            hlen=mk(B), flag=mk(2 * B + 1), temperature=torch.ones(B, device=dev), top_p=torch.zeros(B, device=dev),
+                            top_k=mk(B), greedy=torch.zeros(B, dtype=torch.uint8, device=dev),
+                            seed=torch.zeros(B, dtype=torch.long, device=dev), offset=torch.zeros(B, dtype=torch.long, device=dev),
+                            res=None, **self._extra_state(mk))
             self._st_cap, self._graphs = max_limit, {}
         else:
             for k, v in self._st.items():
@@ -342,10 +390,12 @@ class BatchedSamdDecoder:
 
     def _advance(self, kv_len: int, graph: bool) -> bool:
         """One decode step at key length `kv_len`: the bucket's CUDA graph, captured first if it is new, or the same body
-        eagerly.  Returns `graph`, False from then on when the LM's forward cannot be captured."""
+        eagerly (one graph per bucket and greedy / sampled body).  Returns `graph`, False from then on when the LM's forward
+        cannot be captured."""
         if graph:
             B, dev, graphs = self.B, self.device, self._graphs
-            if kv_len not in graphs:
+            key = (kv_len, self._sampled)
+            if key not in graphs:
                 # warm-up run on a side stream (allocations, lazy initialisation), state restored, then the capture
                 snap = {k: (v.clone() if torch.is_tensor(v) else v) for k, v in self._st.items() if k != "res"}
                 snap_len = self.cache.cache_len.clone()
@@ -377,7 +427,7 @@ class BatchedSamdDecoder:
                     g = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(g):
                         self._step_body(kv_len)
-                    graphs[kv_len] = g
+                    graphs[key] = g
                     self.last_graphed = True
                 except Exception:                          # an LM whose forward cannot be captured: same body, eagerly
                     graph = False
@@ -385,7 +435,7 @@ class BatchedSamdDecoder:
                 restore()                                  # (capture does not run the work; the warm-up did)
                 snap_dyn.close()
             if graph:
-                graphs[kv_len].replay()
+                graphs[key].replay()
                 self.last_graphed = True
                 return True
         self._step_body(kv_len)
@@ -397,7 +447,8 @@ class BatchedSamdDecoder:
         """Register a prompt head; returns its id (the id it already has when these tokens are registered).  The
         prefix's LM prefill runs alone into a pool row, its automaton and static cursor ingest it, and its greedy next
         token (and, in tree mode, the top-8 rows of its positions) are kept.  No slot and no captured graph is touched:
-        it may be called between calls and while a serve() generator is suspended."""
+        it may be called between calls and while a serve() generator is suspended.  The logits row after the prefix is
+        kept too: a prompt equal to the prefix starts from its argmax, or from a draw from its softmax when sampled."""
         tokens = tuple(int(t) for t in tokens)
         pid = self._check_prefix(tokens)
         if self._prefixes[pid] is not None:
@@ -412,7 +463,7 @@ class BatchedSamdDecoder:
         tok = torch.zeros(P, n, dtype=torch.int32, device=dev).index_copy_(0, slot, ids.to(torch.int32))
         eng.step(tok, torch.zeros(P, dtype=torch.int32, device=dev).index_fill_(0, slot, n), None)
         topk = self.table.topk(ids[0], logits[0]) if self.tree is not None else None
-        self._prefixes[pid] = dict(tokens=tokens, ids=ids[0], next=logits[0, n - 1].argmax(-1).to(torch.int32), topk=topk)
+        self._prefixes[pid] = dict(tokens=tokens, ids=ids[0], last=logits[0, n - 1].clone(), topk=topk)
         return pid
 
     def drop_prefix(self, pid: int):
@@ -458,27 +509,27 @@ class BatchedSamdDecoder:
 
     # ---- admission: new requests into free slots, between two steps ---------------------------------------------------
     def _admit(self, reqs: List[tuple]) -> int:
-        """Start the requests `reqs` = [(slot, prompt, limit)] in their (free) slots; returns the longest prompt.  Only
-        the persistent state is written, in place, so the captured graphs stay valid."""
+        """Start the requests `reqs` = [(slot, prompt, limit, SamplingParams or None)] in their (free) slots; returns the
+        longest prompt.  Only the persistent state is written, in place, so the captured graphs stay valid."""
         dev = self.device
-        n_max = max(len(p) for _, p, _ in reqs)
+        n_max = max(len(r[1]) for r in reqs)
         if self._prefixes is not None:
-            hits = [self._longest_prefix(p) for _, p, _ in reqs]
-            for (b, _, _), (_, n) in zip(reqs, hits):
+            hits = [self._longest_prefix(r[1]) for r in reqs]
+            for (b, *_), (_, n) in zip(reqs, hits):
                 self._slot_plen[b] = n
             if any(pid is not None for pid, _ in hits):
                 self._admit_prefixed(reqs, hits)
                 return n_max
         ids = torch.zeros(len(reqs), n_max, dtype=torch.long)
-        for i, (_, p, _) in enumerate(reqs):
+        for i, (_, p, *_) in enumerate(reqs):
             ids[i, :len(p)] = torch.as_tensor(p, dtype=torch.long)
         meta = torch.tensor([[r[0] for r in reqs], [len(r[1]) for r in reqs], [r[2] for r in reqs]], dtype=torch.long)
         ids, meta = ids.to(dev), meta.to(dev)
         slots, lens, limits = meta[0], meta[1].to(torch.int32), meta[2].to(torch.int32)
         logits = self._prefill_slots(ids, slots)
         self._ingest(ids, slots, lens, logits)
-        first = logits[torch.arange(slots.numel(), device=dev), lens.long() - 1].argmax(-1).to(torch.int32)
-        self._set_slots(slots, lens, limits, first)
+        self._set_slots(slots, lens, limits, logits[torch.arange(slots.numel(), device=dev), lens.long() - 1],
+                        [r[3] for r in reqs])
         return n_max
 
     def _admit_prefixed(self, reqs: List[tuple], hits: List[tuple]):
@@ -486,10 +537,11 @@ class BatchedSamdDecoder:
         for the others): their KV rows [0, len(P)) come from the pool (one samd_kv_copy_rows launch), one LM forward
         runs over the suffixes alone (right padded, rows from len(P) on), the unmatched slots' drafters are reset and
         the matched ones cloned from the pool (one samd_dyn_clone launch, static-cursor rows copied), and one samd_step
-        ingests the suffixes - count 0 for a prompt equal to its prefix, which starts from the prefix's next token."""
+        ingests the suffixes - count 0 for a prompt equal to its prefix, which starts from the logits row kept after the
+        prefix."""
         dev, pool = self.device, self.pool
         n = len(reqs)
-        sufs = [p[m:] for (_, p, _), (_, m) in zip(reqs, hits)]
+        sufs = [r[1][m:] for r, (_, m) in zip(reqs, hits)]
         n_suf = max(len(x) for x in sufs)
         hit = [i for i in range(n) if hits[i][0] is not None]
         fw = [i for i in range(n) if len(sufs[i])]                                   # requests with a suffix
@@ -512,14 +564,13 @@ class BatchedSamdDecoder:
         self._ingest_suffixes(ids, slots, suf_lens, [(hits[i][0], len(sufs[i])) for i in range(n)], fw, logits)
         self.prefix_hits += len(hit)
         self.prefix_tokens += sum(hits[i][1] for i in hit)
-        # first start token: the greedy token after the last suffix row, or after the prefix itself
-        first = torch.zeros(n, dtype=torch.int32, device=dev)
+        # the first start token comes from the row after the last suffix token, or after the prefix itself
+        rows = [self._prefixes[hits[i][0]]["last"] if not len(sufs[i]) else None for i in range(n)]
         if fw:
-            first[f] = logits[torch.arange(len(fw), device=dev), suf_lens[f].long() - 1].argmax(-1).to(torch.int32)
-        exact = [i for i in range(n) if not len(sufs[i])]
-        if exact:
-            first[torch.tensor(exact, device=dev)] = torch.stack([self._prefixes[hits[i][0]]["next"] for i in exact])
-        self._set_slots(slots, lens, limits, first)
+            last = logits[torch.arange(len(fw), device=dev), suf_lens[f].long() - 1]
+            for k, i in enumerate(fw):
+                rows[i] = last[k]
+        self._set_slots(slots, lens, limits, torch.stack(rows), [r[3] for r in reqs])
 
     def _copy_prefix_kv(self, slots: torch.Tensor, pids: torch.Tensor, plens: torch.Tensor):
         """KV rows [0, plens[i]) of pool row pids[i] into slot slots[i]: one samd_kv_copy_rows launch."""
@@ -596,11 +647,34 @@ class BatchedSamdDecoder:
         self.eng.step(tokens, counts, None)
         self._prefill_hook(ids, lens, logits)
 
-    def _set_slots(self, slots: torch.Tensor, lens: torch.Tensor, limits: torch.Tensor, first: torch.Tensor):
-        """The admitted slots' step state: cache length, first start token (the prompt's greedy next token), limit, and
-        zero emitted tokens / history."""
+    def _set_slots(self, slots: torch.Tensor, lens: torch.Tensor, limits: torch.Tensor, rows: torch.Tensor,
+                   params: List[Optional[SamplingParams]]):
+        """The admitted slots' step state: cache length, sampling parameters and a fresh Philox stream (sampled calls),
+        first start token from `rows` [n, V] (the logits after each prompt: argmax, or a draw from the plain softmax),
+        limit, and zero emitted tokens / history."""
         st = self._st
         self.cache.cache_len.index_copy_(0, slots, lens)
+        if self._sampled:
+            dev = self.device
+            f = torch.tensor([[sp.temperature, sp.top_p] for sp in params], dtype=torch.float32).T.contiguous().to(dev)
+            i = torch.tensor([[sp.top_k, int(sp.greedy), sp.seed] for sp in params], dtype=torch.long).T.contiguous().to(dev)
+            st["temperature"].index_copy_(0, slots, f[0])
+            st["top_p"].index_copy_(0, slots, f[1])
+            st["top_k"].index_copy_(0, slots, i[0].to(torch.int32))
+            st["greedy"].index_copy_(0, slots, i[1].to(torch.uint8))
+            st["seed"].index_copy_(0, slots, i[2])
+            st["offset"].index_fill_(0, slots, 0)
+            # depth 1: the kernel's walk is empty and the token is drawn from the plain softmax of the row (samd/utils.py
+            # :173-179 with nothing accepted), as the reference's torch.multinomial after the prefill; greedy: its argmax
+            n, V = rows.shape
+            offs = st["offset"][slots]
+            res = self.ver.verify_sample(rows.contiguous().view(n, 1, V), torch.zeros(n, 1, dtype=torch.int32, device=dev),
+                                         None, st["temperature"][slots], st["top_p"][slots], st["top_k"][slots],
+                                         st["seed"][slots], offs, greedy=st["greedy"][slots])
+            st["offset"].index_copy_(0, slots, offs)
+            first = res["next_token"]
+        else:
+            first = rows.argmax(-1).to(torch.int32)
         st["start"].index_copy_(0, slots, first)
         st["limit"].index_copy_(0, slots, limits)
         for k in ("acc_count", "out_len", "hlen"):
@@ -608,8 +682,9 @@ class BatchedSamdDecoder:
         st["done"].index_fill_(0, slots, False)
 
     # ---- the decode loop of generate() and serve() --------------------------------------------------------------------
-    def _run(self, requests: Iterator[tuple], max_limit: int, graph: bool, check_every: int):
-        """Decode the validated requests (index, prompt, limit) of `requests`, at most B at a time.  The decode step has
+    def _run(self, requests: Iterator[tuple], max_limit: int, graph: bool, check_every: int, sampled: bool = False):
+        """Decode the validated requests (index, prompt, limit, SamplingParams or None) of `requests`, at most B at a
+        time, with the greedy step body or (sampled) the sampled one.  The decode step has
         no host synchronisation in it: it is captured once per key-length bucket (64 positions) as a CUDA graph and
         replayed.  Once every `check_every` steps the host reads [done | out_len | longest cache] in one copy; it then
         yields (index, tokens, accept_lengths, slot) for every request found finished (their rows in one more copy),
@@ -618,6 +693,7 @@ class BatchedSamdDecoder:
         self._run_stats."""
         B, T, dev = self.B, self.T, self.device
         self._init_state(max_limit)
+        self._sampled = sampled
         st = self._st
         run = self._run_id = getattr(self, "_run_id", 0) + 1
         self.eng.reset()
@@ -639,7 +715,7 @@ class BatchedSamdDecoder:
                     if r is None:
                         break
                     owner[b] = r[0]
-                    reqs.append((b, r[1], r[2]))
+                    reqs.append((b, r[1], r[2], r[3]))
             admissions += len(reqs)
             return self._admit(reqs) if reqs else 0
 
@@ -675,12 +751,14 @@ class BatchedSamdDecoder:
             self._run_stats.update(prefix_hits=self.prefix_hits, prefix_tokens=self.prefix_tokens)
 
     @torch.inference_mode()
-    def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4):
+    def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4,
+                 sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None):
         """Lossless batched speculative decoding of exactly B prompts in lockstep (request b in slot b), up to
         max_new_tokens each.  The host reads the finished flags once every `check_every` steps - 1 / check_every host
         syncs per step - so a finished batch may run up to check_every - 1 idle steps (every request done: nothing is
         emitted).  graph=False runs the same body eagerly.  Returns (tokens per request, stats); stats["accept_lengths"]
-        holds every request's accepted tokens per step, padded with 0 to the longest request's `steps`."""
+        holds every request's accepted tokens per step, padded with 0 to the longest request's `steps`.  `sampling`: as
+        in serve()."""
         B, T = self.B, self.T
         assert len(prompts) == B
         n_max = max(len(p) for p in prompts)
@@ -691,9 +769,9 @@ class BatchedSamdDecoder:
         if n_max + max_new_tokens + T > self.dyn.max_tokens:
             raise K.SamdError(f"prompt + max_new_tokens + one step = {n_max + max_new_tokens + T} exceeds the automaton "
                               f"capacity max_tokens={self.dyn.max_tokens}")
+        reqs = self._with_sampling(((i, p, max_new_tokens) for i, p in enumerate(prompts)), sampling)
         out, acc = [None] * B, [None] * B
-        for i, tokens, hist, _ in self._run(((i, p, max_new_tokens) for i, p in enumerate(prompts)), max_new_tokens,
-                                            graph, check_every):
+        for i, tokens, hist, _ in self._run(reqs, max_new_tokens, graph, check_every, sampling is not None):
             out[i], acc[i] = tokens, hist
         n_live = max(len(a) for a in acc)
         s = self._run_stats
@@ -702,7 +780,7 @@ class BatchedSamdDecoder:
 
     @torch.inference_mode()
     def serve(self, prompts: Iterable[Sequence[int]], max_new_tokens: Union[int, Sequence[int]], graph: bool = True,
-              check_every: int = 4):
+              check_every: int = 4, sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None):
         """Continuous batching: decode any number of requests through the B slots, refilling a slot with the next queued
         request as soon as the host sees its request finished (once every `check_every` steps).  `prompts` is consumed
         lazily and in order; `max_new_tokens` is one limit for all or a sequence with one per request.  Yields
@@ -716,15 +794,20 @@ class BatchedSamdDecoder:
         With a prefix pool (max_prefixes > 0) every request starts from the longest registered prefix its prompt begins
         with (add_prefix may be called while this generator is suspended; it counts from the next admission on): its
         info also holds "prefix_len" (0 without a match), and serve_stats "prefix_hits" (requests that started from a
-        prefix) and "prefix_tokens" (prompt tokens whose prefill and ingestion were skipped)."""
+        prefix) and "prefix_tokens" (prompt tokens whose prefill and ingestion were skipped).
+
+        `sampling` (None: greedy, lossless): one SamplingParams for every request - request i then uses the Philox key
+        seed + i - or a sequence with one per request.  Each request's processor and stream are its own, so its tokens
+        depend only on its prompt, parameters and seed; a request with greedy=True decodes greedily.  Not with
+        Token-Recycle tree mode (tree=): SamdError."""
         self.serve_stats = None
         if hasattr(max_new_tokens, "__len__"):
             limits = [int(x) for x in max_new_tokens]
             max_limit = max(limits, default=1)
         else:
             limits, max_limit = None, int(max_new_tokens)
-        for i, tokens, hist, slot in self._run(self._requests(prompts, max_new_tokens if limits is None else limits),
-                                               max(max_limit, 1), graph, check_every):
+        reqs = self._with_sampling(self._requests(prompts, max_new_tokens if limits is None else limits), sampling)
+        for i, tokens, hist, slot in self._run(reqs, max(max_limit, 1), graph, check_every, sampling is not None):
             info = {"slot": slot, "accept_lengths": hist}
             if self._prefixes is not None:
                 info["prefix_len"] = self._slot_plen[slot]
@@ -754,6 +837,34 @@ class BatchedSamdDecoder:
                                   f"automaton capacity max_tokens={cap}")
             yield i, p, limit
 
+    def _with_sampling(self, requests: Iterator[tuple], sampling) -> Iterator[tuple]:
+        """(index, prompt, limit, SamplingParams or None) of every request: its own params (seed + index for one shared
+        SamplingParams), checked as it is pulled.  Tree mode is refused at once."""
+        if sampling is not None and getattr(self, "tree", None) is not None:
+            raise K.SamdError("sampling is not supported in Token-Recycle tree mode (tree=): its table update rides on "
+                              "the greedy verify launch")
+        shared = sampling is None or isinstance(sampling, SamplingParams)
+        return self._sampled_requests(requests, sampling if shared else list(sampling), shared)
+
+    @staticmethod
+    def _sampled_requests(requests: Iterator[tuple], sampling, shared: bool) -> Iterator[tuple]:
+        for i, p, limit in requests:
+            if sampling is None:
+                yield i, p, limit, None
+                continue
+            if shared:
+                sp = dataclasses.replace(sampling, seed=sampling.seed + i) if isinstance(sampling.seed, int) else sampling
+            elif i >= len(sampling):
+                raise K.SamdError(f"request {i}: sampling has {len(sampling)} values, fewer than the prompts")
+            else:
+                sp = sampling[i]
+            if not isinstance(sp, SamplingParams):
+                raise K.SamdError(f"request {i}: sampling must be a SamplingParams, got {type(sp).__name__}")
+            bad = sp.problem()
+            if bad:
+                raise K.SamdError(f"request {i}: {bad}")
+            yield i, p, limit, sp
+
 
 class BatchedSamOnlyDecoder(BatchedSamdDecoder):
     """Batched decoding with the `samd_sam_only` flavour (samd_sam_only/samd_model.py:117-157 for B requests in lockstep):
@@ -778,7 +889,9 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
     "accepted" when the compared row's argmax is token 0, and the KV move then copies row cache_len - 1.  The batched path
     table is D wide while a reference tree is only as wide as its own deepest path (and a reference sequence as long as
     its draft), so here pads beyond a request's own width can be compared too - only after every real node of the path
-    was accepted, i.e. when the LM's greedy next token is 0."""
+    was accepted, i.e. when the LM's greedy next token is 0.  A sampled call (sampling=...) verifies every request only up
+    to its own width (samd_verify_sample_requests with the longest path of its row of the table), then samd_kv_compact
+    moves its accepted rows: there the pads beyond a request's own draft are never compared."""
 
     def __init__(self, lm, batch: int, max_cache_len: int, max_predicts: int = 40, alpha: float = 4.0, K: int = 8,
                  len_bias: int = 5, static: Optional[E.StaticSamDevice] = None, eos_token_id: Optional[int] = None,
@@ -803,7 +916,7 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
         T, dev = max_predicts, self.device
         mk = lambda *s: torch.zeros(*s, dtype=torch.int32, device=dev)
         self.buf = dict(tokens=mk(batch, T), position_ids=torch.zeros(batch, T, dtype=torch.long, device=dev),
-                        n_nodes=mk(batch), n_paths=mk(batch), retrieve=mk(batch, T, T),
+                        n_nodes=mk(batch), n_paths=mk(batch), retrieve=mk(batch, T, T), depth=mk(batch),
                         mask=torch.zeros(batch * T * max_cache_len, dtype=dtype, device=dev))
         self._init_pool(max_prefixes)
 
@@ -828,5 +941,13 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
         cache.begin(T, kv_len)
         logits = self.lm(input_ids=buf["tokens"].long(), position_ids=buf["position_ids"], past_key_values=cache,
                          attention_mask=mask[:, None]).logits
+        if self._sampled:
+            # a request's own width - its draft length, or its tree's deepest path - so that the -1 pads beyond it are
+            # never compared; then the accepted rows move into place
+            torch.amax((buf["retrieve"] >= 0).sum(2, dtype=torch.int32), 1, out=buf["depth"])
+            res = self._verify_sample(logits.contiguous(), buf["tokens"], buf["retrieve"], n_paths=buf["n_paths"],
+                                      n_nodes=buf["n_nodes"], depth=buf["depth"])
+            self.ver.kv_compact(res["indices"], res["accept_len"], cache.cache_len)
+            return res
         return self.ver.verify(logits.contiguous(), buf["tokens"], buf["retrieve"], cache_len=cache.cache_len, move_kv=True,
                                n_nodes=buf["n_nodes"], n_paths=buf["n_paths"], out=st["res"])

@@ -623,11 +623,21 @@ class Verifier:
         return out
 
     def verify_sample(self, logits: torch.Tensor, tree_tokens: torch.Tensor, retrieve: Optional[torch.Tensor],
-                      temperature: float, top_p: float, top_k: int, seeds: torch.Tensor, offsets: torch.Tensor,
-                      n_paths: Optional[torch.Tensor] = None, want_sample_p: bool = False) -> dict:
+                      temperature, top_p, top_k, seeds: torch.Tensor, offsets: torch.Tensor,
+                      n_paths: Optional[torch.Tensor] = None, want_sample_p: bool = False,
+                      greedy: Optional[torch.Tensor] = None, done: Optional[torch.Tensor] = None,
+                      n_nodes: Optional[torch.Tensor] = None, depth: Optional[torch.Tensor] = None,
+                      out: Optional[dict] = None) -> dict:
         """Typical-acceptance verification + the draw of the next token (samd/utils.py:142-184, :85-88) for a batch:
         one launch, one CTA per request.  `seeds` / `offsets`: int64 CUDA tensors [B] - the Philox stream of every request
-        (include/samd_b200.h states the contract); `offsets` is advanced in place by the draws used."""
+        (include/samd_b200.h states the contract); `offsets` is advanced in place by the draws used.
+
+        Per request (samd_verify_sample_requests): `temperature` / `top_p` / `top_k` may each be a [B] CUDA tensor
+        (float32, float32, int32) instead of one value; `greedy` [B] uint8/bool: greedy eval_posterior, no draw; `done`
+        [B] uint8/bool: a finished request - no draw, offset untouched, accept_len 0 and nothing else written; `n_nodes`
+        [B] int32: its own row count (-1 wraps to its last row); `depth` [B] int32: its own path width.  `out`: the dict
+        of a previous call (or of the same layout) whose tensors are written instead of new ones, so that a call
+        captured in a CUDA graph allocates nothing."""
         assert logits.is_cuda and logits.dim() == 3 and logits.stride(2) == 1
         B, T, V = logits.shape
         dt = {torch.bfloat16: K.DTYPE_BF16, torch.float16: K.DTYPE_FP16, torch.float32: K.DTYPE_FP32}.get(logits.dtype)
@@ -650,20 +660,56 @@ class Verifier:
         else:
             a.retrieve_dev, a.n_paths, a.depth, a.retrieve_batch_stride, width = None, 1, T, 0, T
         a.n_paths_dev = K.ptr(_i32(n_paths)) if n_paths is not None else None
-        a.temperature, a.top_p, a.top_k = float(temperature), float(top_p), int(top_k)
+        r = K.SampleRequestArgs()
+
+        def per_request(v, dtype, what):
+            if not torch.is_tensor(v):
+                return v, None
+            assert v.dtype == dtype and v.is_cuda and v.is_contiguous() and v.numel() == B, f"{what}: [B] {dtype} CUDA tensor"
+            return 1.0 if what == "temperature" else 0, v.data_ptr()
+
+        t_val, r.temperature_dev = per_request(temperature, torch.float32, "temperature")
+        p_val, r.top_p_dev = per_request(top_p, torch.float32, "top_p")
+        k_val, r.top_k_dev = per_request(top_k, torch.int32, "top_k")
+        a.temperature, a.top_p, a.top_k = float(t_val), float(p_val), int(k_val)
+        for name, t in (("greedy", greedy), ("done", done)):
+            if t is not None:
+                assert t.dtype in (torch.bool, torch.uint8) and t.is_cuda and t.is_contiguous() and t.numel() == B, name
+            setattr(r, name + "_dev", K.ptr(t))
+        r.n_nodes_dev = K.ptr(_i32(n_nodes)) if n_nodes is not None else None
+        r.depth_dev = K.ptr(_i32(depth)) if depth is not None else None
         a.seeds_dev, a.offsets_dev = seeds.data_ptr(), offsets.data_ptr()
-        mk = lambda *s: torch.empty(*s, dtype=torch.int32, device=logits.device)
-        out = dict(best=mk(B), accept_len=mk(B), next_token=mk(B), tokens=mk(B, width), indices=mk(B, width))
+        if out is None or out["tokens"].shape != (B, width):
+            mk = lambda *s: torch.empty(*s, dtype=torch.int32, device=logits.device)
+            out = dict(best=mk(B), accept_len=mk(B), next_token=mk(B), tokens=mk(B, width), indices=mk(B, width))
         a.out_best_dev, a.out_accept_len_dev, a.out_next_token_dev = out["best"].data_ptr(), out["accept_len"].data_ptr(), out["next_token"].data_ptr()
         a.out_tokens_dev, a.out_indices_dev = out["tokens"].data_ptr(), out["indices"].data_ptr()
         if want_sample_p:
-            out["sample_p"] = torch.empty(B, V, dtype=torch.float32, device=logits.device)
+            if "sample_p" not in out or out["sample_p"].shape != (B, V):
+                out["sample_p"] = torch.empty(B, V, dtype=torch.float32, device=logits.device)
             a.out_sample_p_dev = out["sample_p"].data_ptr()
         else:
             a.out_sample_p_dev = None
+        per = any((r.temperature_dev, r.top_p_dev, r.top_k_dev, r.greedy_dev, r.done_dev, r.n_nodes_dev, r.depth_dev))
         with torch.cuda.device(self.device):
-            K.check(K.lib().samd_verify_sample(C.byref(a), K.stream_ptr()), "samd_verify_sample")
+            K.check(K.lib().samd_verify_sample_requests(C.byref(a), C.byref(r) if per else None, K.stream_ptr()),
+                    "samd_verify_sample")
         return out
+
+    def kv_compact(self, indices: torch.Tensor, accept_len: torch.Tensor, cache_len: torch.Tensor):
+        """samd_kv_compact on the bound cache: rows cache_len[b] + indices[b][j] -> cache_len[b] + j for j <
+        accept_len[b] (the layout verify_sample returns), then cache_len += accept_len.  One launch (two with rows)."""
+        assert self._kv_ptrs is not None, "kv_compact before bind_kv"
+        _i32(indices)
+        _i32(accept_len)
+        _i32(cache_len)
+        assert indices.dim() == 2 and indices.shape[0] == accept_len.numel() == cache_len.numel()
+        m = self._kv_meta
+        with torch.cuda.device(self.device):
+            K.check(K.lib().samd_kv_compact(self._kv_ptrs.data_ptr(), m["n_kv"], m["n_heads"], m["row_bytes"],
+                                            m["batch_stride"], m["head_stride"], m["pos_stride"], indices.data_ptr(),
+                                            indices.shape[1], accept_len.data_ptr(), cache_len.data_ptr(),
+                                            indices.shape[0], K.stream_ptr()), "samd_kv_compact")
 
     def close(self):
         if self._h:
