@@ -426,6 +426,39 @@ typedef struct samd_sample_request_args {
 } samd_sample_request_args;
 int samd_verify_sample_requests(const samd_sample_args *args, const samd_sample_request_args *r, void *stream);
 
+/* Per-token log-probabilities of the accepted path of every request, from the logits a verify launch read.  For request
+ * b with a = min(count_dev[b], width) >= 1 and not done, position j < a is scored on row r = indices_dev[b][j] (NULL
+ * indices: r = j; a -1 entry: the request's last live row n_nodes_dev[b] - 1, as samd_verify_compact reads it) against
+ * the target tokens_dev[b][j + 1] when j + 1 < a, else next_token_dev[b]:
+ *     logprob = log_softmax(float32(row))[target]      (raw: no temperature, top-p or top-k)
+ * and, with n_top > 0, the n_top largest entries of the row (value descending, index ascending, NaN largest) with their
+ * log-probabilities.  Positions j < a - 1 go to out_logprob_dev[b][j] / out_top_*[b][j][:], the last one to
+ * out_next_logprob_dev[b] / out_next_top_*[b][:].  A -inf logit gives -inf, a row with a NaN gives NaN, a target
+ * outside [0, V) gives NaN.  Requests with a = 0 or done write nothing, nor does any position j >= a.  Only the scored
+ * rows are read, each once.  The reduction order depends only on V and the launch shape, so a row gives bit-identical
+ * results wherever it sits; no argument depends on the step, so the launch can be captured in a CUDA graph. */
+typedef struct samd_logprob_args {
+    const void    *logits_dev;        /* [B][n_nodes][V], dtype below */
+    int32_t        dtype;             /* SAMD_DTYPE_* */
+    int32_t        batch, n_nodes, vocab;
+    int64_t        batch_stride, row_stride;       /* in elements */
+    const int32_t *indices_dev;       /* [B][width] path row indices (a verify launch's out_indices), or NULL = identity */
+    int32_t        width;             /* row length of indices_dev, tokens_dev and out_logprob_dev (<= n_nodes if identity) */
+    const int32_t *count_dev;         /* [B] scored positions (a verify launch's accept_len) */
+    const int32_t *tokens_dev;        /* [B][width] path tokens (out_tokens); may be NULL when every count is <= 1 */
+    const int32_t *next_token_dev;    /* [B] */
+    const int32_t *n_nodes_dev;       /* [B] live rows per request, or NULL = n_nodes */
+    const uint8_t *done_dev;          /* [B] 1 = finished: nothing written, or NULL */
+    int32_t        n_top;             /* 0 .. 8 */
+    float   *out_logprob_dev;         /* [B][width] (only NULL when width == 1) */
+    float   *out_next_logprob_dev;    /* [B] */
+    int32_t *out_top_ids_dev;         /* [B][width][n_top] (n_top > 0) */
+    float   *out_top_logprob_dev;     /* [B][width][n_top] */
+    int32_t *out_next_top_ids_dev;    /* [B][n_top] */
+    float   *out_next_top_logprob_dev;/* [B][n_top] */
+} samd_logprob_args;
+int samd_token_logprobs(const samd_logprob_args *args, void *stream);
+
 /* TokenRecycle.gen_draft (token_recycle.py:49-59) for a batch: tokens[b][0] = start_tok[b]; every other node takes
  * table[token of its parent][its rank among the parent's children], or 0 when the parent's token has no entry.
  * parent / rank: [n_nodes] device arrays describing the static tree (node 0 = root, parents before children);

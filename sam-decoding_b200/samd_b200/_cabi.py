@@ -69,6 +69,16 @@ class SampleRequestArgs(C.Structure):
     ]
 
 
+class LogprobArgs(C.Structure):
+    _fields_ = [
+        ("logits_dev", vp), ("dtype", C.c_int32), ("batch", C.c_int32), ("n_nodes", C.c_int32), ("vocab", C.c_int32),
+        ("batch_stride", C.c_int64), ("row_stride", C.c_int64), ("indices_dev", vp), ("width", C.c_int32),
+        ("count_dev", vp), ("tokens_dev", vp), ("next_token_dev", vp), ("n_nodes_dev", vp), ("done_dev", vp),
+        ("n_top", C.c_int32), ("out_logprob_dev", vp), ("out_next_logprob_dev", vp), ("out_top_ids_dev", vp),
+        ("out_top_logprob_dev", vp), ("out_next_top_ids_dev", vp), ("out_next_top_logprob_dev", vp),
+    ]
+
+
 class AssembleArgs(C.Structure):
     _fields_ = [
         ("batch", C.c_int32), ("n_nodes", C.c_int32), ("n_paths", C.c_int32), ("depth", C.c_int32), ("type_dev", vp),
@@ -150,6 +160,7 @@ SYMBOLS = {
     "samd_verify_compact": (C.c_int, [vp, C.POINTER(VerifyArgs), vp]),
     "samd_verify_sample": (C.c_int, [C.POINTER(SampleArgs), vp]),
     "samd_verify_sample_requests": (C.c_int, [C.POINTER(SampleArgs), C.POINTER(SampleRequestArgs), vp]),
+    "samd_token_logprobs": (C.c_int, [C.POINTER(LogprobArgs), vp]),
     "samd_recycle_gen_tree": (C.c_int, [vp, C.c_int32, vp, vp, C.c_int32, vp, vp, C.c_int32, C.c_int32, vp, vp]),
     "samd_verify_set_chunk": (None, [C.c_int]),
     "samd_verify_set_overlap": (None, [C.c_int]),

@@ -34,6 +34,11 @@ top-k and a seed per request, as the reference's SamdGenerationConfig(greedy=Fal
 samd_verify_sample_requests with every slot's own processor and Philox stream, and the first token of a request is drawn
 from the plain softmax of its prompt's last row.  A request's tokens depend only on its prompt, its parameters and its
 seed - not on its slot, its neighbours, the batch size, graph or eager execution, check_every, or a prefix pool.
+
+generate(..., logprobs=n) and serve(..., logprobs=n) also return every emitted token's raw log-probability and its n best
+alternatives (n in [0, 8]).  After the verify launch, one samd_token_logprobs launch scores the accepted rows of the step's
+logits; each slot carries the log-probability of its start token (predicted by the previous step's last accepted row,
+or at admission by the prompt's last row), and the commit writes them beside the tokens with the same truncation.
 """
 from __future__ import annotations
 
@@ -75,6 +80,20 @@ class SamplingParams:
         if not isinstance(self.seed, int) or not 0 <= self.seed < 2 ** 63:
             return f"seed must be an int in [0, 2**63), got {self.seed!r}"
         return None
+
+
+def _check_logprobs(logprobs) -> Optional[int]:
+    """generate() / serve()'s `logprobs`: None, or the number of alternatives per token, an int in [0, 8]."""
+    if logprobs is not None and (isinstance(logprobs, bool) or not isinstance(logprobs, int) or not 0 <= logprobs <= 8):
+        raise K.SamdError(f"logprobs must be None or an int in [0, 8], got {logprobs!r}")
+    return logprobs
+
+
+def _logprob_lists(rows: torch.Tensor, n: int) -> tuple:
+    """One finished request's host rows [L, 1 + 2n] (log-probability | top-n values | top-n ids) as serve() returns them:
+    (logprobs, top_logprobs as n (token_id, logprob) pairs per token, or None for n = 0)."""
+    top = [list(zip(i, v)) for i, v in zip(rows[:, 1 + n:].long().tolist(), rows[:, 1:1 + n].tolist())] if n else None
+    return rows[:, 0].tolist(), top
 
 
 class _Layer(CacheLayerMixin):
@@ -270,16 +289,18 @@ class BatchedSamdDecoder:
         mask = torch.zeros(B, T, kv_len, dtype=self.dtype, device=dev)
         mask.masked_fill_(~ok, torch.finfo(self.dtype).min)
         logits = self.lm(input_ids=draft.long(), position_ids=pos, past_key_values=self.cache,
-                         attention_mask=mask[:, None]).logits
+                         attention_mask=mask[:, None]).logits.contiguous()
         if not self.ver_bound:
             self.ver.bind_kv([self.cache.kv[i] for i in range(self.cache.kv.shape[0])])
             self.ver_bound = True
-        return self.ver.verify(logits.contiguous(), draft, self._ret[kind].contiguous(), cache_len=self.cache.cache_len,
-                               move_kv=True, n_nodes=self._n_nodes[kind].contiguous(), n_paths=self._n_paths[kind].contiguous(),
-                               out=res, recycle=self.table)
+        n_nodes = self._n_nodes[kind].contiguous()
+        return self.ver.verify(logits, draft, self._ret[kind].contiguous(), cache_len=self.cache.cache_len,
+                               move_kv=True, n_nodes=n_nodes, n_paths=self._n_paths[kind].contiguous(),
+                               out=res, recycle=self.table), logits, n_nodes
 
-    def _draft_forward_verify(self, kv_len: int) -> dict:
-        """Drafts in, LM forward, fused verify: the part of a step that depends on the draft flavour."""
+    def _draft_forward_verify(self, kv_len: int) -> tuple:
+        """Drafts in, LM forward, fused verify: the part of a step that depends on the draft flavour.  Returns the verify
+        outputs, the logits they were computed from and every request's live row count (None: all T rows)."""
         st, T, cache = self._st, self.T, self.cache
         self.eng.step(st["acc_tokens"], st["acc_count"], st["start"])              # update(accepted) + lookup(start): one launch
         cache.begin(T, kv_len)
@@ -289,10 +310,10 @@ class BatchedSamdDecoder:
         draft[:, 0] = st["start"]                                                  # short matches verify the start token only
         pos = cache.cache_len.long()[:, None] + self._ar[None, :]
         logits = self.lm(input_ids=draft.long(), position_ids=pos, past_key_values=cache,
-                         attention_mask=self._mask(T, kv_len, cache.cache_len)).logits
+                         attention_mask=self._mask(T, kv_len, cache.cache_len)).logits.contiguous()
         if self._sampled:                                      # identity path: no row moves, the commit sets cache_len
-            return self._verify_sample(logits.contiguous(), draft, None)
-        return self.ver.verify(logits.contiguous(), draft, None, cache_len=cache.cache_len, out=st["res"])
+            return self._verify_sample(logits, draft, None), logits, None
+        return self.ver.verify(logits, draft, None, cache_len=cache.cache_len, out=st["res"]), logits, None
 
     def _verify_sample(self, logits: torch.Tensor, tokens: torch.Tensor, retrieve: Optional[torch.Tensor], **kw) -> dict:
         """samd_verify_sample_requests with every slot's processor, greedy flag and Philox stream; finished slots make no
@@ -308,12 +329,21 @@ class BatchedSamdDecoder:
         # a request whose step could run past the cache is finished (samd_model.py:251-254)
         st["done"].logical_or_(cache.cache_len + T > cache.max_len)
         saved_len = cache.cache_len.clone()
-        res = st["res"] = self._draft_forward_verify(kv_len)
-        self._commit(res, saved_len)
+        res, logits, n_nodes = self._draft_forward_verify(kv_len)
+        st["res"] = res
+        lp = None
+        if self._logprobs is not None:                     # the accepted rows' log-probabilities: one more launch
+            n = self._logprobs
+            lp = self._lp_res[n] = self.ver.token_logprobs(logits, res["indices"], res["accept_len"], res["tokens"],
+                                                           res["next_token"], n_top=n, n_nodes=n_nodes, done=st["done"],
+                                                           out=self._lp_res.get(n))
+        self._commit(res, saved_len, lp)
 
-    def _commit(self, res: dict, saved_len: torch.Tensor):
+    def _commit(self, res: dict, saved_len: torch.Tensor, lp: Optional[dict] = None):
         """EOS truncation, emission up to each slot's own limit, cache lengths, the next step's inputs, history and the
-        host flag."""
+        host flag.  With `lp` (token_logprobs of this step) the emitted tokens' log-probabilities go to the columns of
+        st["lp"] (and top-n lists to st["lp_ids"] / st["lp_top"]) parallel to st["out"]: emitted token 0 is the start
+        token, predicted by the previous step's last row (st["start_lp"]), token k >= 1 is scored position k - 1."""
         st, cache = self._st, self.cache
         done = st["done"]
         n_acc = torch.where(done, torch.zeros_like(res["accept_len"]), res["accept_len"])
@@ -328,8 +358,10 @@ class BatchedSamdDecoder:
         out = st["out"]
         cols = st["out_len"].long()[:, None] + ar[None, :]
         keep = ar[None, :] < n_emit[:, None]
-        out.scatter_(1, torch.where(keep, cols, torch.full_like(cols, out.shape[1] - 1)),
-                     torch.where(keep, res["tokens"], torch.zeros_like(res["tokens"])))
+        cols = torch.where(keep, cols, torch.full_like(cols, out.shape[1] - 1))
+        out.scatter_(1, cols, torch.where(keep, res["tokens"], torch.zeros_like(res["tokens"])))
+        if lp is not None:
+            self._commit_logprobs(lp, cols, keep)
         st["out_len"].add_(n_emit)
         done.logical_or_(st["out_len"] >= st["limit"])
         cache.cache_len.copy_(saved_len + n_acc)                                   # finished requests stop advancing
@@ -344,6 +376,21 @@ class BatchedSamdDecoder:
         st["hlen"].add_(live.to(torch.int32))
         # what the host reads every `check_every` steps: [done (B) | out_len (B) | longest cache]
         torch.cat((done.to(torch.int32), st["out_len"], cache.cache_len.max()[None]), out=st["flag"])
+
+    def _commit_logprobs(self, lp: dict, cols: torch.Tensor, keep: torch.Tensor):
+        """_commit's emission of the log-probabilities (and top-n lists) into the columns `cols` where `keep`, then the
+        carry of the next start token's."""
+        st, n, W = self._st, self._logprobs, cols.shape[1]
+        step = torch.cat((st["start_lp"][:, None], lp["logprob"][:, :W - 1]), 1)
+        st["lp"].scatter_(1, cols, torch.where(keep, step, torch.zeros_like(step)))
+        st["start_lp"].copy_(lp["next_logprob"])
+        if n:
+            c, k = cols[:, :, None].expand(-1, -1, n), keep[:, :, None]
+            for dst, start, top, nxt in (("lp_ids", "start_ids", "top_ids", "next_top_ids"),
+                                         ("lp_top", "start_top", "top_logprob", "next_top_logprob")):
+                step = torch.cat((st[start][:, None, :n], lp[top][:, :W - 1]), 1)
+                st[dst][:, :, :n].scatter_(1, c, torch.where(k, step, torch.zeros_like(step)))
+                st[start][:, :n].copy_(lp[nxt])
 
     def _prefill_hook(self, ids: torch.Tensor, lens: torch.Tensor, logits: torch.Tensor):
         """After the prompt's forward and automaton update: TokenRecycle.update over the prompt rows (tree mode)."""
@@ -364,10 +411,11 @@ class BatchedSamdDecoder:
         return {}
 
     # ---- the step state, and the CUDA graphs that refer to it -------------------------------------------------------
-    def _init_state(self, max_limit: int):
+    def _init_state(self, max_limit: int, logprobs: bool = False):
         """Zeroed step state for requests of at most `max_limit` new tokens.  The tensors persist across calls (the
         captured graphs refer to them, and limits are per slot); they are reallocated, and the graphs dropped, only when
-        a call needs longer outputs than any before."""
+        a call needs longer outputs than any before.  The log-probability state is added by the first call that asks
+        for log-probabilities."""
         B, T, dev = self.B, self.T, self.device
         width = T if self.tree is None else self._ret.shape[2]
         cap = getattr(self, "_st_cap", None)
@@ -382,19 +430,26 @@ class BatchedSamdDecoder:
                             top_k=mk(B), greedy=torch.zeros(B, dtype=torch.uint8, device=dev),
                             seed=torch.zeros(B, dtype=torch.long, device=dev), offset=torch.zeros(B, dtype=torch.long, device=dev),
                             res=None, **self._extra_state(mk))
-            self._st_cap, self._graphs = max_limit, {}
+            self._st_cap, self._graphs, self._lp_res = max_limit, {}, {}
         else:
             for k, v in self._st.items():
                 if k != "res":
                     v.zero_()
+        if logprobs and "lp" not in self._st:
+            # lp / lp_top / lp_ids: parallel to out (top-n lists at their widest, 8, so that a call with any n reuses
+            # them); start_*: those of each slot's start token, carried from the step that predicted it
+            W, f32 = self._st["out"].shape[1], lambda *sh: torch.zeros(*sh, device=dev)
+            i32 = lambda *sh: torch.zeros(*sh, dtype=torch.int32, device=dev)
+            self._st.update(lp=f32(B, W), lp_top=f32(B, W, 8), lp_ids=i32(B, W, 8), start_lp=f32(B), start_top=f32(B, 8),
+                            start_ids=i32(B, 8))
 
     def _advance(self, kv_len: int, graph: bool) -> bool:
         """One decode step at key length `kv_len`: the bucket's CUDA graph, captured first if it is new, or the same body
-        eagerly (one graph per bucket and greedy / sampled body).  Returns `graph`, False from then on when the LM's forward
-        cannot be captured."""
+        eagerly (one graph per bucket, greedy / sampled body and logprobs setting).  Returns `graph`, False from then on
+        when the LM's forward cannot be captured."""
         if graph:
             B, dev, graphs = self.B, self.device, self._graphs
-            key = (kv_len, self._sampled)
+            key = (kv_len, self._sampled, self._logprobs)
             if key not in graphs:
                 # warm-up run on a side stream (allocations, lazy initialisation), state restored, then the capture
                 snap = {k: (v.clone() if torch.is_tensor(v) else v) for k, v in self._st.items() if k != "res"}
@@ -650,8 +705,8 @@ class BatchedSamdDecoder:
     def _set_slots(self, slots: torch.Tensor, lens: torch.Tensor, limits: torch.Tensor, rows: torch.Tensor,
                    params: List[Optional[SamplingParams]]):
         """The admitted slots' step state: cache length, sampling parameters and a fresh Philox stream (sampled calls),
-        first start token from `rows` [n, V] (the logits after each prompt: argmax, or a draw from the plain softmax),
-        limit, and zero emitted tokens / history."""
+        first start token from `rows` [n, V] (the logits after each prompt: argmax, or a draw from the plain softmax)
+        and, with logprobs, its log-probability, limit, and zero emitted tokens / history."""
         st = self._st
         self.cache.cache_len.index_copy_(0, slots, lens)
         if self._sampled:
@@ -675,6 +730,14 @@ class BatchedSamdDecoder:
             first = res["next_token"]
         else:
             first = rows.argmax(-1).to(torch.int32)
+        if self._logprobs is not None:                     # the first token's log-probability, from the same row
+            n, (m, V) = self._logprobs, rows.shape
+            lp = self.ver.token_logprobs(rows.contiguous().view(m, 1, V), None,
+                                         torch.ones(m, dtype=torch.int32, device=self.device), None, first, n_top=n)
+            st["start_lp"].index_copy_(0, slots, lp["next_logprob"])
+            if n:
+                st["start_ids"][slots, :n] = lp["next_top_ids"]
+                st["start_top"][slots, :n] = lp["next_top_logprob"]
         st["start"].index_copy_(0, slots, first)
         st["limit"].index_copy_(0, slots, limits)
         for k in ("acc_count", "out_len", "hlen"):
@@ -682,18 +745,20 @@ class BatchedSamdDecoder:
         st["done"].index_fill_(0, slots, False)
 
     # ---- the decode loop of generate() and serve() --------------------------------------------------------------------
-    def _run(self, requests: Iterator[tuple], max_limit: int, graph: bool, check_every: int, sampled: bool = False):
+    def _run(self, requests: Iterator[tuple], max_limit: int, graph: bool, check_every: int, sampled: bool = False,
+             logprobs: Optional[int] = None):
         """Decode the validated requests (index, prompt, limit, SamplingParams or None) of `requests`, at most B at a
-        time, with the greedy step body or (sampled) the sampled one.  The decode step has
-        no host synchronisation in it: it is captured once per key-length bucket (64 positions) as a CUDA graph and
-        replayed.  Once every `check_every` steps the host reads [done | out_len | longest cache] in one copy; it then
-        yields (index, tokens, accept_lengths, slot) for every request found finished (their rows in one more copy),
+        time, with the greedy step body or (sampled) the sampled one; with `logprobs` (0 .. 8) the step also scores the
+        accepted rows.  The decode step has no host synchronisation in it: it is captured once per key-length bucket (64
+        positions) as a CUDA graph and replayed.  Once every `check_every` steps the host reads [done | out_len | longest cache] in one copy; it then
+        yields (index, tokens, accept_lengths, slot, (logprobs, top_logprobs) or None) for every request found finished
+        (their rows in one more copy, their log-probabilities in one more),
         admits queued requests into the free slots, and sizes the next steps' key length from the longest cache.  A
         finished request keeps its slot - riding along, emitting nothing - until that check.  Statistics go to
         self._run_stats."""
         B, T, dev = self.B, self.T, self.device
-        self._init_state(max_limit)
-        self._sampled = sampled
+        self._init_state(max_limit, logprobs is not None)
+        self._sampled, self._logprobs = sampled, logprobs
         st = self._st
         run = self._run_id = getattr(self, "_run_id", 0) + 1
         self.eng.reset()
@@ -737,11 +802,17 @@ class BatchedSamdDecoder:
             if fin:
                 idx = torch.tensor(fin, device=dev)
                 rows = torch.cat((st["out"][idx], st["hist"][idx], st["hlen"][idx, None]), 1).tolist()
-                for b, r in zip(fin, rows):
+                lps = [None] * len(fin)
+                if logprobs is not None:                   # [f, W, 1 + 2n]: log-probability | top-n values | top-n ids
+                    n = logprobs
+                    lpr = torch.cat((st["lp"][idx, :, None], st["lp_top"][idx, :, :n], st["lp_ids"][idx, :, :n].float()),
+                                    2).cpu()
+                    lps = [_logprob_lists(lpr[k, :flag[B + b]], n) for k, b in enumerate(fin)]
+                for b, r, lp in zip(fin, rows, lps):
                     i, owner[b] = owner[b], None
                     hist = r[W:W + r[-1]]
                     live_steps += len(hist)
-                    yield i, r[:flag[B + b]], hist, b
+                    yield i, r[:flag[B + b]], hist, b, lp
                     if self._run_id != run:
                         raise K.SamdError("the decoder ran another generate() / serve() while this serve() was suspended")
             kv_hi = max(kv_hi, admit())
@@ -752,13 +823,15 @@ class BatchedSamdDecoder:
 
     @torch.inference_mode()
     def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4,
-                 sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None):
+                 sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None, logprobs: Optional[int] = None):
         """Lossless batched speculative decoding of exactly B prompts in lockstep (request b in slot b), up to
         max_new_tokens each.  The host reads the finished flags once every `check_every` steps - 1 / check_every host
         syncs per step - so a finished batch may run up to check_every - 1 idle steps (every request done: nothing is
         emitted).  graph=False runs the same body eagerly.  Returns (tokens per request, stats); stats["accept_lengths"]
-        holds every request's accepted tokens per step, padded with 0 to the longest request's `steps`.  `sampling`: as
-        in serve()."""
+        holds every request's accepted tokens per step, padded with 0 to the longest request's `steps`.  `sampling` and
+        `logprobs`: as in serve(); with logprobs, stats["logprobs"] (and, for logprobs > 0, stats["top_logprobs"]) hold
+        every request's list."""
+        logprobs = _check_logprobs(logprobs)
         B, T = self.B, self.T
         assert len(prompts) == B
         n_max = max(len(p) for p in prompts)
@@ -770,17 +843,23 @@ class BatchedSamdDecoder:
             raise K.SamdError(f"prompt + max_new_tokens + one step = {n_max + max_new_tokens + T} exceeds the automaton "
                               f"capacity max_tokens={self.dyn.max_tokens}")
         reqs = self._with_sampling(((i, p, max_new_tokens) for i, p in enumerate(prompts)), sampling)
-        out, acc = [None] * B, [None] * B
-        for i, tokens, hist, _ in self._run(reqs, max_new_tokens, graph, check_every, sampling is not None):
-            out[i], acc[i] = tokens, hist
+        out, acc, lps = [None] * B, [None] * B, [None] * B
+        for i, tokens, hist, _, lp in self._run(reqs, max_new_tokens, graph, check_every, sampling is not None, logprobs):
+            out[i], acc[i], lps[i] = tokens, hist, lp
         n_live = max(len(a) for a in acc)
         s = self._run_stats
-        return out, dict(steps=n_live, steps_run=s["steps_run"], host_syncs=s["host_syncs"], graphed=s["graphed"],
-                         graphs=s["graphs"], accept_lengths=[a + [0] * (n_live - len(a)) for a in acc], **self._extra_stats())
+        stats = dict(steps=n_live, steps_run=s["steps_run"], host_syncs=s["host_syncs"], graphed=s["graphed"],
+                     graphs=s["graphs"], accept_lengths=[a + [0] * (n_live - len(a)) for a in acc], **self._extra_stats())
+        if logprobs is not None:
+            stats["logprobs"] = [lp[0] for lp in lps]
+            if logprobs:
+                stats["top_logprobs"] = [lp[1] for lp in lps]
+        return out, stats
 
     @torch.inference_mode()
     def serve(self, prompts: Iterable[Sequence[int]], max_new_tokens: Union[int, Sequence[int]], graph: bool = True,
-              check_every: int = 4, sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None):
+              check_every: int = 4, sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None,
+              logprobs: Optional[int] = None):
         """Continuous batching: decode any number of requests through the B slots, refilling a slot with the next queued
         request as soon as the host sees its request finished (once every `check_every` steps).  `prompts` is consumed
         lazily and in order; `max_new_tokens` is one limit for all or a sequence with one per request.  Yields
@@ -799,7 +878,15 @@ class BatchedSamdDecoder:
         `sampling` (None: greedy, lossless): one SamplingParams for every request - request i then uses the Philox key
         seed + i - or a sequence with one per request.  Each request's processor and stream are its own, so its tokens
         depend only on its prompt, parameters and seed; a request with greedy=True decodes greedily.  Not with
-        Token-Recycle tree mode (tree=): SamdError."""
+        Token-Recycle tree mode (tree=): SamdError.
+
+        `logprobs` (None: none): an int n in [0, 8].  info["logprobs"] then holds the model's raw log-probability of every
+        token in `tokens`, log_softmax(logits)[token] of the row that predicted it - no temperature, top-p or top-k, in
+        greedy and sampled decoding alike - and, for n > 0, info["top_logprobs"] the n most likely tokens at each of
+        those positions as (token_id, logprob) pairs (value descending, lowest id first among equals).  They are scored
+        on the device from the logits the decode step already computed (one samd_token_logprobs launch per step and per
+        admission); the tokens are the same as without."""
+        logprobs = _check_logprobs(logprobs)
         self.serve_stats = None
         if hasattr(max_new_tokens, "__len__"):
             limits = [int(x) for x in max_new_tokens]
@@ -807,10 +894,15 @@ class BatchedSamdDecoder:
         else:
             limits, max_limit = None, int(max_new_tokens)
         reqs = self._with_sampling(self._requests(prompts, max_new_tokens if limits is None else limits), sampling)
-        for i, tokens, hist, slot in self._run(reqs, max(max_limit, 1), graph, check_every, sampling is not None):
+        for i, tokens, hist, slot, lp in self._run(reqs, max(max_limit, 1), graph, check_every, sampling is not None,
+                                                   logprobs):
             info = {"slot": slot, "accept_lengths": hist}
             if self._prefixes is not None:
                 info["prefix_len"] = self._slot_plen[slot]
+            if lp is not None:
+                info["logprobs"] = lp[0]
+                if logprobs:
+                    info["top_logprobs"] = lp[1]
             yield i, tokens, info
         self.serve_stats = dict(self._run_stats)
 
@@ -929,7 +1021,7 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
     def mask_view(self, kv_len: int) -> torch.Tensor:
         return self.buf["mask"][:self.B * self.T * kv_len].view(self.B, self.T, kv_len)
 
-    def _draft_forward_verify(self, kv_len: int) -> dict:
+    def _draft_forward_verify(self, kv_len: int) -> tuple:
         st, T, cache, eng, buf = self._st, self.T, self.cache, self.eng, self.buf
         eng.step(st["acc_tokens"], st["acc_count"], st["start"])
         if eng.static is not None:
@@ -940,14 +1032,14 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
                      mask, done=st["done"])
         cache.begin(T, kv_len)
         logits = self.lm(input_ids=buf["tokens"].long(), position_ids=buf["position_ids"], past_key_values=cache,
-                         attention_mask=mask[:, None]).logits
+                         attention_mask=mask[:, None]).logits.contiguous()
         if self._sampled:
             # a request's own width - its draft length, or its tree's deepest path - so that the -1 pads beyond it are
             # never compared; then the accepted rows move into place
             torch.amax((buf["retrieve"] >= 0).sum(2, dtype=torch.int32), 1, out=buf["depth"])
-            res = self._verify_sample(logits.contiguous(), buf["tokens"], buf["retrieve"], n_paths=buf["n_paths"],
+            res = self._verify_sample(logits, buf["tokens"], buf["retrieve"], n_paths=buf["n_paths"],
                                       n_nodes=buf["n_nodes"], depth=buf["depth"])
             self.ver.kv_compact(res["indices"], res["accept_len"], cache.cache_len)
-            return res
-        return self.ver.verify(logits.contiguous(), buf["tokens"], buf["retrieve"], cache_len=cache.cache_len, move_kv=True,
-                               n_nodes=buf["n_nodes"], n_paths=buf["n_paths"], out=st["res"])
+            return res, logits, buf["n_nodes"]
+        return self.ver.verify(logits, buf["tokens"], buf["retrieve"], cache_len=cache.cache_len, move_kv=True,
+                               n_nodes=buf["n_nodes"], n_paths=buf["n_paths"], out=st["res"]), logits, buf["n_nodes"]

@@ -696,6 +696,65 @@ class Verifier:
                     "samd_verify_sample")
         return out
 
+    def token_logprobs(self, logits: torch.Tensor, indices: Optional[torch.Tensor], count: torch.Tensor,
+                       tokens: Optional[torch.Tensor], next_token: torch.Tensor, n_top: int = 0,
+                       n_nodes: Optional[torch.Tensor] = None, done: Optional[torch.Tensor] = None,
+                       out: Optional[dict] = None) -> dict:
+        """samd_token_logprobs: the raw log-probability log_softmax(float32(row))[target] of every accepted token, one
+        launch.  `indices` / `count` / `tokens` / `next_token`: a verify call's "indices" [B, W] (None: the identity
+        path), "accept_len", "tokens" [B, W] (None when every count is <= 1) and "next_token".  Position j < count[b] is
+        scored on row indices[b][j] (-1: row n_nodes[b] - 1) against tokens[b][j + 1], the last one against
+        next_token[b].  Returns out["logprob"] [B, W] (positions j < count - 1) and out["next_logprob"] [B] (the last
+        position), and with n_top in 1..8 also out["top_ids"] / out["top_logprob"] [B, W, n_top] and out["next_top_ids"]
+        / out["next_top_logprob"] [B, n_top]: the n_top largest entries of the row (value descending, index ascending,
+        NaN largest).  `done` [B] uint8/bool: finished requests write nothing, nor does any position past count.  `out`:
+        the dict of a previous call with the same shapes, written instead of new tensors (a captured call allocates
+        nothing)."""
+        if isinstance(n_top, bool) or not isinstance(n_top, int) or not 0 <= n_top <= 8:
+            raise K.SamdError(f"token_logprobs: n_top must be an int in [0, 8], got {n_top!r}")
+        if logits.dim() != 3 or logits.stride(2) != 1:
+            raise K.SamdError(f"token_logprobs: logits must be [B, T, V] with unit stride over V, got {tuple(logits.shape)}")
+        B, T, V = logits.shape
+        dt = {torch.bfloat16: K.DTYPE_BF16, torch.float16: K.DTYPE_FP16, torch.float32: K.DTYPE_FP32}.get(logits.dtype)
+        if dt is None:
+            raise K.SamdError(f"token_logprobs: unsupported logits dtype {logits.dtype} (bf16 / fp16 / fp32)")
+        width = indices.shape[1] if indices is not None else tokens.shape[1] if tokens is not None else T
+        for name, t, shape, dtypes in (("indices", indices, (B, width), (torch.int32,)),
+                                       ("tokens", tokens, (B, width), (torch.int32,)),
+                                       ("count", count, (B,), (torch.int32,)), ("next_token", next_token, (B,), (torch.int32,)),
+                                       ("n_nodes", n_nodes, (B,), (torch.int32,)),
+                                       ("done", done, (B,), (torch.bool, torch.uint8))):
+            if t is None:
+                continue
+            if tuple(t.shape) != shape or t.dtype not in dtypes or not t.is_contiguous():
+                raise K.SamdError(f"token_logprobs: {name} must be a contiguous {shape} {dtypes[0]} tensor, got "
+                                  f"{tuple(t.shape)} {t.dtype}")
+        if indices is None and width > T:
+            raise K.SamdError(f"token_logprobs: an identity path of width {width} needs {width} logits rows, got {T}")
+        if not all(t.is_cuda for t in (logits, count, next_token) + tuple(x for x in (indices, tokens, n_nodes, done)
+                                                                          if x is not None)):
+            raise K.SamdError("token_logprobs: every tensor must be on the GPU")
+        f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=logits.device)
+        i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=logits.device)
+        top_shape = out["top_ids"].shape if out is not None and "top_ids" in out else None
+        if out is None or out["logprob"].shape != (B, width) or top_shape != ((B, width, n_top) if n_top else None):
+            out = dict(logprob=f32(B, width), next_logprob=f32(B))
+            if n_top:
+                out.update(top_ids=i32(B, width, n_top), top_logprob=f32(B, width, n_top), next_top_ids=i32(B, n_top),
+                           next_top_logprob=f32(B, n_top))
+        a = K.LogprobArgs()
+        a.logits_dev, a.dtype, a.batch, a.n_nodes, a.vocab = logits.data_ptr(), dt, B, T, V
+        a.batch_stride, a.row_stride = logits.stride(0), logits.stride(1)
+        a.indices_dev, a.width, a.count_dev = K.ptr(indices), width, count.data_ptr()
+        a.tokens_dev, a.next_token_dev, a.n_nodes_dev, a.done_dev = K.ptr(tokens), next_token.data_ptr(), K.ptr(n_nodes), K.ptr(done)
+        a.n_top, a.out_logprob_dev, a.out_next_logprob_dev = n_top, out["logprob"].data_ptr(), out["next_logprob"].data_ptr()
+        if n_top:
+            a.out_top_ids_dev, a.out_top_logprob_dev = out["top_ids"].data_ptr(), out["top_logprob"].data_ptr()
+            a.out_next_top_ids_dev, a.out_next_top_logprob_dev = out["next_top_ids"].data_ptr(), out["next_top_logprob"].data_ptr()
+        with torch.cuda.device(self.device):
+            K.check(K.lib().samd_token_logprobs(C.byref(a), K.stream_ptr()), "samd_token_logprobs")
+        return out
+
     def kv_compact(self, indices: torch.Tensor, accept_len: torch.Tensor, cache_len: torch.Tensor):
         """samd_kv_compact on the bound cache: rows cache_len[b] + indices[b][j] -> cache_len[b] + j for j <
         accept_len[b] (the layout verify_sample returns), then cache_len += accept_len.  One launch (two with rows)."""
