@@ -459,6 +459,38 @@ typedef struct samd_logprob_args {
 } samd_logprob_args;
 int samd_token_logprobs(const samd_logprob_args *args, void *stream);
 
+/* Repetition, presence and frequency penalties on the draft rows of a batch, in place, before a verify launch reads them
+ * (HF RepetitionPenaltyLogitsProcessor; presence / frequency as in the OpenAI API).  Row j < n_nodes_dev[b] of row-batch
+ * b belongs to state row s = slots_dev[b] (NULL: s = b); its context is the prompt, the emitted tokens and the node tokens
+ * on the path from node 0 to node j, both included (NULL tokens_dev: no draft context, e.g. the prompt's last row).  With
+ * c[t] = the output count counts_dev[s][t] & 0x7FFFFFFF plus the occurrences of t on that path, and seen[t] = bit 31 of
+ * counts_dev[s][t] (t is in the prompt) or c[t] > 0, every seen entry becomes, in fp32, each operation rounded on its own:
+ *     x = x < 0 ? x * r : x / r;   x = x - f * (float)c[t];   x = x - p * (c[t] > 0 ? 1 : 0)
+ * and is rounded to nearest into the logits dtype (-inf stays -inf, NaN stays NaN).  Untouched: unseen entries, requests
+ * with r = 1 and p = f = 0, done requests, rows at or past n_nodes_dev[b], and, with a path table, rows on none of the
+ * request's first n_paths_dev[b] paths (a path ends at its first -1).  Each entry is rewritten at most once, from its own
+ * inputs, so the results do not depend on the launch shape; no argument depends on the step, so the launch can be
+ * captured in a CUDA graph. */
+typedef struct samd_penalty_args {
+    void          *logits_dev;        /* [B][n_nodes][V], dtype below, rewritten in place */
+    int32_t        dtype;             /* SAMD_DTYPE_* */
+    int32_t        batch, n_nodes, vocab;          /* n_nodes <= 256 */
+    int64_t        batch_stride, row_stride;       /* in elements */
+    const int32_t *tokens_dev;        /* [B][n_nodes] node tokens, or NULL = no row has draft context */
+    const int32_t *retrieve_dev;      /* [B][n_paths][depth] path table, -1 padded, or NULL = the identity chain */
+    int32_t        n_paths, depth;
+    const int32_t *n_nodes_dev;       /* [B] live rows per request, or NULL = n_nodes */
+    const int32_t *n_paths_dev;       /* [B] live paths per request, or NULL = n_paths */
+    const uint8_t *done_dev;          /* [B] 1 = finished: not touched, or NULL */
+    const int32_t *slots_dev;         /* [B] state row of each row-batch entry, or NULL = identity */
+    int32_t        n_slots;           /* S */
+    const int32_t *counts_dev;        /* [S][V] output count (bits 0..30) | seen in the prompt (bit 31) */
+    const float   *repetition_dev;    /* [S] r > 0 */
+    const float   *presence_dev;      /* [S] p */
+    const float   *frequency_dev;     /* [S] f */
+} samd_penalty_args;
+int samd_apply_penalties(const samd_penalty_args *args, void *stream);
+
 /* TokenRecycle.gen_draft (token_recycle.py:49-59) for a batch: tokens[b][0] = start_tok[b]; every other node takes
  * table[token of its parent][its rank among the parent's children], or 0 when the parent's token has no entry.
  * parent / rank: [n_nodes] device arrays describing the static tree (node 0 = root, parents before children);

@@ -79,6 +79,16 @@ class LogprobArgs(C.Structure):
     ]
 
 
+class PenaltyArgs(C.Structure):
+    _fields_ = [
+        ("logits_dev", vp), ("dtype", C.c_int32), ("batch", C.c_int32), ("n_nodes", C.c_int32), ("vocab", C.c_int32),
+        ("batch_stride", C.c_int64), ("row_stride", C.c_int64), ("tokens_dev", vp), ("retrieve_dev", vp),
+        ("n_paths", C.c_int32), ("depth", C.c_int32), ("n_nodes_dev", vp), ("n_paths_dev", vp), ("done_dev", vp),
+        ("slots_dev", vp), ("n_slots", C.c_int32), ("counts_dev", vp), ("repetition_dev", vp), ("presence_dev", vp),
+        ("frequency_dev", vp),
+    ]
+
+
 class AssembleArgs(C.Structure):
     _fields_ = [
         ("batch", C.c_int32), ("n_nodes", C.c_int32), ("n_paths", C.c_int32), ("depth", C.c_int32), ("type_dev", vp),
@@ -161,6 +171,7 @@ SYMBOLS = {
     "samd_verify_sample": (C.c_int, [C.POINTER(SampleArgs), vp]),
     "samd_verify_sample_requests": (C.c_int, [C.POINTER(SampleArgs), C.POINTER(SampleRequestArgs), vp]),
     "samd_token_logprobs": (C.c_int, [C.POINTER(LogprobArgs), vp]),
+    "samd_apply_penalties": (C.c_int, [C.POINTER(PenaltyArgs), vp]),
     "samd_recycle_gen_tree": (C.c_int, [vp, C.c_int32, vp, vp, C.c_int32, vp, vp, C.c_int32, C.c_int32, vp, vp]),
     "samd_verify_set_chunk": (None, [C.c_int]),
     "samd_verify_set_overlap": (None, [C.c_int]),

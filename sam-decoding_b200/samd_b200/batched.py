@@ -35,14 +35,21 @@ samd_verify_sample_requests with every slot's own processor and Philox stream, a
 from the plain softmax of its prompt's last row.  A request's tokens depend only on its prompt, its parameters and its
 seed - not on its slot, its neighbours, the batch size, graph or eager execution, check_every, or a prefix pool.
 
-generate(..., logprobs=n) and serve(..., logprobs=n) also return every emitted token's raw log-probability and its n best
-alternatives (n in [0, 8]).  After the verify launch, one samd_token_logprobs launch scores the accepted rows of the step's
-logits; each slot carries the log-probability of its start token (predicted by the previous step's last accepted row,
+generate(..., logprobs=n) and serve(..., logprobs=n) also return every emitted token's log-probability (raw, or of the
+penalized row with penalties=) and its n best alternatives (n in [0, 8]).  After the verify launch, one
+samd_token_logprobs launch scores the accepted rows of the step's logits; each slot carries the log-probability of its start token (predicted by the previous step's last accepted row,
 or at admission by the prompt's last row), and the commit writes them beside the tokens with the same truncation.
+
+generate(..., penalties=...) and serve(..., penalties=...) apply repetition, presence and frequency penalties (Penalties,
+one per request) before verification or sampling.  Each draft row is penalized from its own context - prompt, emitted
+tokens and the draft tokens on its path - by one samd_apply_penalties launch between the LM forward and the verify
+launch, so greedy verification stays lossless against plain penalized greedy decoding.  Every slot keeps a device count
+table row (output counts, a bit for the prompt's tokens), filled at admission and by the commit.
 """
 from __future__ import annotations
 
 import dataclasses
+import math
 from typing import Iterable, Iterator, List, Optional, Sequence, Union
 
 import torch
@@ -79,6 +86,32 @@ class SamplingParams:
             return f"top_k must be an int >= 0, got {self.top_k!r}"
         if not isinstance(self.seed, int) or not 0 <= self.seed < 2 ** 63:
             return f"seed must be an int in [0, 2**63), got {self.seed!r}"
+        return None
+
+
+@dataclasses.dataclass(frozen=True)
+class Penalties:
+    """Penalties on repeated tokens for one request, applied to the logits before temperature, top-p and top-k (the
+    order of HF and vLLM).  repetition_penalty r > 0 (HF's RepetitionPenaltyLogitsProcessor: every token of the prompt
+    or the output so far is divided by r, or multiplied by r when negative); presence_penalty p and frequency_penalty f
+    in [-2, 2] (the OpenAI API: p is subtracted once from a token that occurs in the output, f once per occurrence; the
+    prompt is not counted).  The defaults change nothing.  The decoders check the values of every request when it is
+    pulled and name its index in the error."""
+    repetition_penalty: float = 1.0
+    presence_penalty: float = 0.0
+    frequency_penalty: float = 0.0
+
+    def problem(self) -> Optional[str]:
+        """What is wrong with these values (None: nothing)."""
+        for name in ("repetition_penalty", "presence_penalty", "frequency_penalty"):
+            v = getattr(self, name)
+            if isinstance(v, bool) or not isinstance(v, (int, float)) or not math.isfinite(v):
+                return f"{name} must be a finite float, got {v!r}"
+        if not self.repetition_penalty > 0:
+            return f"repetition_penalty must be > 0, got {self.repetition_penalty!r}"
+        for name in ("presence_penalty", "frequency_penalty"):
+            if not -2.0 <= getattr(self, name) <= 2.0:
+                return f"{name} must be in [-2, 2], got {getattr(self, name)!r}"
         return None
 
 
@@ -293,10 +326,11 @@ class BatchedSamdDecoder:
         if not self.ver_bound:
             self.ver.bind_kv([self.cache.kv[i] for i in range(self.cache.kv.shape[0])])
             self.ver_bound = True
-        n_nodes = self._n_nodes[kind].contiguous()
-        return self.ver.verify(logits, draft, self._ret[kind].contiguous(), cache_len=self.cache.cache_len,
-                               move_kv=True, n_nodes=n_nodes, n_paths=self._n_paths[kind].contiguous(),
-                               out=res, recycle=self.table), logits, n_nodes
+        n_nodes, ret = self._n_nodes[kind].contiguous(), self._ret[kind].contiguous()
+        n_paths = self._n_paths[kind].contiguous()
+        self._penalize(logits, draft, ret, n_nodes, n_paths)
+        return self.ver.verify(logits, draft, ret, cache_len=self.cache.cache_len, move_kv=True, n_nodes=n_nodes,
+                               n_paths=n_paths, out=res, recycle=self.table), logits, n_nodes
 
     def _draft_forward_verify(self, kv_len: int) -> tuple:
         """Drafts in, LM forward, fused verify: the part of a step that depends on the draft flavour.  Returns the verify
@@ -311,9 +345,19 @@ class BatchedSamdDecoder:
         pos = cache.cache_len.long()[:, None] + self._ar[None, :]
         logits = self.lm(input_ids=draft.long(), position_ids=pos, past_key_values=cache,
                          attention_mask=self._mask(T, kv_len, cache.cache_len)).logits.contiguous()
+        self._penalize(logits, draft)
         if self._sampled:                                      # identity path: no row moves, the commit sets cache_len
             return self._verify_sample(logits, draft, None), logits, None
         return self.ver.verify(logits, draft, None, cache_len=cache.cache_len, out=st["res"]), logits, None
+
+    def _penalize(self, logits: torch.Tensor, tokens: torch.Tensor, retrieve: Optional[torch.Tensor] = None,
+                  n_nodes: Optional[torch.Tensor] = None, n_paths: Optional[torch.Tensor] = None):
+        """Between the LM forward and the verify launch of a penalized call: every live draft row penalized in place from
+        its own path (identity chain without `retrieve`), one samd_apply_penalties launch.  Nothing otherwise."""
+        if self._penalized:
+            st = self._st
+            E.apply_penalties(logits, st["pen_counts"], st["pen_r"], st["pen_p"], st["pen_f"], tokens=tokens,
+                              retrieve=retrieve, n_nodes=n_nodes, n_paths=n_paths, done=st["done"])
 
     def _verify_sample(self, logits: torch.Tensor, tokens: torch.Tensor, retrieve: Optional[torch.Tensor], **kw) -> dict:
         """samd_verify_sample_requests with every slot's processor, greedy flag and Philox stream; finished slots make no
@@ -359,7 +403,10 @@ class BatchedSamdDecoder:
         cols = st["out_len"].long()[:, None] + ar[None, :]
         keep = ar[None, :] < n_emit[:, None]
         cols = torch.where(keep, cols, torch.full_like(cols, out.shape[1] - 1))
-        out.scatter_(1, cols, torch.where(keep, res["tokens"], torch.zeros_like(res["tokens"])))
+        emitted = torch.where(keep, res["tokens"], torch.zeros_like(res["tokens"]))
+        out.scatter_(1, cols, emitted)
+        if self._penalized:                                                        # the emitted tokens join the slot's counts
+            st["pen_counts"].scatter_add_(1, emitted.long(), keep.int())
         if lp is not None:
             self._commit_logprobs(lp, cols, keep)
         st["out_len"].add_(n_emit)
@@ -411,11 +458,11 @@ class BatchedSamdDecoder:
         return {}
 
     # ---- the step state, and the CUDA graphs that refer to it -------------------------------------------------------
-    def _init_state(self, max_limit: int, logprobs: bool = False):
+    def _init_state(self, max_limit: int, logprobs: bool = False, penalized: bool = False):
         """Zeroed step state for requests of at most `max_limit` new tokens.  The tensors persist across calls (the
         captured graphs refer to them, and limits are per slot); they are reallocated, and the graphs dropped, only when
         a call needs longer outputs than any before.  The log-probability state is added by the first call that asks
-        for log-probabilities."""
+        for log-probabilities, the penalty state by the first call with penalties."""
         B, T, dev = self.B, self.T, self.device
         width = T if self.tree is None else self._ret.shape[2]
         cap = getattr(self, "_st_cap", None)
@@ -442,14 +489,20 @@ class BatchedSamdDecoder:
             i32 = lambda *sh: torch.zeros(*sh, dtype=torch.int32, device=dev)
             self._st.update(lp=f32(B, W), lp_top=f32(B, W, 8), lp_ids=i32(B, W, 8), start_lp=f32(B), start_top=f32(B, 8),
                             start_ids=i32(B, 8))
+        if penalized and "pen_counts" not in self._st:
+            # pen_counts: every slot's output count per token, E.PENALTY_PROMPT_BIT set for its prompt's tokens;
+            # pen_r / pen_p / pen_f: its repetition, presence and frequency penalties
+            V = self.lm.config.vocab_size
+            self._st.update(pen_counts=torch.zeros(B, V, dtype=torch.int32, device=dev), pen_r=torch.ones(B, device=dev),
+                            pen_p=torch.zeros(B, device=dev), pen_f=torch.zeros(B, device=dev))
 
     def _advance(self, kv_len: int, graph: bool) -> bool:
         """One decode step at key length `kv_len`: the bucket's CUDA graph, captured first if it is new, or the same body
-        eagerly (one graph per bucket, greedy / sampled body and logprobs setting).  Returns `graph`, False from then on
-        when the LM's forward cannot be captured."""
+        eagerly (one graph per bucket, greedy / sampled body, logprobs setting and penalized or not).  Returns `graph`,
+        False from then on when the LM's forward cannot be captured."""
         if graph:
             B, dev, graphs = self.B, self.device, self._graphs
-            key = (kv_len, self._sampled, self._logprobs)
+            key = (kv_len, self._sampled, self._logprobs, self._penalized)
             if key not in graphs:
                 # warm-up run on a side stream (allocations, lazy initialisation), state restored, then the capture
                 snap = {k: (v.clone() if torch.is_tensor(v) else v) for k, v in self._st.items() if k != "res"}
@@ -564,7 +617,8 @@ class BatchedSamdDecoder:
 
     # ---- admission: new requests into free slots, between two steps ---------------------------------------------------
     def _admit(self, reqs: List[tuple]) -> int:
-        """Start the requests `reqs` = [(slot, prompt, limit, SamplingParams or None)] in their (free) slots; returns the
+        """Start the requests `reqs` = [(slot, prompt, limit, SamplingParams or None, Penalties or None)] in their (free)
+        slots; returns the
         longest prompt.  Only the persistent state is written, in place, so the captured graphs stay valid."""
         dev = self.device
         n_max = max(len(r[1]) for r in reqs)
@@ -583,8 +637,7 @@ class BatchedSamdDecoder:
         slots, lens, limits = meta[0], meta[1].to(torch.int32), meta[2].to(torch.int32)
         logits = self._prefill_slots(ids, slots)
         self._ingest(ids, slots, lens, logits)
-        self._set_slots(slots, lens, limits, logits[torch.arange(slots.numel(), device=dev), lens.long() - 1],
-                        [r[3] for r in reqs])
+        self._set_slots(slots, lens, limits, logits[torch.arange(slots.numel(), device=dev), lens.long() - 1], reqs)
         return n_max
 
     def _admit_prefixed(self, reqs: List[tuple], hits: List[tuple]):
@@ -625,7 +678,7 @@ class BatchedSamdDecoder:
             last = logits[torch.arange(len(fw), device=dev), suf_lens[f].long() - 1]
             for k, i in enumerate(fw):
                 rows[i] = last[k]
-        self._set_slots(slots, lens, limits, torch.stack(rows), [r[3] for r in reqs])
+        self._set_slots(slots, lens, limits, torch.stack(rows), reqs)
 
     def _copy_prefix_kv(self, slots: torch.Tensor, pids: torch.Tensor, plens: torch.Tensor):
         """KV rows [0, plens[i]) of pool row pids[i] into slot slots[i]: one samd_kv_copy_rows launch."""
@@ -703,12 +756,15 @@ class BatchedSamdDecoder:
         self._prefill_hook(ids, lens, logits)
 
     def _set_slots(self, slots: torch.Tensor, lens: torch.Tensor, limits: torch.Tensor, rows: torch.Tensor,
-                   params: List[Optional[SamplingParams]]):
+                   reqs: List[tuple]):
         """The admitted slots' step state: cache length, sampling parameters and a fresh Philox stream (sampled calls),
-        first start token from `rows` [n, V] (the logits after each prompt: argmax, or a draw from the plain softmax)
-        and, with logprobs, its log-probability, limit, and zero emitted tokens / history."""
-        st = self._st
+        penalty state (penalized calls), first start token from `rows` [n, V] (the logits after each prompt, penalized
+        from the prompt alone in a penalized call: argmax, or a draw from the plain softmax) and, with logprobs, its
+        log-probability, limit, and zero emitted tokens / history."""
+        st, params = self._st, [r[3] for r in reqs]
         self.cache.cache_len.index_copy_(0, slots, lens)
+        if self._penalized:
+            rows = self._admit_penalties(slots, rows, reqs)
         if self._sampled:
             dev = self.device
             f = torch.tensor([[sp.temperature, sp.top_p] for sp in params], dtype=torch.float32).T.contiguous().to(dev)
@@ -744,12 +800,33 @@ class BatchedSamdDecoder:
             st[k].index_fill_(0, slots, 0)
         st["done"].index_fill_(0, slots, False)
 
+    def _admit_penalties(self, slots: torch.Tensor, rows: torch.Tensor, reqs: List[tuple]) -> torch.Tensor:
+        """The admitted slots' penalty state - output counts zeroed, the whole prompt's tokens marked seen, r / p / f
+        written - and a penalized copy of `rows` (the prefix pool's stored rows stay as they are)."""
+        st, dev, V = self._st, self.device, rows.shape[-1]
+        n, n_max = len(reqs), max(len(r[1]) for r in reqs)
+        ids = torch.zeros(n, n_max, dtype=torch.long)
+        for i, r in enumerate(reqs):
+            ids[i, :len(r[1])] = torch.as_tensor(r[1], dtype=torch.long)
+            ids[i, len(r[1]):] = r[1][0]                       # pads repeat a prompt token: token 0 is not marked
+        vals = torch.tensor([[r[4].repetition_penalty, r[4].presence_penalty, r[4].frequency_penalty] for r in reqs],
+                            dtype=torch.float32).T.contiguous()
+        ids, vals = ids.to(dev), vals.to(dev)
+        st["pen_counts"].index_copy_(0, slots, torch.zeros(n, V, dtype=torch.int32, device=dev).scatter_(
+            1, ids, E.PENALTY_PROMPT_BIT))
+        for k, name in enumerate(("pen_r", "pen_p", "pen_f")):
+            st[name].index_copy_(0, slots, vals[k])
+        rows = rows.clone()
+        E.apply_penalties(rows.view(n, 1, V), st["pen_counts"], st["pen_r"], st["pen_p"], st["pen_f"],
+                          slots=slots.to(torch.int32))
+        return rows
+
     # ---- the decode loop of generate() and serve() --------------------------------------------------------------------
     def _run(self, requests: Iterator[tuple], max_limit: int, graph: bool, check_every: int, sampled: bool = False,
-             logprobs: Optional[int] = None):
-        """Decode the validated requests (index, prompt, limit, SamplingParams or None) of `requests`, at most B at a
-        time, with the greedy step body or (sampled) the sampled one; with `logprobs` (0 .. 8) the step also scores the
-        accepted rows.  The decode step has no host synchronisation in it: it is captured once per key-length bucket (64
+             logprobs: Optional[int] = None, penalized: bool = False):
+        """Decode the validated requests (index, prompt, limit, SamplingParams or None, Penalties or None) of
+        `requests`, at most B at a time, with the greedy step body or (sampled) the sampled one; with `logprobs` (0 .. 8)
+        the step also scores the accepted rows, and `penalized` penalizes the draft rows before verification.  The decode step has no host synchronisation in it: it is captured once per key-length bucket (64
         positions) as a CUDA graph and replayed.  Once every `check_every` steps the host reads [done | out_len | longest cache] in one copy; it then
         yields (index, tokens, accept_lengths, slot, (logprobs, top_logprobs) or None) for every request found finished
         (their rows in one more copy, their log-probabilities in one more),
@@ -757,8 +834,8 @@ class BatchedSamdDecoder:
         finished request keeps its slot - riding along, emitting nothing - until that check.  Statistics go to
         self._run_stats."""
         B, T, dev = self.B, self.T, self.device
-        self._init_state(max_limit, logprobs is not None)
-        self._sampled, self._logprobs = sampled, logprobs
+        self._init_state(max_limit, logprobs is not None, penalized)
+        self._sampled, self._logprobs, self._penalized = sampled, logprobs, penalized
         st = self._st
         run = self._run_id = getattr(self, "_run_id", 0) + 1
         self.eng.reset()
@@ -780,7 +857,7 @@ class BatchedSamdDecoder:
                     if r is None:
                         break
                     owner[b] = r[0]
-                    reqs.append((b, r[1], r[2], r[3]))
+                    reqs.append((b, r[1], r[2], r[3], r[4]))
             admissions += len(reqs)
             return self._admit(reqs) if reqs else 0
 
@@ -823,13 +900,14 @@ class BatchedSamdDecoder:
 
     @torch.inference_mode()
     def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4,
-                 sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None, logprobs: Optional[int] = None):
+                 sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None, logprobs: Optional[int] = None,
+                 penalties: Union[None, Penalties, Sequence[Penalties]] = None):
         """Lossless batched speculative decoding of exactly B prompts in lockstep (request b in slot b), up to
         max_new_tokens each.  The host reads the finished flags once every `check_every` steps - 1 / check_every host
         syncs per step - so a finished batch may run up to check_every - 1 idle steps (every request done: nothing is
         emitted).  graph=False runs the same body eagerly.  Returns (tokens per request, stats); stats["accept_lengths"]
-        holds every request's accepted tokens per step, padded with 0 to the longest request's `steps`.  `sampling` and
-        `logprobs`: as in serve(); with logprobs, stats["logprobs"] (and, for logprobs > 0, stats["top_logprobs"]) hold
+        holds every request's accepted tokens per step, padded with 0 to the longest request's `steps`.  `sampling`,
+        `logprobs` and `penalties`: as in serve(); with logprobs, stats["logprobs"] (and, for logprobs > 0, stats["top_logprobs"]) hold
         every request's list."""
         logprobs = _check_logprobs(logprobs)
         B, T = self.B, self.T
@@ -843,8 +921,10 @@ class BatchedSamdDecoder:
             raise K.SamdError(f"prompt + max_new_tokens + one step = {n_max + max_new_tokens + T} exceeds the automaton "
                               f"capacity max_tokens={self.dyn.max_tokens}")
         reqs = self._with_sampling(((i, p, max_new_tokens) for i, p in enumerate(prompts)), sampling)
+        reqs = self._with_penalties(reqs, penalties)
         out, acc, lps = [None] * B, [None] * B, [None] * B
-        for i, tokens, hist, _, lp in self._run(reqs, max_new_tokens, graph, check_every, sampling is not None, logprobs):
+        for i, tokens, hist, _, lp in self._run(reqs, max_new_tokens, graph, check_every, sampling is not None, logprobs,
+                                                penalties is not None):
             out[i], acc[i], lps[i] = tokens, hist, lp
         n_live = max(len(a) for a in acc)
         s = self._run_stats
@@ -859,7 +939,7 @@ class BatchedSamdDecoder:
     @torch.inference_mode()
     def serve(self, prompts: Iterable[Sequence[int]], max_new_tokens: Union[int, Sequence[int]], graph: bool = True,
               check_every: int = 4, sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None,
-              logprobs: Optional[int] = None):
+              logprobs: Optional[int] = None, penalties: Union[None, Penalties, Sequence[Penalties]] = None):
         """Continuous batching: decode any number of requests through the B slots, refilling a slot with the next queued
         request as soon as the host sees its request finished (once every `check_every` steps).  `prompts` is consumed
         lazily and in order; `max_new_tokens` is one limit for all or a sequence with one per request.  Yields
@@ -880,12 +960,20 @@ class BatchedSamdDecoder:
         depend only on its prompt, parameters and seed; a request with greedy=True decodes greedily.  Not with
         Token-Recycle tree mode (tree=): SamdError.
 
-        `logprobs` (None: none): an int n in [0, 8].  info["logprobs"] then holds the model's raw log-probability of every
+        `logprobs` (None: none): an int n in [0, 8].  info["logprobs"] then holds the model's log-probability of every
         token in `tokens`, log_softmax(logits)[token] of the row that predicted it - no temperature, top-p or top-k, in
-        greedy and sampled decoding alike - and, for n > 0, info["top_logprobs"] the n most likely tokens at each of
-        those positions as (token_id, logprob) pairs (value descending, lowest id first among equals).  They are scored
-        on the device from the logits the decode step already computed (one samd_token_logprobs launch per step and per
-        admission); the tokens are the same as without."""
+        greedy and sampled decoding alike; with `penalties`, of the penalized row the token was chosen from, so under
+        greedy decoding top_logprobs[0] is the emitted token - and, for n > 0, info["top_logprobs"] the n most likely
+        tokens at each of those positions as (token_id, logprob) pairs (value descending, lowest id first among equals).
+        They are scored on the device from the logits the decode step already computed (one samd_token_logprobs launch
+        per step and per admission); the tokens are the same as without.
+
+        `penalties` (None: none): one Penalties for every request or a sequence with one per request - repetition,
+        presence and frequency penalties applied to every logits row before verification (and before temperature,
+        top-p and top-k when sampled).  A row is penalized from its own context: the prompt, the tokens emitted so far
+        and the draft tokens on its path, so greedy decoding stays lossless against plain penalized greedy decoding.
+        Tree mode (tree=) is allowed; its successor table then learns from penalized rows, which changes drafts, not
+        tokens.  Neutral Penalties() give the tokens of penalties=None."""
         logprobs = _check_logprobs(logprobs)
         self.serve_stats = None
         if hasattr(max_new_tokens, "__len__"):
@@ -894,8 +982,9 @@ class BatchedSamdDecoder:
         else:
             limits, max_limit = None, int(max_new_tokens)
         reqs = self._with_sampling(self._requests(prompts, max_new_tokens if limits is None else limits), sampling)
+        reqs = self._with_penalties(reqs, penalties)
         for i, tokens, hist, slot, lp in self._run(reqs, max(max_limit, 1), graph, check_every, sampling is not None,
-                                                   logprobs):
+                                                   logprobs, penalties is not None):
             info = {"slot": slot, "accept_lengths": hist}
             if self._prefixes is not None:
                 info["prefix_len"] = self._slot_plen[slot]
@@ -956,6 +1045,34 @@ class BatchedSamdDecoder:
             if bad:
                 raise K.SamdError(f"request {i}: {bad}")
             yield i, p, limit, sp
+
+    @staticmethod
+    def _with_penalties(requests: Iterator[tuple], penalties) -> Iterator[tuple]:
+        """(index, prompt, limit, SamplingParams or None, Penalties or None) of every request: the shared Penalties or
+        its own, checked as it is pulled."""
+        shared = penalties is None or isinstance(penalties, Penalties)
+        if not shared:
+            try:
+                penalties = list(penalties)
+            except TypeError:
+                raise K.SamdError(f"penalties must be None, a Penalties or a sequence of them, got "
+                                  f"{type(penalties).__name__}") from None
+        for i, p, limit, sp in requests:
+            if penalties is None:
+                yield i, p, limit, sp, None
+                continue
+            if shared:
+                pn = penalties
+            elif i >= len(penalties):
+                raise K.SamdError(f"request {i}: penalties has {len(penalties)} values, fewer than the prompts")
+            else:
+                pn = penalties[i]
+            if not isinstance(pn, Penalties):
+                raise K.SamdError(f"request {i}: penalties must be a Penalties, got {type(pn).__name__}")
+            bad = pn.problem()
+            if bad:
+                raise K.SamdError(f"request {i}: {bad}")
+            yield i, p, limit, sp, pn
 
 
 class BatchedSamOnlyDecoder(BatchedSamdDecoder):
@@ -1033,6 +1150,7 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
         cache.begin(T, kv_len)
         logits = self.lm(input_ids=buf["tokens"].long(), position_ids=buf["position_ids"], past_key_values=cache,
                          attention_mask=mask[:, None]).logits.contiguous()
+        self._penalize(logits, buf["tokens"], buf["retrieve"], buf["n_nodes"], buf["n_paths"])
         if self._sampled:
             # a request's own width - its draft length, or its tree's deepest path - so that the -1 pads beyond it are
             # never compared; then the accepted rows move into place

@@ -520,6 +520,74 @@ def kv_copy_rows(dst: tuple, src: tuple, dst_row: torch.Tensor, src_row: torch.T
                 "samd_kv_copy_rows")
 
 
+PENALTY_PROMPT_BIT = -2 ** 31           # bit 31 of a count-table entry: the token occurs in the prompt
+
+
+def apply_penalties(logits: torch.Tensor, counts: torch.Tensor, repetition: torch.Tensor, presence: torch.Tensor,
+                    frequency: torch.Tensor, tokens: Optional[torch.Tensor] = None, retrieve: Optional[torch.Tensor] = None,
+                    n_nodes: Optional[torch.Tensor] = None, n_paths: Optional[torch.Tensor] = None,
+                    done: Optional[torch.Tensor] = None, slots: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """samd_apply_penalties: repetition / presence / frequency penalties on the draft rows `logits` [B, T, V] (fp32,
+    bf16 or fp16, unit stride over V), in place, one launch; returns `logits`.  Row j of request b is penalized from
+    its own context: the prompt, the emitted tokens and the node tokens `tokens` [B, T] on the path from node 0 to
+    node j - the identity chain without `retrieve`, else the path of `retrieve` [B, P, D] (-1 padded, the table a
+    verify call walks) that lists node j.  tokens=None: no row has draft context (the prompt's last row at
+    admission).  Per state row s = slots[b] (int32 [B]; None: s = b): `counts` [S, V] int32, the output count of
+    every token with PENALTY_PROMPT_BIT set for the prompt's tokens, and `repetition` / `presence` / `frequency`
+    [S] float32.  With c = output count + occurrences on the path, a token that is in the prompt or has c > 0
+    becomes (x < 0 ? x * r : x / r) - f * c - p * (c > 0), each operation rounded in fp32.  `n_nodes` / `n_paths`
+    [B] int32: live rows and paths per request (rows past n_nodes are not touched); `done` [B] bool/uint8:
+    finished requests are not touched, nor are neutral ones (r = 1, p = f = 0).  Every argument is checked before
+    anything reaches the device."""
+    if logits.dim() != 3 or logits.stride(2) != 1:
+        raise K.SamdError(f"apply_penalties: logits must be [B, T, V] with unit stride over V, got {tuple(logits.shape)}")
+    B, T, V = logits.shape
+    dt = {torch.bfloat16: K.DTYPE_BF16, torch.float16: K.DTYPE_FP16, torch.float32: K.DTYPE_FP32}.get(logits.dtype)
+    if dt is None:
+        raise K.SamdError(f"apply_penalties: unsupported logits dtype {logits.dtype} (bf16 / fp16 / fp32)")
+    if not 1 <= T <= 256:
+        raise K.SamdError(f"apply_penalties: at most 256 rows per request, got {T}")
+    if counts.dim() != 2 or counts.shape[1] != V:
+        raise K.SamdError(f"apply_penalties: counts must be [S, {V}], got {tuple(counts.shape)}")
+    S = counts.shape[0]
+    if slots is None and S != B:
+        raise K.SamdError(f"apply_penalties: without slots counts needs one row per request ({B}), got {S}")
+    if retrieve is not None and tokens is None:
+        raise K.SamdError("apply_penalties: a path table needs the node tokens")
+    if retrieve is not None and (retrieve.dim() != 3 or retrieve.shape[0] != B or 0 in retrieve.shape):
+        raise K.SamdError(f"apply_penalties: retrieve must be [{B}, P, D], got {tuple(retrieve.shape)}")
+    if n_paths is not None and retrieve is None:
+        raise K.SamdError("apply_penalties: n_paths needs a path table")
+    for name, t, shape, dtypes in (("counts", counts, (S, V), (torch.int32,)),
+                                   ("repetition", repetition, (S,), (torch.float32,)),
+                                   ("presence", presence, (S,), (torch.float32,)),
+                                   ("frequency", frequency, (S,), (torch.float32,)),
+                                   ("tokens", tokens, (B, T), (torch.int32,)),
+                                   ("retrieve", retrieve, None if retrieve is None else tuple(retrieve.shape), (torch.int32,)),
+                                   ("n_nodes", n_nodes, (B,), (torch.int32,)), ("n_paths", n_paths, (B,), (torch.int32,)),
+                                   ("done", done, (B,), (torch.bool, torch.uint8)), ("slots", slots, (B,), (torch.int32,))):
+        if t is None:
+            continue
+        if tuple(t.shape) != shape or t.dtype not in dtypes or not t.is_contiguous():
+            raise K.SamdError(f"apply_penalties: {name} must be a contiguous {shape} {dtypes[0]} tensor, got "
+                              f"{tuple(t.shape)} {t.dtype}")
+    tensors = [logits, counts, repetition, presence, frequency] + [x for x in (tokens, retrieve, n_nodes, n_paths, done, slots)
+                                                                    if x is not None]
+    if not all(t.is_cuda and t.device == logits.device for t in tensors):
+        raise K.SamdError("apply_penalties: every tensor must be on the logits' GPU")
+    a = K.PenaltyArgs()
+    a.logits_dev, a.dtype, a.batch, a.n_nodes, a.vocab = logits.data_ptr(), dt, B, T, V
+    a.batch_stride, a.row_stride = logits.stride(0), logits.stride(1)
+    a.tokens_dev, a.retrieve_dev = K.ptr(tokens), K.ptr(retrieve)
+    a.n_paths, a.depth = (retrieve.shape[1], retrieve.shape[2]) if retrieve is not None else (1, T)
+    a.n_nodes_dev, a.n_paths_dev, a.done_dev, a.slots_dev = K.ptr(n_nodes), K.ptr(n_paths), K.ptr(done), K.ptr(slots)
+    a.n_slots, a.counts_dev = S, counts.data_ptr()
+    a.repetition_dev, a.presence_dev, a.frequency_dev = repetition.data_ptr(), presence.data_ptr(), frequency.data_ptr()
+    with torch.cuda.device(logits.device):
+        K.check(K.lib().samd_apply_penalties(C.byref(a), K.stream_ptr()), "samd_apply_penalties")
+    return logits
+
+
 class Verifier:
     """Fused greedy verification + KV compaction (samd/utils.py:127-141, samd/samd_model.py:159-211,
     samd/cache.py:118-133) for a batch of requests: one persistent launch."""
@@ -700,8 +768,9 @@ class Verifier:
                        tokens: Optional[torch.Tensor], next_token: torch.Tensor, n_top: int = 0,
                        n_nodes: Optional[torch.Tensor] = None, done: Optional[torch.Tensor] = None,
                        out: Optional[dict] = None) -> dict:
-        """samd_token_logprobs: the raw log-probability log_softmax(float32(row))[target] of every accepted token, one
-        launch.  `indices` / `count` / `tokens` / `next_token`: a verify call's "indices" [B, W] (None: the identity
+        """samd_token_logprobs: the log-probability log_softmax(float32(row))[target] of every accepted token, one
+        launch, from the rows as they are - raw, or after apply_penalties rewrote them (the rows the tokens were chosen
+        from; no temperature, top-p or top-k either way).  `indices` / `count` / `tokens` / `next_token`: a verify call's "indices" [B, W] (None: the identity
         path), "accept_len", "tokens" [B, W] (None when every count is <= 1) and "next_token".  Position j < count[b] is
         scored on row indices[b][j] (-1: row n_nodes[b] - 1) against tokens[b][j + 1], the last one against
         next_token[b].  Returns out["logprob"] [B, W] (positions j < count - 1) and out["next_logprob"] [B] (the last
