@@ -491,6 +491,31 @@ typedef struct samd_penalty_args {
 } samd_penalty_args;
 int samd_apply_penalties(const samd_penalty_args *args, void *stream);
 
+/* Stop sequences: where does this step's output end?  Request b has emitted hist_dev[b][0 .. hist_len_dev[b]) so far
+ * and this step would emit tokens_dev[b][0 .. count_dev[b]).  Sequence j (stop_len_dev[b][j] = L in [1, 16] ids
+ * stop_tokens_dev[b][j][0 .. L); L = 0 marks an unused entry) ends at step position i < count when the output tokens
+ * at output positions hist_len + i - L + 1 .. hist_len + i equal it; positions before 0 (the prompt) never match, and
+ * only the last SAMD_STOP_MAX_LEN - 1 history tokens are read.  out_count_dev[b] = e + 1 for the earliest such i = e,
+ * out_hit_dev[b] = the lowest j ending there; without a match, or for a done request or count 0: count and -1.  Tokens
+ * at or past count are never read.  out_count_dev may alias count_dev.  The result depends only on the inputs; no
+ * argument depends on the step, so the launch can be captured in a CUDA graph. */
+#define SAMD_STOP_MAX_SEQS 16
+#define SAMD_STOP_MAX_LEN  16
+typedef struct samd_stop_args {
+    int32_t        batch, width;      /* width <= 256 */
+    const int32_t *tokens_dev;        /* [B][width] this step's accepted tokens */
+    const int32_t *count_dev;         /* [B] candidate tokens (<= width) */
+    const int32_t *hist_dev;          /* [B][hist_stride] output emitted so far */
+    int32_t        hist_stride;
+    const int32_t *hist_len_dev;      /* [B] */
+    const int32_t *stop_tokens_dev;   /* [B][SAMD_STOP_MAX_SEQS][SAMD_STOP_MAX_LEN] */
+    const int32_t *stop_len_dev;      /* [B][SAMD_STOP_MAX_SEQS], 0 = unused */
+    const uint8_t *done_dev;          /* [B] 1 = finished, or NULL */
+    int32_t       *out_count_dev;     /* [B] */
+    int32_t       *out_hit_dev;       /* [B] sequence index or -1 */
+} samd_stop_args;
+int samd_stop_match(const samd_stop_args *args, void *stream);
+
 /* TokenRecycle.gen_draft (token_recycle.py:49-59) for a batch: tokens[b][0] = start_tok[b]; every other node takes
  * table[token of its parent][its rank among the parent's children], or 0 when the parent's token has no entry.
  * parent / rank: [n_nodes] device arrays describing the static tree (node 0 = root, parents before children);

@@ -21,6 +21,8 @@ DRAFT_STATIC_TREE = 3
 DTYPE_BF16 = 0
 DTYPE_FP16 = 1
 DTYPE_FP32 = 2
+STOP_MAX_SEQS = 16
+STOP_MAX_LEN = 16
 
 c_i32p = C.POINTER(C.c_int32)
 c_i64p = C.POINTER(C.c_int64)
@@ -86,6 +88,14 @@ class PenaltyArgs(C.Structure):
         ("n_paths", C.c_int32), ("depth", C.c_int32), ("n_nodes_dev", vp), ("n_paths_dev", vp), ("done_dev", vp),
         ("slots_dev", vp), ("n_slots", C.c_int32), ("counts_dev", vp), ("repetition_dev", vp), ("presence_dev", vp),
         ("frequency_dev", vp),
+    ]
+
+
+class StopArgs(C.Structure):
+    _fields_ = [
+        ("batch", C.c_int32), ("width", C.c_int32), ("tokens_dev", vp), ("count_dev", vp), ("hist_dev", vp),
+        ("hist_stride", C.c_int32), ("hist_len_dev", vp), ("stop_tokens_dev", vp), ("stop_len_dev", vp), ("done_dev", vp),
+        ("out_count_dev", vp), ("out_hit_dev", vp),
     ]
 
 
@@ -172,6 +182,7 @@ SYMBOLS = {
     "samd_verify_sample_requests": (C.c_int, [C.POINTER(SampleArgs), C.POINTER(SampleRequestArgs), vp]),
     "samd_token_logprobs": (C.c_int, [C.POINTER(LogprobArgs), vp]),
     "samd_apply_penalties": (C.c_int, [C.POINTER(PenaltyArgs), vp]),
+    "samd_stop_match": (C.c_int, [C.POINTER(StopArgs), vp]),
     "samd_recycle_gen_tree": (C.c_int, [vp, C.c_int32, vp, vp, C.c_int32, vp, vp, C.c_int32, C.c_int32, vp, vp]),
     "samd_verify_set_chunk": (None, [C.c_int]),
     "samd_verify_set_overlap": (None, [C.c_int]),

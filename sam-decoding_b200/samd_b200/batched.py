@@ -45,11 +45,19 @@ one per request) before verification or sampling.  Each draft row is penalized f
 tokens and the draft tokens on its path - by one samd_apply_penalties launch between the LM forward and the verify
 launch, so greedy verification stays lossless against plain penalized greedy decoding.  Every slot keeps a device count
 table row (output counts, a bit for the prompt's tokens), filled at admission and by the commit.
+
+generate(..., stop=...) and serve(..., stop=...) end a request at the earliest of its stop sequences (StopSequences: up
+to 16 sequences of up to 16 token ids, matched against the output only).  One step accepts up to T tokens, so a sequence
+may end inside a step or straddle two: after the EOS cut, one samd_stop_match launch in the commit finds each request's
+earliest match among the tokens the step would emit (and the last 15 it emitted before), and the commit emits up to it.
+Every request also gets a finish reason: "stop" (EOS or a stop sequence), "length" (max_new_tokens) or "cache" (the
+max_cache_len guard).
 """
 from __future__ import annotations
 
 import dataclasses
 import math
+import numbers
 from typing import Iterable, Iterator, List, Optional, Sequence, Union
 
 import torch
@@ -112,6 +120,33 @@ class Penalties:
         for name in ("presence_penalty", "frequency_penalty"):
             if not -2.0 <= getattr(self, name) <= 2.0:
                 return f"{name} must be in [-2, 2], got {getattr(self, name)!r}"
+        return None
+
+
+@dataclasses.dataclass(frozen=True)
+class StopSequences:
+    """Stop sequences of one request: at most 16 sequences of 1 to 16 token ids in [0, V) each (ids, not strings: a
+    string that tokenizes several ways is passed as one sequence per tokenization).  The request's output ends at the
+    earliest output position where one of them ends - matched against the output alone, never the prompt - and the
+    matched tokens stay in it, as EOS does; among sequences ending there the lowest index wins.  StopSequences(()) stops
+    nothing.  The decoders check the sequences of every request when it is pulled and name its index in the error."""
+    sequences: Sequence[Sequence[int]] = ()
+
+    def problem(self, vocab: int) -> Optional[str]:
+        """What is wrong with these sequences for a vocabulary of `vocab` tokens (None: nothing)."""
+        seqs = self.sequences
+        if not isinstance(seqs, (list, tuple)):
+            return f"sequences must be a list or tuple of token id sequences, got {type(seqs).__name__}"
+        if len(seqs) > K.STOP_MAX_SEQS:
+            return f"at most {K.STOP_MAX_SEQS} sequences, got {len(seqs)}"
+        for j, seq in enumerate(seqs):
+            if not isinstance(seq, (list, tuple)):
+                return f"sequence {j} must be a list or tuple of token ids, got {type(seq).__name__}"
+            if not 1 <= len(seq) <= K.STOP_MAX_LEN:
+                return f"sequence {j} must have 1 to {K.STOP_MAX_LEN} token ids, got {len(seq)}"
+            for t in seq:
+                if isinstance(t, bool) or not isinstance(t, numbers.Integral) or not 0 <= t < vocab:
+                    return f"sequence {j}: token ids must be ints in [0, {vocab}), got {t!r}"
         return None
 
 
@@ -384,7 +419,7 @@ class BatchedSamdDecoder:
         self._commit(res, saved_len, lp)
 
     def _commit(self, res: dict, saved_len: torch.Tensor, lp: Optional[dict] = None):
-        """EOS truncation, emission up to each slot's own limit, cache lengths, the next step's inputs, history and the
+        """EOS truncation, the stop-sequence cut (calls with stops), emission up to each slot's own limit, cache lengths, the next step's inputs, history and the
         host flag.  With `lp` (token_logprobs of this step) the emitted tokens' log-probabilities go to the columns of
         st["lp"] (and top-n lists to st["lp_ids"] / st["lp_top"]) parallel to st["out"]: emitted token 0 is the start
         token, predicted by the previous step's last row (st["start_lp"]), token k >= 1 is scored position k - 1."""
@@ -398,6 +433,14 @@ class BatchedSamdDecoder:
             done.logical_or_(is_eos.any(1))
             n_acc = torch.minimum(n_acc, first)
         room = (st["limit"] - st["out_len"]).clamp(min=0)
+        if self._stopped:                  # the earliest stop sequence among the tokens the step would emit: cut there
+            cand = torch.minimum(n_acc, room)
+            cut, hit = E.match_stops(res["tokens"], cand, st["out"], st["out_len"], st["stop_tok"], st["stop_len"],
+                                     out_count=cand, out_hit=st["stop_step"])
+            stopped = hit >= 0
+            n_acc = torch.where(stopped, cut, n_acc)
+            done.logical_or_(stopped)
+            torch.maximum(st["stop_hit"], hit, out=st["stop_hit"])            # (-1 from admission until a hit)
         n_emit = torch.minimum(n_acc, room)
         out = st["out"]
         cols = st["out_len"].long()[:, None] + ar[None, :]
@@ -458,11 +501,12 @@ class BatchedSamdDecoder:
         return {}
 
     # ---- the step state, and the CUDA graphs that refer to it -------------------------------------------------------
-    def _init_state(self, max_limit: int, logprobs: bool = False, penalized: bool = False):
+    def _init_state(self, max_limit: int, logprobs: bool = False, penalized: bool = False, stopped: bool = False):
         """Zeroed step state for requests of at most `max_limit` new tokens.  The tensors persist across calls (the
         captured graphs refer to them, and limits are per slot); they are reallocated, and the graphs dropped, only when
         a call needs longer outputs than any before.  The log-probability state is added by the first call that asks
-        for log-probabilities, the penalty state by the first call with penalties."""
+        for log-probabilities, the penalty state by the first call with penalties, the stop state by the first call with
+        stop sequences."""
         B, T, dev = self.B, self.T, self.device
         width = T if self.tree is None else self._ret.shape[2]
         cap = getattr(self, "_st_cap", None)
@@ -495,14 +539,20 @@ class BatchedSamdDecoder:
             V = self.lm.config.vocab_size
             self._st.update(pen_counts=torch.zeros(B, V, dtype=torch.int32, device=dev), pen_r=torch.ones(B, device=dev),
                             pen_p=torch.zeros(B, device=dev), pen_f=torch.zeros(B, device=dev))
+        if stopped and "stop_tok" not in self._st:
+            # stop_tok / stop_len: every slot's stop sequences (length 0: unused); stop_hit: the index of the one that
+            # ended it, -1 until then; stop_step: the step's match
+            S, L = K.STOP_MAX_SEQS, K.STOP_MAX_LEN
+            i32 = lambda *sh: torch.zeros(*sh, dtype=torch.int32, device=dev)
+            self._st.update(stop_tok=i32(B, S, L), stop_len=i32(B, S), stop_hit=i32(B), stop_step=i32(B))
 
     def _advance(self, kv_len: int, graph: bool) -> bool:
         """One decode step at key length `kv_len`: the bucket's CUDA graph, captured first if it is new, or the same body
-        eagerly (one graph per bucket, greedy / sampled body, logprobs setting and penalized or not).  Returns `graph`,
+        eagerly (one graph per bucket, greedy / sampled body, logprobs setting, penalized or not and stopped or not).  Returns `graph`,
         False from then on when the LM's forward cannot be captured."""
         if graph:
             B, dev, graphs = self.B, self.device, self._graphs
-            key = (kv_len, self._sampled, self._logprobs, self._penalized)
+            key = (kv_len, self._sampled, self._logprobs, self._penalized, self._stopped)
             if key not in graphs:
                 # warm-up run on a side stream (allocations, lazy initialisation), state restored, then the capture
                 snap = {k: (v.clone() if torch.is_tensor(v) else v) for k, v in self._st.items() if k != "res"}
@@ -617,9 +667,8 @@ class BatchedSamdDecoder:
 
     # ---- admission: new requests into free slots, between two steps ---------------------------------------------------
     def _admit(self, reqs: List[tuple]) -> int:
-        """Start the requests `reqs` = [(slot, prompt, limit, SamplingParams or None, Penalties or None)] in their (free)
-        slots; returns the
-        longest prompt.  Only the persistent state is written, in place, so the captured graphs stay valid."""
+        """Start the requests `reqs` = [(slot, prompt, limit, SamplingParams or None, Penalties or None, StopSequences or
+        None)] in their (free) slots; returns the longest prompt.  Only the persistent state is written, in place, so the captured graphs stay valid."""
         dev = self.device
         n_max = max(len(r[1]) for r in reqs)
         if self._prefixes is not None:
@@ -760,7 +809,7 @@ class BatchedSamdDecoder:
         """The admitted slots' step state: cache length, sampling parameters and a fresh Philox stream (sampled calls),
         penalty state (penalized calls), first start token from `rows` [n, V] (the logits after each prompt, penalized
         from the prompt alone in a penalized call: argmax, or a draw from the plain softmax) and, with logprobs, its
-        log-probability, limit, and zero emitted tokens / history."""
+        log-probability, stop sequences (calls with stops), limit, and zero emitted tokens / history."""
         st, params = self._st, [r[3] for r in reqs]
         self.cache.cache_len.index_copy_(0, slots, lens)
         if self._penalized:
@@ -795,6 +844,17 @@ class BatchedSamdDecoder:
                 st["start_ids"][slots, :n] = lp["next_top_ids"]
                 st["start_top"][slots, :n] = lp["next_top_logprob"]
         st["start"].index_copy_(0, slots, first)
+        if self._stopped:
+            n, S, L = len(reqs), K.STOP_MAX_SEQS, K.STOP_MAX_LEN
+            tab = [[0] * (S * L + S) for _ in reqs]                           # [stop_tok | stop_len] per request
+            for row, r in zip(tab, reqs):
+                for j, seq in enumerate(r[5].sequences):
+                    row[j * L:j * L + len(seq)] = [int(t) for t in seq]
+                    row[S * L + j] = len(seq)
+            tab = torch.tensor(tab, dtype=torch.int32).to(self.device)
+            st["stop_tok"].index_copy_(0, slots, tab[:, :S * L].reshape(n, S, L))
+            st["stop_len"].index_copy_(0, slots, tab[:, S * L:].contiguous())
+            st["stop_hit"].index_fill_(0, slots, -1)
         st["limit"].index_copy_(0, slots, limits)
         for k in ("acc_count", "out_len", "hlen"):
             st[k].index_fill_(0, slots, 0)
@@ -823,26 +883,30 @@ class BatchedSamdDecoder:
 
     # ---- the decode loop of generate() and serve() --------------------------------------------------------------------
     def _run(self, requests: Iterator[tuple], max_limit: int, graph: bool, check_every: int, sampled: bool = False,
-             logprobs: Optional[int] = None, penalized: bool = False):
-        """Decode the validated requests (index, prompt, limit, SamplingParams or None, Penalties or None) of
-        `requests`, at most B at a time, with the greedy step body or (sampled) the sampled one; with `logprobs` (0 .. 8)
-        the step also scores the accepted rows, and `penalized` penalizes the draft rows before verification.  The decode step has no host synchronisation in it: it is captured once per key-length bucket (64
+             logprobs: Optional[int] = None, penalized: bool = False, stopped: bool = False):
+        """Decode the validated requests (index, prompt, limit, SamplingParams or None, Penalties or None, StopSequences
+        or None) of `requests`, at most B at a time, with the greedy step body or (sampled) the sampled one; with
+        `logprobs` (0 .. 8) the step also scores the accepted rows, `penalized` penalizes the draft rows before
+        verification and `stopped` cuts each request's output at its first stop sequence.  The decode step has no host synchronisation in it: it is captured once per key-length bucket (64
         positions) as a CUDA graph and replayed.  Once every `check_every` steps the host reads [done | out_len | longest cache] in one copy; it then
-        yields (index, tokens, accept_lengths, slot, (logprobs, top_logprobs) or None) for every request found finished
-        (their rows in one more copy, their log-probabilities in one more),
+        yields (index, tokens, accept_lengths, slot, (logprobs, top_logprobs) or None, finish reason, stop index or None)
+        for every request found finished (their rows and stop indices in one more copy, their log-probabilities in one
+        more),
         admits queued requests into the free slots, and sizes the next steps' key length from the longest cache.  A
         finished request keeps its slot - riding along, emitting nothing - until that check.  Statistics go to
         self._run_stats."""
         B, T, dev = self.B, self.T, self.device
-        self._init_state(max_limit, logprobs is not None, penalized)
-        self._sampled, self._logprobs, self._penalized = sampled, logprobs, penalized
+        self._init_state(max_limit, logprobs is not None, penalized, stopped)
+        self._sampled, self._logprobs, self._penalized, self._stopped = sampled, logprobs, penalized, stopped
         st = self._st
         run = self._run_id = getattr(self, "_run_id", 0) + 1
         self.eng.reset()
         self.cache.cache_len.zero_()
         st["done"].fill_(True)                                                     # an empty slot rides along finished
         owner = [None] * B                                                         # request index in each slot
+        limit_of = [0] * B                                                         # and its max_new_tokens
         W, max_accept = st["out"].shape[1], st["acc_tokens"].shape[1]              # (the most one step adds to a cache)
+        H = st["hist"].shape[1]
         flag_host = torch.zeros(2 * B + 1, dtype=torch.int32).pin_memory()
         steps = syncs = since = admissions = live_steps = 0
         self.prefix_hits = self.prefix_tokens = 0
@@ -856,8 +920,8 @@ class BatchedSamdDecoder:
                     r = next(requests, None)
                     if r is None:
                         break
-                    owner[b] = r[0]
-                    reqs.append((b, r[1], r[2], r[3], r[4]))
+                    owner[b], limit_of[b] = r[0], r[2]
+                    reqs.append((b,) + tuple(r[1:]))
             admissions += len(reqs)
             return self._admit(reqs) if reqs else 0
 
@@ -878,7 +942,10 @@ class BatchedSamdDecoder:
             fin = [b for b in range(B) if owner[b] is not None and flag[b]]
             if fin:
                 idx = torch.tensor(fin, device=dev)
-                rows = torch.cat((st["out"][idx], st["hist"][idx], st["hlen"][idx, None]), 1).tolist()
+                cols = (st["out"][idx], st["hist"][idx], st["hlen"][idx, None])
+                if stopped:
+                    cols += (st["stop_hit"][idx, None],)
+                rows = torch.cat(cols, 1).tolist()
                 lps = [None] * len(fin)
                 if logprobs is not None:                   # [f, W, 1 + 2n]: log-probability | top-n values | top-n ids
                     n = logprobs
@@ -887,9 +954,10 @@ class BatchedSamdDecoder:
                     lps = [_logprob_lists(lpr[k, :flag[B + b]], n) for k, b in enumerate(fin)]
                 for b, r, lp in zip(fin, rows, lps):
                     i, owner[b] = owner[b], None
-                    hist = r[W:W + r[-1]]
+                    hist = r[W:W + r[W + H]]
                     live_steps += len(hist)
-                    yield i, r[:flag[B + b]], hist, b, lp
+                    tokens, hit = r[:flag[B + b]], r[W + H + 1] if stopped else -1
+                    yield i, tokens, hist, b, lp, self._finish_reason(tokens, hit, limit_of[b]), hit if hit >= 0 else None
                     if self._run_id != run:
                         raise K.SamdError("the decoder ran another generate() / serve() while this serve() was suspended")
             kv_hi = max(kv_hi, admit())
@@ -898,17 +966,26 @@ class BatchedSamdDecoder:
         if self._prefixes is not None:
             self._run_stats.update(prefix_hits=self.prefix_hits, prefix_tokens=self.prefix_tokens)
 
+    def _finish_reason(self, tokens: List[int], stop_hit: int, limit: int) -> str:
+        """Why a finished request ended: "stop" (a stop sequence, or EOS - truncation keeps it as the last token),
+        "length" (max_new_tokens) or "cache" (the max_cache_len guard, which finished it before either)."""
+        if stop_hit >= 0 or (self.eos is not None and tokens and tokens[-1] == self.eos):
+            return "stop"
+        return "length" if len(tokens) >= limit else "cache"
+
     @torch.inference_mode()
     def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4,
                  sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None, logprobs: Optional[int] = None,
-                 penalties: Union[None, Penalties, Sequence[Penalties]] = None):
+                 penalties: Union[None, Penalties, Sequence[Penalties]] = None,
+                 stop: Union[None, StopSequences, Sequence[StopSequences]] = None):
         """Lossless batched speculative decoding of exactly B prompts in lockstep (request b in slot b), up to
         max_new_tokens each.  The host reads the finished flags once every `check_every` steps - 1 / check_every host
         syncs per step - so a finished batch may run up to check_every - 1 idle steps (every request done: nothing is
         emitted).  graph=False runs the same body eagerly.  Returns (tokens per request, stats); stats["accept_lengths"]
         holds every request's accepted tokens per step, padded with 0 to the longest request's `steps`.  `sampling`,
-        `logprobs` and `penalties`: as in serve(); with logprobs, stats["logprobs"] (and, for logprobs > 0, stats["top_logprobs"]) hold
-        every request's list."""
+        `logprobs`, `penalties` and `stop`: as in serve(); with logprobs, stats["logprobs"] (and, for logprobs > 0,
+        stats["top_logprobs"]) hold every request's list.  stats["finish_reasons"] holds every request's finish reason
+        and, with stop, stats["stop_indices"] its stop index."""
         logprobs = _check_logprobs(logprobs)
         B, T = self.B, self.T
         assert len(prompts) == B
@@ -921,15 +998,18 @@ class BatchedSamdDecoder:
             raise K.SamdError(f"prompt + max_new_tokens + one step = {n_max + max_new_tokens + T} exceeds the automaton "
                               f"capacity max_tokens={self.dyn.max_tokens}")
         reqs = self._with_sampling(((i, p, max_new_tokens) for i, p in enumerate(prompts)), sampling)
-        reqs = self._with_penalties(reqs, penalties)
-        out, acc, lps = [None] * B, [None] * B, [None] * B
-        for i, tokens, hist, _, lp in self._run(reqs, max_new_tokens, graph, check_every, sampling is not None, logprobs,
-                                                penalties is not None):
-            out[i], acc[i], lps[i] = tokens, hist, lp
+        reqs = self._with_stops(self._with_penalties(reqs, penalties), stop, self.lm.config.vocab_size)
+        out, acc, lps, why, hits = [None] * B, [None] * B, [None] * B, [None] * B, [None] * B
+        for i, tokens, hist, _, lp, reason, hit in self._run(reqs, max_new_tokens, graph, check_every, sampling is not None,
+                                                             logprobs, penalties is not None, stop is not None):
+            out[i], acc[i], lps[i], why[i], hits[i] = tokens, hist, lp, reason, hit
         n_live = max(len(a) for a in acc)
         s = self._run_stats
         stats = dict(steps=n_live, steps_run=s["steps_run"], host_syncs=s["host_syncs"], graphed=s["graphed"],
-                     graphs=s["graphs"], accept_lengths=[a + [0] * (n_live - len(a)) for a in acc], **self._extra_stats())
+                     graphs=s["graphs"], accept_lengths=[a + [0] * (n_live - len(a)) for a in acc], finish_reasons=why,
+                     **self._extra_stats())
+        if stop is not None:
+            stats["stop_indices"] = hits
         if logprobs is not None:
             stats["logprobs"] = [lp[0] for lp in lps]
             if logprobs:
@@ -939,11 +1019,12 @@ class BatchedSamdDecoder:
     @torch.inference_mode()
     def serve(self, prompts: Iterable[Sequence[int]], max_new_tokens: Union[int, Sequence[int]], graph: bool = True,
               check_every: int = 4, sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None,
-              logprobs: Optional[int] = None, penalties: Union[None, Penalties, Sequence[Penalties]] = None):
+              logprobs: Optional[int] = None, penalties: Union[None, Penalties, Sequence[Penalties]] = None,
+              stop: Union[None, StopSequences, Sequence[StopSequences]] = None):
         """Continuous batching: decode any number of requests through the B slots, refilling a slot with the next queued
         request as soon as the host sees its request finished (once every `check_every` steps).  `prompts` is consumed
         lazily and in order; `max_new_tokens` is one limit for all or a sequence with one per request.  Yields
-        (index, tokens, {"slot", "accept_lengths"}) per request in completion order; `tokens` are what generate() emits
+        (index, tokens, {"slot", "accept_lengths", "finish_reason"}) per request in completion order; `tokens` are what generate() emits
         for that prompt, `accept_lengths` has one entry per live decode step.  A request is validated when it is pulled
         (SamdError naming its index).  self.serve_stats is set once the generator is exhausted: steps_run, host_syncs
         (flag reads), graphed, graphs, admissions, live_slot_steps (slot-steps of unfinished requests) and, for
@@ -973,7 +1054,17 @@ class BatchedSamdDecoder:
         top-p and top-k when sampled).  A row is penalized from its own context: the prompt, the tokens emitted so far
         and the draft tokens on its path, so greedy decoding stays lossless against plain penalized greedy decoding.
         Tree mode (tree=) is allowed; its successor table then learns from penalized rows, which changes drafts, not
-        tokens.  Neutral Penalties() give the tokens of penalties=None."""
+        tokens.  Neutral Penalties() give the tokens of penalties=None.
+
+        info["finish_reason"] says why a request ended: "stop" (EOS or a stop sequence), "length" (max_new_tokens) or
+        "cache" (a step could run past max_cache_len).  `stop` (None: none): one StopSequences for every request or a
+        sequence with one per request.  The output ends at the earliest output position where one of the request's
+        sequences ends - the prompt is never matched, a sequence may end inside a step or straddle two - so `tokens`
+        (and `logprobs`) are a prefix of what the request emits without stop, ending with the matched tokens;
+        info["stop_index"] is the index of the matched sequence in the request's list (the lowest among those ending
+        there), None when none ended it.  A sequence that would complete after max_new_tokens does not fire; one that
+        ends on EOS does.  The match runs on the device in the step (one samd_stop_match launch), so a stopped request
+        frees its slot and emits nothing more from that step on."""
         logprobs = _check_logprobs(logprobs)
         self.serve_stats = None
         if hasattr(max_new_tokens, "__len__"):
@@ -982,10 +1073,13 @@ class BatchedSamdDecoder:
         else:
             limits, max_limit = None, int(max_new_tokens)
         reqs = self._with_sampling(self._requests(prompts, max_new_tokens if limits is None else limits), sampling)
-        reqs = self._with_penalties(reqs, penalties)
-        for i, tokens, hist, slot, lp in self._run(reqs, max(max_limit, 1), graph, check_every, sampling is not None,
-                                                   logprobs, penalties is not None):
-            info = {"slot": slot, "accept_lengths": hist}
+        reqs = self._with_stops(self._with_penalties(reqs, penalties), stop, self.lm.config.vocab_size)
+        for i, tokens, hist, slot, lp, reason, hit in self._run(reqs, max(max_limit, 1), graph, check_every,
+                                                                sampling is not None, logprobs, penalties is not None,
+                                                                stop is not None):
+            info = {"slot": slot, "accept_lengths": hist, "finish_reason": reason}
+            if stop is not None:
+                info["stop_index"] = hit
             if self._prefixes is not None:
                 info["prefix_len"] = self._slot_plen[slot]
             if lp is not None:
@@ -1073,6 +1167,34 @@ class BatchedSamdDecoder:
             if bad:
                 raise K.SamdError(f"request {i}: {bad}")
             yield i, p, limit, sp, pn
+
+    @staticmethod
+    def _with_stops(requests: Iterator[tuple], stop, vocab: int) -> Iterator[tuple]:
+        """(index, prompt, limit, SamplingParams or None, Penalties or None, StopSequences or None) of every request: the
+        shared StopSequences or its own, checked against the vocabulary as it is pulled."""
+        shared = stop is None or isinstance(stop, StopSequences)
+        if not shared:
+            try:
+                stop = list(stop)
+            except TypeError:
+                raise K.SamdError(f"stop must be None, a StopSequences or a sequence of them, got "
+                                  f"{type(stop).__name__}") from None
+        for i, p, limit, sp, pn in requests:
+            if stop is None:
+                yield i, p, limit, sp, pn, None
+                continue
+            if shared:
+                ss = stop
+            elif i >= len(stop):
+                raise K.SamdError(f"request {i}: stop has {len(stop)} values, fewer than the prompts")
+            else:
+                ss = stop[i]
+            if not isinstance(ss, StopSequences):
+                raise K.SamdError(f"request {i}: stop must be a StopSequences, got {type(ss).__name__}")
+            bad = ss.problem(vocab)
+            if bad:
+                raise K.SamdError(f"request {i}: {bad}")
+            yield i, p, limit, sp, pn, ss
 
 
 class BatchedSamOnlyDecoder(BatchedSamdDecoder):

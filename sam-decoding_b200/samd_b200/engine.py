@@ -588,6 +588,53 @@ def apply_penalties(logits: torch.Tensor, counts: torch.Tensor, repetition: torc
     return logits
 
 
+def match_stops(tokens: torch.Tensor, count: torch.Tensor, hist: torch.Tensor, hist_len: torch.Tensor,
+                stop_tokens: torch.Tensor, stop_len: torch.Tensor, done: Optional[torch.Tensor] = None,
+                out_count: Optional[torch.Tensor] = None, out_hit: Optional[torch.Tensor] = None) -> tuple:
+    """samd_stop_match: where each request's output of this step ends, one launch.  Request b has emitted
+    hist[b, :hist_len[b]] (int32 [B, H]) and this step would emit tokens[b, :count[b]] (int32 [B, W], W <= 256).
+    Its stop sequences are stop_tokens[b, j, :stop_len[b, j]] (int32 [B, 16, 16] and [B, 16]; length 0 = unused, at most
+    16 ids).  A sequence matches where it ends the output at a step position i < count, against output tokens only
+    (never before output position 0).  Returns (out_count, out_hit) int32 [B]: e + 1 and the lowest sequence index
+    ending at the earliest such position e, or count and -1 (also for a `done` request or count 0).  out_count may be
+    `count` itself; passing both outputs makes a captured call allocate nothing.  Every argument is checked before
+    anything reaches the device."""
+    if tokens.dim() != 2 or not 1 <= tokens.shape[1] <= 256:
+        raise K.SamdError(f"match_stops: tokens must be [B, W] with 1 <= W <= 256, got {tuple(tokens.shape)}")
+    B, W = tokens.shape
+    if hist.dim() != 2 or hist.shape[0] != B or hist.shape[1] == 0:
+        raise K.SamdError(f"match_stops: hist must be [{B}, H] with H >= 1, got {tuple(hist.shape)}")
+    S, L = K.STOP_MAX_SEQS, K.STOP_MAX_LEN
+    for name, t, shape, dtypes in (("tokens", tokens, (B, W), (torch.int32,)), ("count", count, (B,), (torch.int32,)),
+                                   ("hist", hist, tuple(hist.shape), (torch.int32,)),
+                                   ("hist_len", hist_len, (B,), (torch.int32,)),
+                                   ("stop_tokens", stop_tokens, (B, S, L), (torch.int32,)),
+                                   ("stop_len", stop_len, (B, S), (torch.int32,)),
+                                   ("done", done, (B,), (torch.bool, torch.uint8)),
+                                   ("out_count", out_count, (B,), (torch.int32,)), ("out_hit", out_hit, (B,), (torch.int32,))):
+        if t is None:
+            continue
+        if tuple(t.shape) != shape or t.dtype not in dtypes or not t.is_contiguous():
+            raise K.SamdError(f"match_stops: {name} must be a contiguous {shape} {dtypes[0]} tensor, got "
+                              f"{tuple(t.shape)} {t.dtype}")
+    tensors = [tokens, count, hist, hist_len, stop_tokens, stop_len] + [x for x in (done, out_count, out_hit)
+                                                                         if x is not None]
+    if not all(t.is_cuda and t.device == tokens.device for t in tensors):
+        raise K.SamdError("match_stops: every tensor must be on the tokens' GPU")
+    if out_count is None:
+        out_count = torch.empty(B, dtype=torch.int32, device=tokens.device)
+    if out_hit is None:
+        out_hit = torch.empty(B, dtype=torch.int32, device=tokens.device)
+    a = K.StopArgs()
+    a.batch, a.width, a.tokens_dev, a.count_dev = B, W, tokens.data_ptr(), count.data_ptr()
+    a.hist_dev, a.hist_stride, a.hist_len_dev = hist.data_ptr(), hist.shape[1], hist_len.data_ptr()
+    a.stop_tokens_dev, a.stop_len_dev, a.done_dev = stop_tokens.data_ptr(), stop_len.data_ptr(), K.ptr(done)
+    a.out_count_dev, a.out_hit_dev = out_count.data_ptr(), out_hit.data_ptr()
+    with torch.cuda.device(tokens.device):
+        K.check(K.lib().samd_stop_match(C.byref(a), K.stream_ptr()), "samd_stop_match")
+    return out_count, out_hit
+
+
 class Verifier:
     """Fused greedy verification + KV compaction (samd/utils.py:127-141, samd/samd_model.py:159-211,
     samd/cache.py:118-133) for a batch of requests: one persistent launch."""
