@@ -389,7 +389,7 @@ typedef struct samd_sample_args {
     const int32_t *retrieve_dev;      /* [P][D] shared, or [B][P][D] when retrieve_batch_stride != 0; NULL = one identity path */
     int32_t        n_paths, depth;
     int64_t        retrieve_batch_stride;
-    const int32_t *n_paths_dev;       /* [B] live paths per request, or NULL */
+    const int32_t *n_paths_dev;       /* [B] live paths per request (<= n_paths), or NULL */
     float          temperature;       /* >= 1e-5 */
     float          top_p;             /* active when 1e-8 <= top_p < 1 */
     int32_t        top_k;             /* active when > 0 */

@@ -28,7 +28,7 @@
 #include <string.h>
 
 #define ST 256                 // threads per CTA
-#define MAX_REJ 64             // distinct rejected tokens remembered per level (>= paths sharing a prefix)
+#define MAX_REJ 64             // distinct rejected tokens of a level listed in shared memory (see kWide)
 #define MAX_GREEDY_T 256       // node rows of a request with greedy requests in the launch
 
 struct PhiloxState {
@@ -249,7 +249,30 @@ struct SampleParams {
     samd_sample_request_args r;                                 // every pointer NULL: the shared scalars of `a`
 };
 
-template <int kDtype>
+// Until a level accepts, every candidate tested there is rejected: at level `level`, token x has been rejected before
+// path `upto` iff it is cand(p', level) of an earlier path p' that shares path prefix_of's first `level` tokens
+// (candidate_tokens = tokens_ext[retrieve]: -1 picks the appended 0, as in the kernel's cand)
+__device__ __forceinline__ bool level_has(const samd_sample_args &A, int b, const int32_t *tok, int x, int upto, int level,
+                                          int prefix_of) {
+    auto cand = [&](int p, int j) {
+        const int r = A.retrieve_dev ? A.retrieve_dev[(size_t)b * A.retrieve_batch_stride + (size_t)p * A.depth + j] : j;
+        return r < 0 ? 0 : tok[r];
+    };
+    for (int p = 0; p < upto; ++p) {
+        if (cand(p, level) != x) continue;
+        bool eq = true;
+        for (int j = 0; j < level && eq; ++j) eq = cand(p, j) == cand(prefix_of, j);
+        if (eq) return true;
+    }
+    return false;
+}
+
+// kWide: the path table has more than MAX_REJ paths, so a level may reject more tokens than s_rej lists.  Then a
+// token past the list is found in the path table with level_has.  That costs up to n_paths prefix
+// comparisons for every kept token in each of the three passes over the vocabulary - slow, but only a caller passing
+// more than 64 paths through the C ABI gets there (the batched decoders' trees have at most 8 children per node), and
+// the host picks this instantiation from the table's width, so the common one compiles without it.
+template <int kDtype, bool kWide>
 __global__ void __launch_bounds__(ST) verify_sample_kernel(SampleParams P) {
     __shared__ float s_red[ST / 32];
     __shared__ unsigned long long s_red64[ST / 32];
@@ -324,7 +347,7 @@ __global__ void __launch_bounds__(ST) verify_sample_kernel(SampleParams P) {
         rng.off = A.offsets_dev[b];
         rng.used = 0;
     }
-    int accept_len = 1, best = 0, n_rej = 0;
+    int accept_len = 1, best = 0, n_rej = 0;                    // n_rej: rejected tokens of the level (kWide: all)
     bool adjust = false;
     RowDist dist;                                               // the last level's processed distribution
     size_t dist_off = 0;
@@ -349,7 +372,12 @@ __global__ void __launch_bounds__(ST) verify_sample_kernel(SampleParams P) {
             if (!eq) continue;
             const int x = cand(p, i);
             bool seen = false;
-            for (int q = 0; q < n_rej; ++q) seen |= s_rej[q] == x;
+            if constexpr (kWide) {
+                for (int q = 0; q < min(n_rej, MAX_REJ); ++q) seen |= s_rej[q] == x;
+                if (!seen && n_rej > MAX_REJ) seen = level_has(A, b, tok, x, p, i, best);
+            } else {
+                for (int q = 0; q < n_rej; ++q) seen |= s_rej[q] == x;
+            }
             if (seen) continue;
             const float r = philox_uniform(rng);
             const float px = prob_of<kDtype>(dist, A.logits_dev, dist_off, x) / (1.0f - rej_mass);
@@ -362,7 +390,8 @@ __global__ void __launch_bounds__(ST) verify_sample_kernel(SampleParams P) {
             __syncthreads();
             if (threadIdx.x == 0 && n_rej < MAX_REJ) s_rej[n_rej] = x;
             __syncthreads();
-            n_rej = min(n_rej + 1, MAX_REJ);
+            if constexpr (kWide) n_rej += 1;
+            else n_rej = min(n_rej + 1, MAX_REJ);
             adjust = true;
         }
     }
@@ -374,9 +403,16 @@ __global__ void __launch_bounds__(ST) verify_sample_kernel(SampleParams P) {
         n_rej = 0;
     }
     auto p_next = [&](int x) {
-        for (int q = 0; q < n_rej; ++q)
-            if (s_rej[q] == x) return 0.f;
-        return prob_of<kDtype>(dist, A.logits_dev, dist_off, x);
+        if constexpr (kWide) {
+            for (int q = 0; q < min(n_rej, MAX_REJ); ++q)
+                if (s_rej[q] == x) return 0.f;
+            const float px = prob_of<kDtype>(dist, A.logits_dev, dist_off, x);
+            return n_rej > MAX_REJ && px > 0.f && level_has(A, b, tok, x, n_paths, accept_len, best) ? 0.f : px;
+        } else {
+            for (int q = 0; q < n_rej; ++q)
+                if (s_rej[q] == x) return 0.f;
+            return prob_of<kDtype>(dist, A.logits_dev, dist_off, x);
+        }
     };
     // inverse-CDF draw in index order: contiguous blocks per thread, a scan over the blocks, then inside the block
     const int chunk = (V + ST - 1) / ST;
@@ -433,8 +469,11 @@ extern "C" int samd_verify_sample_requests(const samd_sample_args *a, const samd
     P.a = *a;
     if (r) P.r = *r;
     else memset(&P.r, 0, sizeof(P.r));
-    auto kern = a->dtype == SAMD_DTYPE_BF16 ? verify_sample_kernel<SAMD_DTYPE_BF16>
-                : a->dtype == SAMD_DTYPE_FP16 ? verify_sample_kernel<SAMD_DTYPE_FP16> : verify_sample_kernel<SAMD_DTYPE_FP32>;
+    // a level can reject more than MAX_REJ distinct tokens only if the table has more paths than that
+    const bool wide = a->retrieve_dev && a->n_paths > MAX_REJ;
+    auto kern = a->dtype == SAMD_DTYPE_BF16 ? (wide ? verify_sample_kernel<SAMD_DTYPE_BF16, true> : verify_sample_kernel<SAMD_DTYPE_BF16, false>)
+                : a->dtype == SAMD_DTYPE_FP16 ? (wide ? verify_sample_kernel<SAMD_DTYPE_FP16, true> : verify_sample_kernel<SAMD_DTYPE_FP16, false>)
+                : (wide ? verify_sample_kernel<SAMD_DTYPE_FP32, true> : verify_sample_kernel<SAMD_DTYPE_FP32, false>);
     kern<<<a->batch, ST, 0, (cudaStream_t)stream>>>(P);
     samd_count_launch();
     SAMD_CUDA(cudaGetLastError());
