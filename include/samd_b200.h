@@ -516,6 +516,53 @@ typedef struct samd_stop_args {
 } samd_stop_args;
 int samd_stop_match(const samd_stop_args *args, void *stream);
 
+/* Logit bias, banned token sequences and min_tokens on the draft rows of a batch, in place, after any penalties and
+ * before a verify launch reads them.  Row j < n_nodes_dev[b] of row-batch b belongs to state row s = slots_dev[b] (NULL:
+ * s = b).  Its context is the output so far, hist_dev[s][0 .. hist_len_dev[s]) (NULL hist_len_dev: empty), then the node
+ * tokens on the path from node 0 to node j, both included; node 0 sits at output position hist_len, so a node at depth d
+ * predicts output position hist_len + d + 1.  NULL tokens_dev is the admission form: no node tokens, every row predicts
+ * position hist_len.  In this order:
+ *   - bias: for each of the slot's bias_n_dev[s] entries (distinct ids), x = round_to_dtype(fp32(x) + bias); a -inf bias
+ *     stores -inf (a ban, whatever x was).  -inf stays -inf and NaN stays NaN under a finite bias.
+ *   - bans, each storing -inf: for every bad word (bad_len_dev[s][k] = L in [1, 16]; 0 = unused) whose first L - 1 ids
+ *     end the row's context, its last id (L = 1: banned on every row); and on a row predicting a position below
+ *     min_tokens_dev[s], eos_token (>= 0) and, for every stop sequence whose first L - 1 ids end the context, its last id.
+ * The context never reaches before output position 0, and only its last SAMD_BAD_MAX_LEN - 1 tokens are read.
+ * Untouched: done requests, slots with no bias, no bad word and min_tokens 0, rows at or past n_nodes_dev[b], and, with a
+ * path table, rows on none of the request's first n_paths_dev[b] paths (a path ends at its first -1).  Every (row, token)
+ * is read-modify-written at most once; the results depend only on the inputs and no argument depends on the step, so the
+ * launch can be captured in a CUDA graph. */
+#define SAMD_BIAS_MAX     256
+#define SAMD_BAD_MAX_SEQS 16
+#define SAMD_BAD_MAX_LEN  16
+typedef struct samd_logit_control_args {
+    void          *logits_dev;        /* [B][n_nodes][V], dtype below, rewritten in place */
+    int32_t        dtype;             /* SAMD_DTYPE_* */
+    int32_t        batch, n_nodes, vocab;          /* n_nodes <= 256 */
+    int64_t        batch_stride, row_stride;       /* in elements */
+    const int32_t *tokens_dev;        /* [B][n_nodes] node tokens, or NULL = the admission form */
+    const int32_t *retrieve_dev;      /* [B][n_paths][depth] path table, -1 padded, or NULL = the identity chain */
+    int32_t        n_paths, depth;
+    const int32_t *n_nodes_dev;       /* [B] live rows per request, or NULL = n_nodes */
+    const int32_t *n_paths_dev;       /* [B] live paths per request, or NULL = n_paths */
+    const uint8_t *done_dev;          /* [B] 1 = finished: not touched, or NULL */
+    const int32_t *slots_dev;         /* [B] state row of each row-batch entry, or NULL = identity */
+    int32_t        n_slots;           /* S */
+    const int32_t *hist_dev;          /* [S][hist_stride] output emitted so far (may be NULL without hist_len_dev) */
+    int32_t        hist_stride;
+    const int32_t *hist_len_dev;      /* [S], or NULL = 0 */
+    const int32_t *bias_ids_dev;      /* [S][SAMD_BIAS_MAX] distinct token ids */
+    const float   *bias_dev;          /* [S][SAMD_BIAS_MAX] finite or -inf */
+    const int32_t *bias_n_dev;        /* [S] entries in use */
+    const int32_t *bad_tokens_dev;    /* [S][SAMD_BAD_MAX_SEQS][SAMD_BAD_MAX_LEN] */
+    const int32_t *bad_len_dev;       /* [S][SAMD_BAD_MAX_SEQS], 0 = unused */
+    const int32_t *min_tokens_dev;    /* [S] */
+    const int32_t *stop_tokens_dev;   /* [S][SAMD_STOP_MAX_SEQS][SAMD_STOP_MAX_LEN], or NULL = no stop sequences */
+    const int32_t *stop_len_dev;      /* [S][SAMD_STOP_MAX_SEQS], 0 = unused (NULL with stop_tokens_dev) */
+    int32_t        eos_token;         /* -1 = none */
+} samd_logit_control_args;
+int samd_apply_logit_controls(const samd_logit_control_args *args, void *stream);
+
 /* TokenRecycle.gen_draft (token_recycle.py:49-59) for a batch: tokens[b][0] = start_tok[b]; every other node takes
  * table[token of its parent][its rank among the parent's children], or 0 when the parent's token has no entry.
  * parent / rank: [n_nodes] device arrays describing the static tree (node 0 = root, parents before children);

@@ -23,6 +23,9 @@ DTYPE_FP16 = 1
 DTYPE_FP32 = 2
 STOP_MAX_SEQS = 16
 STOP_MAX_LEN = 16
+BIAS_MAX = 256
+BAD_MAX_SEQS = 16
+BAD_MAX_LEN = 16
 
 c_i32p = C.POINTER(C.c_int32)
 c_i64p = C.POINTER(C.c_int64)
@@ -96,6 +99,17 @@ class StopArgs(C.Structure):
         ("batch", C.c_int32), ("width", C.c_int32), ("tokens_dev", vp), ("count_dev", vp), ("hist_dev", vp),
         ("hist_stride", C.c_int32), ("hist_len_dev", vp), ("stop_tokens_dev", vp), ("stop_len_dev", vp), ("done_dev", vp),
         ("out_count_dev", vp), ("out_hit_dev", vp),
+    ]
+
+
+class LogitControlArgs(C.Structure):
+    _fields_ = [
+        ("logits_dev", vp), ("dtype", C.c_int32), ("batch", C.c_int32), ("n_nodes", C.c_int32), ("vocab", C.c_int32),
+        ("batch_stride", C.c_int64), ("row_stride", C.c_int64), ("tokens_dev", vp), ("retrieve_dev", vp),
+        ("n_paths", C.c_int32), ("depth", C.c_int32), ("n_nodes_dev", vp), ("n_paths_dev", vp), ("done_dev", vp),
+        ("slots_dev", vp), ("n_slots", C.c_int32), ("hist_dev", vp), ("hist_stride", C.c_int32), ("hist_len_dev", vp),
+        ("bias_ids_dev", vp), ("bias_dev", vp), ("bias_n_dev", vp), ("bad_tokens_dev", vp), ("bad_len_dev", vp),
+        ("min_tokens_dev", vp), ("stop_tokens_dev", vp), ("stop_len_dev", vp), ("eos_token", C.c_int32),
     ]
 
 
@@ -183,6 +197,7 @@ SYMBOLS = {
     "samd_token_logprobs": (C.c_int, [C.POINTER(LogprobArgs), vp]),
     "samd_apply_penalties": (C.c_int, [C.POINTER(PenaltyArgs), vp]),
     "samd_stop_match": (C.c_int, [C.POINTER(StopArgs), vp]),
+    "samd_apply_logit_controls": (C.c_int, [C.POINTER(LogitControlArgs), vp]),
     "samd_recycle_gen_tree": (C.c_int, [vp, C.c_int32, vp, vp, C.c_int32, vp, vp, C.c_int32, C.c_int32, vp, vp]),
     "samd_verify_set_chunk": (None, [C.c_int]),
     "samd_verify_set_overlap": (None, [C.c_int]),

@@ -52,13 +52,19 @@ may end inside a step or straddle two: after the EOS cut, one samd_stop_match la
 earliest match among the tokens the step would emit (and the last 15 it emitted before), and the commit emits up to it.
 Every request also gets a finish reason: "stop" (EOS or a stop sequence), "length" (max_new_tokens) or "cache" (the
 max_cache_len guard).
+
+generate(..., controls=...) and serve(..., controls=...) add a logit bias, banned token sequences ("bad words") and
+min_tokens (LogitControls, one per request).  Like the penalties they depend on each draft row's own context - the
+output so far plus the draft tokens on its path - and on the output position it predicts, so one
+samd_apply_logit_controls launch rewrites every live row right after the penalties, and greedy verification stays
+lossless against plain controlled greedy decoding.
 """
 from __future__ import annotations
 
 import dataclasses
 import math
 import numbers
-from typing import Iterable, Iterator, List, Optional, Sequence, Union
+from typing import Iterable, Iterator, List, Mapping, Optional, Sequence, Tuple, Union
 
 import torch
 from transformers.cache_utils import Cache, CacheLayerMixin
@@ -134,19 +140,77 @@ class StopSequences:
 
     def problem(self, vocab: int) -> Optional[str]:
         """What is wrong with these sequences for a vocabulary of `vocab` tokens (None: nothing)."""
-        seqs = self.sequences
-        if not isinstance(seqs, (list, tuple)):
-            return f"sequences must be a list or tuple of token id sequences, got {type(seqs).__name__}"
-        if len(seqs) > K.STOP_MAX_SEQS:
-            return f"at most {K.STOP_MAX_SEQS} sequences, got {len(seqs)}"
-        for j, seq in enumerate(seqs):
-            if not isinstance(seq, (list, tuple)):
-                return f"sequence {j} must be a list or tuple of token ids, got {type(seq).__name__}"
-            if not 1 <= len(seq) <= K.STOP_MAX_LEN:
-                return f"sequence {j} must have 1 to {K.STOP_MAX_LEN} token ids, got {len(seq)}"
-            for t in seq:
-                if isinstance(t, bool) or not isinstance(t, numbers.Integral) or not 0 <= t < vocab:
-                    return f"sequence {j}: token ids must be ints in [0, {vocab}), got {t!r}"
+        return _sequences_problem(self.sequences, vocab, "sequences", "sequence", K.STOP_MAX_SEQS, K.STOP_MAX_LEN)
+
+
+def _sequences_problem(seqs, vocab: int, field: str, item: str, max_seqs: int, max_len: int) -> Optional[str]:
+    """What is wrong with a list of token id sequences `seqs` (the field `field`, whose entries are called `item`): at
+    most max_seqs sequences of 1 to max_len ids in [0, vocab) each (None: nothing)."""
+    if not isinstance(seqs, (list, tuple)):
+        return f"{field} must be a list or tuple of token id sequences, got {type(seqs).__name__}"
+    if len(seqs) > max_seqs:
+        return f"at most {max_seqs} {item}s, got {len(seqs)}"
+    for j, seq in enumerate(seqs):
+        if not isinstance(seq, (list, tuple)):
+            return f"{item} {j} must be a list or tuple of token ids, got {type(seq).__name__}"
+        if not 1 <= len(seq) <= max_len:
+            return f"{item} {j} must have 1 to {max_len} token ids, got {len(seq)}"
+        for t in seq:
+            if isinstance(t, bool) or not isinstance(t, numbers.Integral) or not 0 <= t < vocab:
+                return f"{item} {j}: token ids must be ints in [0, {vocab}), got {t!r}"
+    return None
+
+
+@dataclasses.dataclass(frozen=True)
+class LogitControls:
+    """Logit controls of one request, applied to every logits row after the penalties and before temperature, top-p and
+    top-k.  The decoders check the values of every request when it is pulled and name its index in the error.
+
+    logit_bias: {token_id: bias} or a sequence of (token_id, bias) pairs (a repeated id is an error), at most 256
+    distinct ids in [0, V).  A bias is a float in [-100, 100] (the OpenAI range), added to the logit in fp32 and rounded
+    once into the logits' dtype, or -inf: the token is banned.
+    bad_words: at most 16 sequences of 1 to 16 token ids.  Where the request's context - its output so far, never the
+    prompt, then the tokens a draft row's path adds - ends with a sequence's first L - 1 ids, its last id is banned (a
+    one-id sequence is banned everywhere), so the output never contains a bad word.
+    min_tokens: an int m in [0, max_new_tokens].  While fewer than m tokens have been emitted, the decoder's
+    eos_token_id and the last id of every stop sequence (stop=) whose head ends the context are banned, so neither EOS
+    nor a stop sequence ends the request before m tokens (HF's MinNewTokensLengthLogitsProcessor, extended to
+    multi-token stops); the max_cache_len guard still may.
+    A banned token's logit is -inf.  LogitControls() changes nothing."""
+    logit_bias: Union[Mapping[int, float], Sequence[Tuple[int, float]]] = ()
+    bad_words: Sequence[Sequence[int]] = ()
+    min_tokens: int = 0
+
+    def bias_items(self) -> list:
+        """logit_bias as a list of (token_id, bias) pairs."""
+        lb = self.logit_bias
+        return list(lb.items()) if isinstance(lb, Mapping) else list(lb)
+
+    def problem(self, vocab: int) -> Optional[str]:
+        """What is wrong with these values for a vocabulary of `vocab` tokens (None: nothing)."""
+        lb = self.logit_bias
+        if not isinstance(lb, (Mapping, list, tuple)):
+            return f"logit_bias must be a mapping or a sequence of (token_id, bias) pairs, got {type(lb).__name__}"
+        seen = set()
+        for k, pair in enumerate(self.bias_items()):
+            if not isinstance(pair, (list, tuple)) or len(pair) != 2:
+                return f"logit_bias entry {k} must be a (token_id, bias) pair, got {pair!r}"
+            t, v = pair
+            if isinstance(t, bool) or not isinstance(t, numbers.Integral) or not 0 <= t < vocab:
+                return f"logit_bias: token ids must be ints in [0, {vocab}), got {t!r}"
+            if int(t) in seen:
+                return f"logit_bias: token id {int(t)} appears more than once"
+            seen.add(int(t))
+            if isinstance(v, bool) or not isinstance(v, numbers.Real) or not (-100.0 <= v <= 100.0 or v == -math.inf):
+                return f"logit_bias: the bias of token {int(t)} must be a float in [-100, 100] or -inf, got {v!r}"
+        if len(seen) > K.BIAS_MAX:
+            return f"logit_bias: at most {K.BIAS_MAX} token ids, got {len(seen)}"
+        bad = _sequences_problem(self.bad_words, vocab, "bad_words", "bad word", K.BAD_MAX_SEQS, K.BAD_MAX_LEN)
+        if bad:
+            return bad
+        m = self.min_tokens
+        if isinstance(m, bool) or not isinstance(m, numbers.Integral) or m < 0:
+            return f"min_tokens must be an int >= 0, got {m!r}"
         return None
 
 
@@ -364,6 +428,7 @@ class BatchedSamdDecoder:
         n_nodes, ret = self._n_nodes[kind].contiguous(), self._ret[kind].contiguous()
         n_paths = self._n_paths[kind].contiguous()
         self._penalize(logits, draft, ret, n_nodes, n_paths)
+        self._control(logits, draft, ret, n_nodes, n_paths)
         return self.ver.verify(logits, draft, ret, cache_len=self.cache.cache_len, move_kv=True, n_nodes=n_nodes,
                                n_paths=n_paths, out=res, recycle=self.table), logits, n_nodes
 
@@ -381,6 +446,7 @@ class BatchedSamdDecoder:
         logits = self.lm(input_ids=draft.long(), position_ids=pos, past_key_values=cache,
                          attention_mask=self._mask(T, kv_len, cache.cache_len)).logits.contiguous()
         self._penalize(logits, draft)
+        self._control(logits, draft)
         if self._sampled:                                      # identity path: no row moves, the commit sets cache_len
             return self._verify_sample(logits, draft, None), logits, None
         return self.ver.verify(logits, draft, None, cache_len=cache.cache_len, out=st["res"]), logits, None
@@ -393,6 +459,19 @@ class BatchedSamdDecoder:
             st = self._st
             E.apply_penalties(logits, st["pen_counts"], st["pen_r"], st["pen_p"], st["pen_f"], tokens=tokens,
                               retrieve=retrieve, n_nodes=n_nodes, n_paths=n_paths, done=st["done"])
+
+    def _control(self, logits: torch.Tensor, tokens: torch.Tensor, retrieve: Optional[torch.Tensor] = None,
+                 n_nodes: Optional[torch.Tensor] = None, n_paths: Optional[torch.Tensor] = None):
+        """Right after _penalize, in a call with logit controls: every live draft row's bias, bad words and min_tokens
+        bans from its own context (the slot's output so far, then its path) and the output position it predicts, one
+        samd_apply_logit_controls launch.  Nothing otherwise."""
+        if self._controlled:
+            st = self._st
+            stops = dict(stop_tokens=st["stop_tok"], stop_len=st["stop_len"]) if self._stopped else {}
+            E.apply_logit_controls(logits, st["ctl_bias_ids"], st["ctl_bias"], st["ctl_bias_n"], st["ctl_bad_tok"],
+                                   st["ctl_bad_len"], st["ctl_min"], tokens=tokens, retrieve=retrieve, n_nodes=n_nodes,
+                                   n_paths=n_paths, done=st["done"], hist=st["out"], hist_len=st["out_len"],
+                                   eos=None if self.eos is None else int(self.eos), **stops)
 
     def _verify_sample(self, logits: torch.Tensor, tokens: torch.Tensor, retrieve: Optional[torch.Tensor], **kw) -> dict:
         """samd_verify_sample_requests with every slot's processor, greedy flag and Philox stream; finished slots make no
@@ -501,12 +580,13 @@ class BatchedSamdDecoder:
         return {}
 
     # ---- the step state, and the CUDA graphs that refer to it -------------------------------------------------------
-    def _init_state(self, max_limit: int, logprobs: bool = False, penalized: bool = False, stopped: bool = False):
+    def _init_state(self, max_limit: int, logprobs: bool = False, penalized: bool = False, stopped: bool = False,
+                    controlled: bool = False):
         """Zeroed step state for requests of at most `max_limit` new tokens.  The tensors persist across calls (the
         captured graphs refer to them, and limits are per slot); they are reallocated, and the graphs dropped, only when
         a call needs longer outputs than any before.  The log-probability state is added by the first call that asks
         for log-probabilities, the penalty state by the first call with penalties, the stop state by the first call with
-        stop sequences."""
+        stop sequences, the logit-control state by the first call with controls."""
         B, T, dev = self.B, self.T, self.device
         width = T if self.tree is None else self._ret.shape[2]
         cap = getattr(self, "_st_cap", None)
@@ -545,14 +625,22 @@ class BatchedSamdDecoder:
             S, L = K.STOP_MAX_SEQS, K.STOP_MAX_LEN
             i32 = lambda *sh: torch.zeros(*sh, dtype=torch.int32, device=dev)
             self._st.update(stop_tok=i32(B, S, L), stop_len=i32(B, S), stop_hit=i32(B), stop_step=i32(B))
+        if controlled and "ctl_min" not in self._st:
+            # ctl_bias_ids / ctl_bias / ctl_bias_n: every slot's logit bias entries; ctl_bad_tok / ctl_bad_len: its bad
+            # words (length 0: unused); ctl_min: its min_tokens
+            M, S, L = K.BIAS_MAX, K.BAD_MAX_SEQS, K.BAD_MAX_LEN
+            i32 = lambda *sh: torch.zeros(*sh, dtype=torch.int32, device=dev)
+            self._st.update(ctl_bias_ids=i32(B, M), ctl_bias=torch.zeros(B, M, device=dev), ctl_bias_n=i32(B),
+                            ctl_bad_tok=i32(B, S, L), ctl_bad_len=i32(B, S), ctl_min=i32(B))
 
     def _advance(self, kv_len: int, graph: bool) -> bool:
         """One decode step at key length `kv_len`: the bucket's CUDA graph, captured first if it is new, or the same body
-        eagerly (one graph per bucket, greedy / sampled body, logprobs setting, penalized or not and stopped or not).  Returns `graph`,
+        eagerly (one graph per bucket, greedy / sampled body, logprobs setting, penalized or not, stopped or not and
+        controlled or not).  Returns `graph`,
         False from then on when the LM's forward cannot be captured."""
         if graph:
             B, dev, graphs = self.B, self.device, self._graphs
-            key = (kv_len, self._sampled, self._logprobs, self._penalized, self._stopped)
+            key = (kv_len, self._sampled, self._logprobs, self._penalized, self._stopped, self._controlled)
             if key not in graphs:
                 # warm-up run on a side stream (allocations, lazy initialisation), state restored, then the capture
                 snap = {k: (v.clone() if torch.is_tensor(v) else v) for k, v in self._st.items() if k != "res"}
@@ -668,7 +756,7 @@ class BatchedSamdDecoder:
     # ---- admission: new requests into free slots, between two steps ---------------------------------------------------
     def _admit(self, reqs: List[tuple]) -> int:
         """Start the requests `reqs` = [(slot, prompt, limit, SamplingParams or None, Penalties or None, StopSequences or
-        None)] in their (free) slots; returns the longest prompt.  Only the persistent state is written, in place, so the captured graphs stay valid."""
+        None, LogitControls or None)] in their (free) slots; returns the longest prompt.  Only the persistent state is written, in place, so the captured graphs stay valid."""
         dev = self.device
         n_max = max(len(r[1]) for r in reqs)
         if self._prefixes is not None:
@@ -806,14 +894,28 @@ class BatchedSamdDecoder:
 
     def _set_slots(self, slots: torch.Tensor, lens: torch.Tensor, limits: torch.Tensor, rows: torch.Tensor,
                    reqs: List[tuple]):
-        """The admitted slots' step state: cache length, sampling parameters and a fresh Philox stream (sampled calls),
-        penalty state (penalized calls), first start token from `rows` [n, V] (the logits after each prompt, penalized
-        from the prompt alone in a penalized call: argmax, or a draw from the plain softmax) and, with logprobs, its
-        log-probability, stop sequences (calls with stops), limit, and zero emitted tokens / history."""
+        """The admitted slots' step state: cache length, stop sequences (calls with stops), sampling parameters and a
+        fresh Philox stream (sampled calls), penalty state (penalized calls), logit controls (controlled calls), first
+        start token from `rows` [n, V] (the logits after each prompt, penalized from the prompt alone in a penalized
+        call, then controlled as the row predicting output position 0 in a controlled one: argmax, or a draw from the
+        softmax) and, with logprobs, its log-probability, limit, and zero emitted tokens / history."""
         st, params = self._st, [r[3] for r in reqs]
         self.cache.cache_len.index_copy_(0, slots, lens)
+        if self._stopped:
+            n, S, L = len(reqs), K.STOP_MAX_SEQS, K.STOP_MAX_LEN
+            tab = [[0] * (S * L + S) for _ in reqs]                           # [stop_tok | stop_len] per request
+            for row, r in zip(tab, reqs):
+                for j, seq in enumerate(r[5].sequences):
+                    row[j * L:j * L + len(seq)] = [int(t) for t in seq]
+                    row[S * L + j] = len(seq)
+            tab = torch.tensor(tab, dtype=torch.int32).to(self.device)
+            st["stop_tok"].index_copy_(0, slots, tab[:, :S * L].reshape(n, S, L))
+            st["stop_len"].index_copy_(0, slots, tab[:, S * L:].contiguous())
+            st["stop_hit"].index_fill_(0, slots, -1)
         if self._penalized:
             rows = self._admit_penalties(slots, rows, reqs)
+        if self._controlled:
+            rows = self._admit_controls(slots, rows, reqs)
         if self._sampled:
             dev = self.device
             f = torch.tensor([[sp.temperature, sp.top_p] for sp in params], dtype=torch.float32).T.contiguous().to(dev)
@@ -844,17 +946,6 @@ class BatchedSamdDecoder:
                 st["start_ids"][slots, :n] = lp["next_top_ids"]
                 st["start_top"][slots, :n] = lp["next_top_logprob"]
         st["start"].index_copy_(0, slots, first)
-        if self._stopped:
-            n, S, L = len(reqs), K.STOP_MAX_SEQS, K.STOP_MAX_LEN
-            tab = [[0] * (S * L + S) for _ in reqs]                           # [stop_tok | stop_len] per request
-            for row, r in zip(tab, reqs):
-                for j, seq in enumerate(r[5].sequences):
-                    row[j * L:j * L + len(seq)] = [int(t) for t in seq]
-                    row[S * L + j] = len(seq)
-            tab = torch.tensor(tab, dtype=torch.int32).to(self.device)
-            st["stop_tok"].index_copy_(0, slots, tab[:, :S * L].reshape(n, S, L))
-            st["stop_len"].index_copy_(0, slots, tab[:, S * L:].contiguous())
-            st["stop_hit"].index_fill_(0, slots, -1)
         st["limit"].index_copy_(0, slots, limits)
         for k in ("acc_count", "out_len", "hlen"):
             st[k].index_fill_(0, slots, 0)
@@ -881,13 +972,45 @@ class BatchedSamdDecoder:
                           slots=slots.to(torch.int32))
         return rows
 
+    def _admit_controls(self, slots: torch.Tensor, rows: torch.Tensor, reqs: List[tuple]) -> torch.Tensor:
+        """The admitted slots' logit-control tables, and a controlled copy of `rows`: each is the row predicting output
+        position 0, with no context (the prefix pool's stored rows stay as they are)."""
+        st, n, V = self._st, len(reqs), rows.shape[-1]
+        M, S, L = K.BIAS_MAX, K.BAD_MAX_SEQS, K.BAD_MAX_LEN
+        ids, bias = torch.zeros(n, M, dtype=torch.int32), torch.zeros(n, M)
+        small = torch.zeros(n, 2 + S + S * L, dtype=torch.int32)                 # [bias_n | min | bad_len | bad_tok]
+        for i, r in enumerate(reqs):
+            lc = r[6]
+            items = lc.bias_items()
+            if items:
+                ids[i, :len(items)] = torch.tensor([int(t) for t, _ in items], dtype=torch.int32)
+                bias[i, :len(items)] = torch.tensor([float(v) for _, v in items], dtype=torch.float32)
+            small[i, 0], small[i, 1] = len(items), int(lc.min_tokens)
+            for j, seq in enumerate(lc.bad_words):
+                small[i, 2 + j] = len(seq)
+                small[i, 2 + S + j * L:2 + S + j * L + len(seq)] = torch.tensor([int(t) for t in seq], dtype=torch.int32)
+        ids, bias, small = ids.to(self.device), bias.to(self.device), small.to(self.device)
+        st["ctl_bias_ids"].index_copy_(0, slots, ids)
+        st["ctl_bias"].index_copy_(0, slots, bias)
+        st["ctl_bias_n"].index_copy_(0, slots, small[:, 0].contiguous())
+        st["ctl_min"].index_copy_(0, slots, small[:, 1].contiguous())
+        st["ctl_bad_len"].index_copy_(0, slots, small[:, 2:2 + S].contiguous())
+        st["ctl_bad_tok"].index_copy_(0, slots, small[:, 2 + S:].reshape(n, S, L))
+        stops = dict(stop_tokens=st["stop_tok"], stop_len=st["stop_len"]) if self._stopped else {}
+        rows = rows.clone()
+        E.apply_logit_controls(rows.view(n, 1, V), st["ctl_bias_ids"], st["ctl_bias"], st["ctl_bias_n"],
+                               st["ctl_bad_tok"], st["ctl_bad_len"], st["ctl_min"], slots=slots.to(torch.int32),
+                               eos=None if self.eos is None else int(self.eos), **stops)
+        return rows
+
     # ---- the decode loop of generate() and serve() --------------------------------------------------------------------
     def _run(self, requests: Iterator[tuple], max_limit: int, graph: bool, check_every: int, sampled: bool = False,
-             logprobs: Optional[int] = None, penalized: bool = False, stopped: bool = False):
+             logprobs: Optional[int] = None, penalized: bool = False, stopped: bool = False, controlled: bool = False):
         """Decode the validated requests (index, prompt, limit, SamplingParams or None, Penalties or None, StopSequences
-        or None) of `requests`, at most B at a time, with the greedy step body or (sampled) the sampled one; with
-        `logprobs` (0 .. 8) the step also scores the accepted rows, `penalized` penalizes the draft rows before
-        verification and `stopped` cuts each request's output at its first stop sequence.  The decode step has no host synchronisation in it: it is captured once per key-length bucket (64
+        or None, LogitControls or None) of `requests`, at most B at a time, with the greedy step body or (sampled) the
+        sampled one; with `logprobs` (0 .. 8) the step also scores the accepted rows, `penalized` penalizes the draft
+        rows before verification, `controlled` then applies each request's logit controls, and `stopped` cuts each
+        request's output at its first stop sequence.  The decode step has no host synchronisation in it: it is captured once per key-length bucket (64
         positions) as a CUDA graph and replayed.  Once every `check_every` steps the host reads [done | out_len | longest cache] in one copy; it then
         yields (index, tokens, accept_lengths, slot, (logprobs, top_logprobs) or None, finish reason, stop index or None)
         for every request found finished (their rows and stop indices in one more copy, their log-probabilities in one
@@ -896,8 +1019,9 @@ class BatchedSamdDecoder:
         finished request keeps its slot - riding along, emitting nothing - until that check.  Statistics go to
         self._run_stats."""
         B, T, dev = self.B, self.T, self.device
-        self._init_state(max_limit, logprobs is not None, penalized, stopped)
+        self._init_state(max_limit, logprobs is not None, penalized, stopped, controlled)
         self._sampled, self._logprobs, self._penalized, self._stopped = sampled, logprobs, penalized, stopped
+        self._controlled = controlled
         st = self._st
         run = self._run_id = getattr(self, "_run_id", 0) + 1
         self.eng.reset()
@@ -977,13 +1101,14 @@ class BatchedSamdDecoder:
     def generate(self, prompts: Sequence[Sequence[int]], max_new_tokens: int, graph: bool = True, check_every: int = 4,
                  sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None, logprobs: Optional[int] = None,
                  penalties: Union[None, Penalties, Sequence[Penalties]] = None,
-                 stop: Union[None, StopSequences, Sequence[StopSequences]] = None):
+                 stop: Union[None, StopSequences, Sequence[StopSequences]] = None,
+                 controls: Union[None, LogitControls, Sequence[LogitControls]] = None):
         """Lossless batched speculative decoding of exactly B prompts in lockstep (request b in slot b), up to
         max_new_tokens each.  The host reads the finished flags once every `check_every` steps - 1 / check_every host
         syncs per step - so a finished batch may run up to check_every - 1 idle steps (every request done: nothing is
         emitted).  graph=False runs the same body eagerly.  Returns (tokens per request, stats); stats["accept_lengths"]
         holds every request's accepted tokens per step, padded with 0 to the longest request's `steps`.  `sampling`,
-        `logprobs`, `penalties` and `stop`: as in serve(); with logprobs, stats["logprobs"] (and, for logprobs > 0,
+        `logprobs`, `penalties`, `stop` and `controls`: as in serve(); with logprobs, stats["logprobs"] (and, for logprobs > 0,
         stats["top_logprobs"]) hold every request's list.  stats["finish_reasons"] holds every request's finish reason
         and, with stop, stats["stop_indices"] its stop index."""
         logprobs = _check_logprobs(logprobs)
@@ -997,11 +1122,13 @@ class BatchedSamdDecoder:
         if n_max + max_new_tokens + T > self.dyn.max_tokens:
             raise K.SamdError(f"prompt + max_new_tokens + one step = {n_max + max_new_tokens + T} exceeds the automaton "
                               f"capacity max_tokens={self.dyn.max_tokens}")
+        V = self.lm.config.vocab_size
         reqs = self._with_sampling(((i, p, max_new_tokens) for i, p in enumerate(prompts)), sampling)
-        reqs = self._with_stops(self._with_penalties(reqs, penalties), stop, self.lm.config.vocab_size)
+        reqs = self._with_controls(self._with_stops(self._with_penalties(reqs, penalties), stop, V), controls, V)
         out, acc, lps, why, hits = [None] * B, [None] * B, [None] * B, [None] * B, [None] * B
         for i, tokens, hist, _, lp, reason, hit in self._run(reqs, max_new_tokens, graph, check_every, sampling is not None,
-                                                             logprobs, penalties is not None, stop is not None):
+                                                             logprobs, penalties is not None, stop is not None,
+                                                             controls is not None):
             out[i], acc[i], lps[i], why[i], hits[i] = tokens, hist, lp, reason, hit
         n_live = max(len(a) for a in acc)
         s = self._run_stats
@@ -1020,7 +1147,8 @@ class BatchedSamdDecoder:
     def serve(self, prompts: Iterable[Sequence[int]], max_new_tokens: Union[int, Sequence[int]], graph: bool = True,
               check_every: int = 4, sampling: Union[None, SamplingParams, Sequence[SamplingParams]] = None,
               logprobs: Optional[int] = None, penalties: Union[None, Penalties, Sequence[Penalties]] = None,
-              stop: Union[None, StopSequences, Sequence[StopSequences]] = None):
+              stop: Union[None, StopSequences, Sequence[StopSequences]] = None,
+              controls: Union[None, LogitControls, Sequence[LogitControls]] = None):
         """Continuous batching: decode any number of requests through the B slots, refilling a slot with the next queued
         request as soon as the host sees its request finished (once every `check_every` steps).  `prompts` is consumed
         lazily and in order; `max_new_tokens` is one limit for all or a sequence with one per request.  Yields
@@ -1064,7 +1192,17 @@ class BatchedSamdDecoder:
         info["stop_index"] is the index of the matched sequence in the request's list (the lowest among those ending
         there), None when none ended it.  A sequence that would complete after max_new_tokens does not fire; one that
         ends on EOS does.  The match runs on the device in the step (one samd_stop_match launch), so a stopped request
-        frees its slot and emits nothing more from that step on."""
+        frees its slot and emits nothing more from that step on.
+
+        `controls` (None: none): one LogitControls for every request or a sequence with one per request - a logit bias,
+        bad words and min_tokens (min_tokens <= the request's max_new_tokens), applied to every logits row after the
+        penalties and before temperature, top-p and top-k: first the bias, then the bans.  Each draft row is controlled
+        from its own context (the output so far and the draft tokens on its path) and the output position it predicts
+        (a row at path depth d predicts out_len + d + 1), so greedy decoding stays lossless against plain controlled
+        greedy decoding; the first token comes from the prompt's last row controlled as position 0.  All modes are
+        allowed; in tree mode the successor table learns from controlled rows (drafts change, tokens do not), and
+        logprobs are those of the controlled rows.  Neutral LogitControls() give the tokens of controls=None.  One
+        samd_apply_logit_controls launch per step and one per admission batch."""
         logprobs = _check_logprobs(logprobs)
         self.serve_stats = None
         if hasattr(max_new_tokens, "__len__"):
@@ -1072,11 +1210,12 @@ class BatchedSamdDecoder:
             max_limit = max(limits, default=1)
         else:
             limits, max_limit = None, int(max_new_tokens)
+        V = self.lm.config.vocab_size
         reqs = self._with_sampling(self._requests(prompts, max_new_tokens if limits is None else limits), sampling)
-        reqs = self._with_stops(self._with_penalties(reqs, penalties), stop, self.lm.config.vocab_size)
+        reqs = self._with_controls(self._with_stops(self._with_penalties(reqs, penalties), stop, V), controls, V)
         for i, tokens, hist, slot, lp, reason, hit in self._run(reqs, max(max_limit, 1), graph, check_every,
                                                                 sampling is not None, logprobs, penalties is not None,
-                                                                stop is not None):
+                                                                stop is not None, controls is not None):
             info = {"slot": slot, "accept_lengths": hist, "finish_reason": reason}
             if stop is not None:
                 info["stop_index"] = hit
@@ -1196,6 +1335,37 @@ class BatchedSamdDecoder:
                 raise K.SamdError(f"request {i}: {bad}")
             yield i, p, limit, sp, pn, ss
 
+    @staticmethod
+    def _with_controls(requests: Iterator[tuple], controls, vocab: int) -> Iterator[tuple]:
+        """(index, prompt, limit, SamplingParams or None, Penalties or None, StopSequences or None, LogitControls or None)
+        of every request: the shared LogitControls or its own, checked against the vocabulary and the request's
+        max_new_tokens as it is pulled."""
+        shared = controls is None or isinstance(controls, LogitControls)
+        if not shared:
+            try:
+                controls = list(controls)
+            except TypeError:
+                raise K.SamdError(f"controls must be None, a LogitControls or a sequence of them, got "
+                                  f"{type(controls).__name__}") from None
+        for i, p, limit, sp, pn, ss in requests:
+            if controls is None:
+                yield i, p, limit, sp, pn, ss, None
+                continue
+            if shared:
+                lc = controls
+            elif i >= len(controls):
+                raise K.SamdError(f"request {i}: controls has {len(controls)} values, fewer than the prompts")
+            else:
+                lc = controls[i]
+            if not isinstance(lc, LogitControls):
+                raise K.SamdError(f"request {i}: controls must be a LogitControls, got {type(lc).__name__}")
+            bad = lc.problem(vocab)
+            if bad:
+                raise K.SamdError(f"request {i}: {bad}")
+            if lc.min_tokens > limit:
+                raise K.SamdError(f"request {i}: min_tokens {lc.min_tokens} exceeds max_new_tokens {limit}")
+            yield i, p, limit, sp, pn, ss, lc
+
 
 class BatchedSamOnlyDecoder(BatchedSamdDecoder):
     """Batched decoding with the `samd_sam_only` flavour (samd_sam_only/samd_model.py:117-157 for B requests in lockstep):
@@ -1273,6 +1443,7 @@ class BatchedSamOnlyDecoder(BatchedSamdDecoder):
         logits = self.lm(input_ids=buf["tokens"].long(), position_ids=buf["position_ids"], past_key_values=cache,
                          attention_mask=mask[:, None]).logits.contiguous()
         self._penalize(logits, buf["tokens"], buf["retrieve"], buf["n_nodes"], buf["n_paths"])
+        self._control(logits, buf["tokens"], buf["retrieve"], buf["n_nodes"], buf["n_paths"])
         if self._sampled:
             # a request's own width - its draft length, or its tree's deepest path - so that the -1 pads beyond it are
             # never compared; then the accepted rows move into place

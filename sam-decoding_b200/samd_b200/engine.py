@@ -635,6 +635,95 @@ def match_stops(tokens: torch.Tensor, count: torch.Tensor, hist: torch.Tensor, h
     return out_count, out_hit
 
 
+def apply_logit_controls(logits: torch.Tensor, bias_ids: torch.Tensor, bias: torch.Tensor, bias_n: torch.Tensor,
+                         bad_tokens: torch.Tensor, bad_len: torch.Tensor, min_tokens: torch.Tensor,
+                         tokens: Optional[torch.Tensor] = None, retrieve: Optional[torch.Tensor] = None,
+                         n_nodes: Optional[torch.Tensor] = None, n_paths: Optional[torch.Tensor] = None,
+                         done: Optional[torch.Tensor] = None, slots: Optional[torch.Tensor] = None,
+                         hist: Optional[torch.Tensor] = None, hist_len: Optional[torch.Tensor] = None,
+                         stop_tokens: Optional[torch.Tensor] = None, stop_len: Optional[torch.Tensor] = None,
+                         eos: Optional[int] = None) -> torch.Tensor:
+    """samd_apply_logit_controls: logit bias, banned token sequences and min_tokens on the draft rows `logits` [B, T, V]
+    (fp32, bf16 or fp16, unit stride over V), in place, one launch; returns `logits`.  Per state row s = slots[b] (int32
+    [B]; None: s = b): `bias_ids` / `bias` [S, 256] (int32 distinct ids / float32 finite or -inf) with `bias_n` [S]
+    entries in use, `bad_tokens` / `bad_len` [S, 16, 16] / [S, 16] int32 (length 0 = unused), `min_tokens` [S] int32,
+    optionally the stop sequences `stop_tokens` / `stop_len` (as match_stops takes them) and the output so far,
+    hist[s, :hist_len[s]] (int32 [S, H] and [S]; None: empty).  Row j's context is that output, then the node tokens
+    `tokens` [B, T] on the path from node 0 to node j - the identity chain without `retrieve`, else the path of
+    `retrieve` [B, P, D] (-1 padded) that lists node j - and node 0 sits at output position hist_len, so a node at depth
+    d predicts position hist_len + d + 1.  tokens=None: no node tokens, every row predicts position hist_len (the
+    prompt's last row at admission).  Each biased entry becomes round(fp32(x) + bias) (a -inf bias stores -inf); then
+    -inf goes on the last id of every bad word whose first L - 1 ids end the context and, on rows predicting a position
+    below min_tokens, on `eos` and on the last id of every stop sequence whose head ends the context.  `n_nodes` /
+    `n_paths` [B] int32: live rows and paths per request; `done` [B] bool/uint8: finished requests are not touched, nor
+    are neutral slots.  Every argument is checked before anything reaches the device."""
+    if logits.dim() != 3 or logits.stride(2) != 1:
+        raise K.SamdError(f"apply_logit_controls: logits must be [B, T, V] with unit stride over V, got "
+                          f"{tuple(logits.shape)}")
+    B, T, V = logits.shape
+    dt = {torch.bfloat16: K.DTYPE_BF16, torch.float16: K.DTYPE_FP16, torch.float32: K.DTYPE_FP32}.get(logits.dtype)
+    if dt is None:
+        raise K.SamdError(f"apply_logit_controls: unsupported logits dtype {logits.dtype} (bf16 / fp16 / fp32)")
+    if not 1 <= T <= 256:
+        raise K.SamdError(f"apply_logit_controls: at most 256 rows per request, got {T}")
+    if min_tokens.dim() != 1 or min_tokens.shape[0] == 0:
+        raise K.SamdError(f"apply_logit_controls: min_tokens must be [S] with S >= 1, got {tuple(min_tokens.shape)}")
+    S = min_tokens.shape[0]
+    if slots is None and S != B:
+        raise K.SamdError(f"apply_logit_controls: without slots the tables need one row per request ({B}), got {S}")
+    if retrieve is not None and tokens is None:
+        raise K.SamdError("apply_logit_controls: a path table needs the node tokens")
+    if retrieve is not None and (retrieve.dim() != 3 or retrieve.shape[0] != B or 0 in retrieve.shape):
+        raise K.SamdError(f"apply_logit_controls: retrieve must be [{B}, P, D], got {tuple(retrieve.shape)}")
+    if n_paths is not None and retrieve is None:
+        raise K.SamdError("apply_logit_controls: n_paths needs a path table")
+    if hist_len is not None and (hist is None or hist.dim() != 2 or hist.shape[0] != S or hist.shape[1] == 0):
+        raise K.SamdError(f"apply_logit_controls: hist_len needs hist [{S}, H] with H >= 1, got "
+                          f"{None if hist is None else tuple(hist.shape)}")
+    if (stop_tokens is None) != (stop_len is None):
+        raise K.SamdError("apply_logit_controls: stop_tokens and stop_len go together")
+    if eos is not None and (isinstance(eos, bool) or not isinstance(eos, int) or not 0 <= eos < V):
+        raise K.SamdError(f"apply_logit_controls: eos must be None or a token id in [0, {V}), got {eos!r}")
+    M, NB, LB = K.BIAS_MAX, K.BAD_MAX_SEQS, K.BAD_MAX_LEN
+    i32, f32 = (torch.int32,), (torch.float32,)
+    for name, t, shape, dtypes in (("bias_ids", bias_ids, (S, M), i32), ("bias", bias, (S, M), f32),
+                                   ("bias_n", bias_n, (S,), i32), ("bad_tokens", bad_tokens, (S, NB, LB), i32),
+                                   ("bad_len", bad_len, (S, NB), i32), ("min_tokens", min_tokens, (S,), i32),
+                                   ("tokens", tokens, (B, T), i32),
+                                   ("retrieve", retrieve, None if retrieve is None else tuple(retrieve.shape), i32),
+                                   ("n_nodes", n_nodes, (B,), i32), ("n_paths", n_paths, (B,), i32),
+                                   ("done", done, (B,), (torch.bool, torch.uint8)), ("slots", slots, (B,), i32),
+                                   ("hist", hist, None if hist is None else tuple(hist.shape), i32),
+                                   ("hist_len", hist_len, (S,), i32),
+                                   ("stop_tokens", stop_tokens, (S, K.STOP_MAX_SEQS, K.STOP_MAX_LEN), i32),
+                                   ("stop_len", stop_len, (S, K.STOP_MAX_SEQS), i32)):
+        if t is None:
+            continue
+        if tuple(t.shape) != shape or t.dtype not in dtypes or not t.is_contiguous():
+            raise K.SamdError(f"apply_logit_controls: {name} must be a contiguous {shape} {dtypes[0]} tensor, got "
+                              f"{tuple(t.shape)} {t.dtype}")
+    opt = (tokens, retrieve, n_nodes, n_paths, done, slots, hist, hist_len, stop_tokens, stop_len)
+    tensors = [logits, bias_ids, bias, bias_n, bad_tokens, bad_len, min_tokens] + [x for x in opt if x is not None]
+    if not all(t.is_cuda and t.device == logits.device for t in tensors):
+        raise K.SamdError("apply_logit_controls: every tensor must be on the logits' GPU")
+    a = K.LogitControlArgs()
+    a.logits_dev, a.dtype, a.batch, a.n_nodes, a.vocab = logits.data_ptr(), dt, B, T, V
+    a.batch_stride, a.row_stride = logits.stride(0), logits.stride(1)
+    a.tokens_dev, a.retrieve_dev = K.ptr(tokens), K.ptr(retrieve)
+    a.n_paths, a.depth = (retrieve.shape[1], retrieve.shape[2]) if retrieve is not None else (1, T)
+    a.n_nodes_dev, a.n_paths_dev, a.done_dev, a.slots_dev = K.ptr(n_nodes), K.ptr(n_paths), K.ptr(done), K.ptr(slots)
+    a.n_slots = S
+    a.hist_dev, a.hist_len_dev = K.ptr(hist), K.ptr(hist_len)
+    a.hist_stride = hist.shape[1] if hist is not None else 0
+    a.bias_ids_dev, a.bias_dev, a.bias_n_dev = bias_ids.data_ptr(), bias.data_ptr(), bias_n.data_ptr()
+    a.bad_tokens_dev, a.bad_len_dev, a.min_tokens_dev = bad_tokens.data_ptr(), bad_len.data_ptr(), min_tokens.data_ptr()
+    a.stop_tokens_dev, a.stop_len_dev = K.ptr(stop_tokens), K.ptr(stop_len)
+    a.eos_token = -1 if eos is None else eos
+    with torch.cuda.device(logits.device):
+        K.check(K.lib().samd_apply_logit_controls(C.byref(a), K.stream_ptr()), "samd_apply_logit_controls")
+    return logits
+
+
 class Verifier:
     """Fused greedy verification + KV compaction (samd/utils.py:127-141, samd/samd_model.py:159-211,
     samd/cache.py:118-133) for a batch of requests: one persistent launch."""
